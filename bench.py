@@ -41,6 +41,14 @@ Also in the JSON line (round 2):
   roofline  of the dominant kernel; K7 advances TWO timesteps per launch with the 72 B per
             cell of one pass, so algorithmic bytes per update = 36; `traffic` is the ncu
             figure of the committed capture named in `traffic_source`.
+
+--dump-outputs DIR writes what the last timed step of `value` computed, so that two builds
+can be compared output for output on the same inputs (the workload is seeded):
+  av_vels.npy           float32 (T,), the step's av_vels as lbm_gpu_run returns them
+  cells_rows.npy        float32 (64, nx, 9), lattice rows after the step (lbm_gpu_download layout)
+  cells_rows_index.npy  float64 (64,), which rows: a fixed seeded sample of the grid
+About 38 MB at nx = 16384.  The last timed step then fetches its av_vels (one small kernel
+after the step's end event: the device time is unchanged, `gpu_launches` counts it).
 """
 import argparse
 import ctypes
@@ -55,6 +63,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the tree may be read-only: no __pycache__ written into it
 
 from tools.make_inputs import channel_mask  # noqa: E402
 
@@ -66,6 +75,7 @@ DENSITY, ACCEL, OMEGA = 0.1, 0.005, 1.85
 BYTES_PER_UPDATE = 72.0            # 9 fp32 loads + 9 fp32 stores (SURVEY.md section 8d)
 CPU_SAMPLE_ROWS = min(1024, ROWS_PER_GPU)   # CPU legs run a 16384 x 1024 slab of the same generator
 HBM_FALLBACK_GBS = 6650.0          # B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
+DUMP_ROWS, DUMP_SEED = 64, 20240229          # --dump-outputs: lattice rows sampled, and their seed
 
 
 # ------------------------------------------------------------------------- clocks ----
@@ -292,6 +302,15 @@ class Ranks:
         a = np.asarray(a, dtype=np.float64)
         return a if self.dist is None else np.array(self._reduce(a, self.dist.ReduceOp.SUM, _f64()))
 
+    def sum_f32_array(self, a):
+        """element-wise float32 sum over ranks, through the GPU (for arrays too big for sum_array)"""
+        if self.dist is None:
+            return a
+        import torch
+        t = torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)).cuda()
+        self.dist.all_reduce(t, op=self.dist.ReduceOp.SUM)
+        return t.cpu().numpy()
+
     def sum_u64(self, x):
         """wrapping 64-bit sum over ranks (16-bit pieces in int64, so nothing overflows on the way)"""
         if self.dist is None:
@@ -483,6 +502,24 @@ def shipped_block(L):
     return res
 
 
+def dump_outputs(path, lat, R, sums, ny, row0, nrows):
+    """--dump-outputs: the av_vels of the last timed step and a seeded sample of lattice rows
+    after it.  Each rank downloads the sampled rows it holds; rank 0 writes the files."""
+    free = R.sum(float(lat.info().local_free_cells))
+    av = (R.sum_array(sums) / free).astype(np.float32)        # lbm_gpu_run's own rounding
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(ny, size=min(DUMP_ROWS, ny), replace=False))
+    cells = np.zeros((rows.size, NX, 9), dtype=np.float32)
+    for i, r in enumerate(rows):
+        if row0 <= r < row0 + nrows:
+            cells[i] = lat.download_rows(int(r), 1)[0]
+    cells = R.sum_f32_array(cells)          # each row is held by one rank, the others add zeros
+    if R.rank == 0:
+        os.makedirs(path, exist_ok=True)
+        np.save(os.path.join(path, "av_vels.npy"), av)
+        np.save(os.path.join(path, "cells_rows.npy"), cells)
+        np.save(os.path.join(path, "cells_rows_index.npy"), rows.astype(np.float64))
+
+
 def library_id(L):
     import hashlib
     with open(L.LIB_PATH, "rb") as f:
@@ -504,7 +541,13 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-shipped", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/*.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the GPU arm (--impl b200)")
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs at least one timed step (--steps >= 1)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3                      # timing rule: at least 3 warm-up steps
 
@@ -560,14 +603,18 @@ def main():
         connect(lat, L, slabs, R)
         return lat
 
-    def timed_runs(lat, n_runs, warm):
+    def timed_runs(lat, n_runs, warm, last_sums=None):
         for _ in range(warm):
             lat.run_timed(T)
         barrier()
         t0 = time.perf_counter()
         dev_ms = 0.0
-        for _ in range(n_runs):
-            dev_ms += lat.run_timed(T)          # returns with the device idle (stream sync inside)
+        for i in range(n_runs):
+            if last_sums is not None and i == n_runs - 1:
+                last_sums[...] = lat.run_sums(T)     # same device-timed step, av_vels sums fetched after it
+                dev_ms += lat.info().last_run_device_ms
+            else:
+                dev_ms += lat.run_timed(T)          # returns with the device idle (stream sync inside)
         barrier()
         return max_over_ranks(dev_ms), max_over_ranks(time.perf_counter() - t0)
 
@@ -588,9 +635,12 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    dev_ms, wall_s = timed_runs(lat, K, 0)
+    last_sums = np.empty(T) if args.dump_outputs else None
+    dev_ms, wall_s = timed_runs(lat, K, 0, last_sums)
     clocks = sampler.stop() if rank == 0 else None
     launches = lat.info().kernel_launches - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, lat, R, last_sums, ny, row0, nrows)
     mass1 = sum_over_ranks(lat.digest()[0])
     av_tail = lat.run_sums(2)               # sanity: the numbers are finite and positive
     assert np.all(np.isfinite(av_tail)) and np.all(av_tail > 0), av_tail

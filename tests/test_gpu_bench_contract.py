@@ -43,3 +43,45 @@ def test_gpu_arm_prints_contract_line():
     assert e["h2d_bytes_per_step"] == cells * 4 and e["d2h_bytes_per_step"] == 4 * cells * 4 + 20 * 4
     assert d["config"]["workload"].startswith("synthetic 4096x4096 channel")
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
+
+
+def test_dump_outputs_is_reproducible_and_follows_steps(tmp_path):
+    """--dump-outputs: the arrays are those of the last timed step (rebuilt here with a fresh
+    lattice); the same arguments give the same arrays; one more timed step gives others."""
+    import numpy as np
+    import lbm_b200 as L
+    from tools.make_inputs import channel_mask
+    nx, ny, T, warmup = 4096, 2048, 20, 3
+    env = dict(os.environ, LBM_BENCH_NX=str(nx), LBM_BENCH_ROWS=str(ny))
+
+    def dump(name, steps):
+        d = tmp_path / name
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", str(warmup),
+                            "--timesteps", str(T), "--dump-outputs", str(d), "--no-cpu-baseline", "--no-e2e",
+                            "--no-parity", "--no-shipped", "--no-strong"],
+                           stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, env=env, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+        assert all(p.suffix == ".npy" for p in d.iterdir())
+        return {p.stem: np.load(p) for p in d.iterdir()}
+
+    a, b, c = dump("a", 2), dump("b", 2), dump("c", 3)
+    assert set(a) == {"av_vels", "cells_rows", "cells_rows_index"}
+    assert a["av_vels"].shape == (T,) and a["cells_rows"].shape == (64, nx, 9)
+    # the same workload from scratch: warm-up plus timed steps of T timesteps, the last one fetched
+    with L.Lattice(nx, ny, 0.1, 0.005, 1.85, obstacles=channel_mask(nx, ny)) as lat:
+        for _ in range(warmup + 2 - 1):
+            lat.run_timed(T)
+        av = (lat.run_sums(T) / lat.info().local_free_cells).astype(np.float32)
+        rows = np.stack([lat.download_rows(int(r), 1)[0] for r in a["cells_rows_index"]])
+    assert np.array_equal(a["av_vels"], av)
+    assert np.array_equal(a["cells_rows"], rows)
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert np.all(a["av_vels"] > 0) and np.isfinite(a["cells_rows"]).all()
+    assert (np.abs(a["cells_rows"]).sum(axis=(1, 2)) > 0).all()        # every sampled row was filled in
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+    assert np.array_equal(a["cells_rows_index"], c["cells_rows_index"])
+    assert not np.array_equal(a["cells_rows"], c["cells_rows"])
+    assert not np.array_equal(a["av_vels"], c["av_vels"])
