@@ -28,6 +28,7 @@ KERNEL_CLUSTER = 256
 KERNEL_TB2 = 512
 SYNC_EVENTS = 1024
 KERNEL_PAIRS = 2048
+KERNEL_TB3 = 4096
 IPC_DESC_BYTES = 256
 
 

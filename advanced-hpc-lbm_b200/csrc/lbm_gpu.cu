@@ -7,6 +7,7 @@
 #include "lbm_kernels.cuh"
 #include "lbm_cluster.cuh"
 #include "lbm_tb2.cuh"
+#include "lbm_tb3.cuh"
 #include "lbm_pairs.cuh"
 
 #include <unistd.h>
@@ -92,6 +93,8 @@ enum SyncWord { kFlagFromBelow = 0, kFlagFromAbove = 1, kBoundaryDone = 2, kScra
                 kScratch2 = 5, kGridBarrier = 6, kAbort = 7, kSyncError = 8 /* must follow kAbort */,
                 kAvScratch = 16 /* kAvWords words */, kSyncWords = 16 + 128 };
 constexpr int kTb2MinRows = 8;                             // per slab, for the two-step kernel
+constexpr int kTb3MinRows = 12;                            // for the three-step kernel (one slab)
+constexpr double kTb3MinWaves = 4.0;                       // K10 by default from this many waves of its blocks on
 constexpr int kAvWords = LBM_AV_STRIDE * LBM_AV_SLOTS;     // words of one step's |u| sums (1 KiB)
 constexpr int kMaxSegmentSteps = 1 << 16;                  // 64 MiB of sums per run segment
 
@@ -171,6 +174,8 @@ class Grid : public GridBase {
   bool tb2 = false;            // two timesteps per pass (K7) wherever two steps remain
   int tb2_strips = 0, tb2_wout = 0, tb2_seg_rows = 0, tb2_span = 0, tb2_threads = 0;
   int tb2_tail_rows = 16, tb2_tail_segs = 0;   // K7: height and number of the short segments that end a launch
+  bool tb3 = false;            // three timesteps per pass (K10) wherever three steps remain (K7 for two, K1a for one)
+  int tb3_seg_rows = 0;        // K10: rows per segment
   int pairs_tile_rows = 0;     // K9: rows per block
   bool failed = false;         // a neighbour never arrived: the lattice contents are void
   unsigned long long timeout_ns = 10000000000ULL;
@@ -346,7 +351,7 @@ class Grid : public GridBase {
     if (flags & LBM_GPU_KERNEL_SCALAR) kernel = LBM_GPU_KERNEL_SCALAR;
     else if (flags & LBM_GPU_KERNEL_VEC4) kernel = LBM_GPU_KERNEL_VEC4;
     else if (flags & LBM_GPU_KERNEL_PERSISTENT) kernel = LBM_GPU_KERNEL_PERSISTENT;
-    else if (flags & LBM_GPU_KERNEL_TB2) kernel = LBM_GPU_KERNEL_VEC4;         // decided in choose_tb2()
+    else if (flags & (LBM_GPU_KERNEL_TB2 | LBM_GPU_KERNEL_TB3)) kernel = LBM_GPU_KERNEL_VEC4;   // decided in choose_tb2()
     else if (flags & LBM_GPU_KERNEL_PAIRS) kernel = LBM_GPU_KERNEL_VEC4;       // decided in choose_pairs()
     else if (flags & LBM_GPU_KERNEL_CLUSTER) kernel = LBM_GPU_KERNEL_VEC4;     // decided in choose_kernel()
     else kernel = LBM_GPU_KERNEL_VEC4;                         // refined in choose_kernel()
@@ -429,7 +434,7 @@ class Grid : public GridBase {
   void choose_kernel() {
     const bool forced = flags & (LBM_GPU_KERNEL_SCALAR | LBM_GPU_KERNEL_VEC4 | LBM_GPU_KERNEL_PERSISTENT |
                                  LBM_GPU_KERNEL_TMA | LBM_GPU_KERNEL_CLUSTER | LBM_GPU_KERNEL_TB2 |
-                                 LBM_GPU_KERNEL_PAIRS);
+                                 LBM_GPU_KERNEL_PAIRS | LBM_GPU_KERNEL_TB3);
     // K6 is opt-in only: 16 SMs doing all the arithmetic are no faster than K5 spreading it
     // over the whole chip (profiles/r01_small_grids.md).
     if (flags & LBM_GPU_KERNEL_CLUSTER) {
@@ -502,17 +507,10 @@ class Grid : public GridBase {
       // that is nearly empty leaves the SMs idle (16384 rows in 64-row segments: 19.03 waves).
       // Score each height by (rows / (rows + 2)) x (waves / ceil(waves)) and take the best; grids
       // with few blocks prefer short segments so that there are several waves at all.
-      int sms = 148, rows_max = 0;
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, slabs[0].device);
+      int rows_max = 0;
       for (auto& s : slabs) rows_max = std::max(rows_max, s.rows);
-      const double resident = (double)LBM_TB2_MIN_BLOCKS * sms;
-      double best = -1.0;
-      tb2_seg_rows = 64;
-      for (int h = 16; h <= 128; h++) {
-        const double waves = (double)tb2_strips * ((rows_max + h - 1) / h) / resident;
-        const double score = (double)h / (h + 2) * waves / std::ceil(waves) * (waves >= 4.0 ? 1.0 : 0.25 * waves);
-        if (score > best + 1e-9) { best = score; tb2_seg_rows = h; }
-      }
+      const double resident = (double)LBM_TB2_MIN_BLOCKS * sm_count();
+      tb2_seg_rows = best_segment_rows(rows_max, resident, 2, 128);
       if (const char* e = getenv("LBM_TB2_SEG_ROWS")) tb2_seg_rows = std::max(2, atoi(e));   // tuning knob
       // A block lives (segment height) x ~2.6 us; the last blocks of a launch to be scheduled
       // leave the other SMs idle for about half of that.  So the launch ENDS with short
@@ -523,6 +521,58 @@ class Grid : public GridBase {
       if (tb2_tail_rows < 2) tb2_tail_segs = 0;
       tb2 = true;
       kernel = LBM_GPU_KERNEL_TB2;
+    }
+  }
+
+  int sm_count() const {
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, slabs[0].device);
+    return sms;
+  }
+  // blocks of a launch of `rows` rows in segments of h rows, in waves of `resident` blocks
+  double tb_waves(int rows, int h, double resident) const { return (double)tb2_strips * ((rows + h - 1) / h) / resident; }
+  // Segment height of K7 (extra = 2 recomputed rows) and K10 (4).  The blocks of a launch run
+  // in "waves" of the resident blocks and a last wave that is nearly empty leaves the SMs idle
+  // (16384 rows in 64-row segments: 19.03 waves of K7).  Score each height by
+  // (rows / (rows + extra)) x (waves / ceil(waves)) and take the best; grids with few blocks
+  // prefer short segments so that there are several waves at all.
+  int best_segment_rows(int rows, double resident, int extra, int h_max) const {
+    double best = -1.0;
+    int best_h = 64;
+    for (int h = 16; h <= h_max; h++) {
+      const double waves = tb_waves(rows, h, resident);
+      const double score = (double)h / (h + extra) * waves / std::ceil(waves) * (waves >= 4.0 ? 1.0 : 0.25 * waves);
+      if (score > best + 1e-9) { best = score; best_h = h; }
+    }
+    return best_h;
+  }
+
+  // K10 (three timesteps per pass) on top of K7: one slab that holds the whole grid (its
+  // rows beyond the ends are its own, so no three-deep ghost zones are needed), at least
+  // kTb3MinRows rows, and the K7 conditions.
+  bool tb3_possible() const {
+    return slabs.size() == 1 && slabs[0].rows == prm.ny && slabs[0].row0 == 0 && !(flags & LBM_GPU_KERNEL_TB2) &&
+           tb2_possible(slabs[0].rows) && slabs[0].rows >= kTb3MinRows &&
+           !(getenv("LBM_GPU_NO_TB3") && getenv("LBM_GPU_NO_TB3")[0] == '1');
+  }
+  // Default: K10 where it was measured faster than K7 (profiles/r03_size_sweep.log), i.e. where
+  // its blocks fill enough waves of the SMs; with few waves the launch tail of K10's longer
+  // blocks costs more than the bytes it saves.
+  bool tb3_pays() const {
+    const double resident = (double)LBM_TB3_MIN_BLOCKS * sm_count();
+    return tb_waves(slabs[0].rows, 64, resident) >= kTb3MinWaves;
+  }
+  void enable_tb3() {
+    if constexpr (sizeof(real) == 4) {
+      Slab<real>& s = slabs[0];
+      CK(cudaSetDevice(s.device));
+      for (const void* fn : {(const void*)lbm::lbm_step3_tb<false>, (const void*)lbm::lbm_step3_tb<true>})
+        CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(lbm::Tb3Smem)));
+      const double resident = (double)LBM_TB3_MIN_BLOCKS * sm_count();
+      tb3_seg_rows = best_segment_rows(s.rows, resident, 4, 96);   // 96 rows measured best at 16384^2 (profiles/r03_k10.md)
+      if (const char* e = getenv("LBM_TB3_SEG_ROWS")) tb3_seg_rows = std::max(1, atoi(e));   // tuning knob
+      tb3 = true;
+      kernel = LBM_GPU_KERNEL_TB3;
     }
   }
 
@@ -545,6 +595,17 @@ class Grid : public GridBase {
       nsegs--;
     }
     g.n_big = nsegs;
+    return g;
+  }
+
+  // segments of the slab for K10: equal heights (one slab: no rows need to sit in edge segments)
+  Tb2Segments tb3_segments(int rows) const {
+    Tb2Segments g;
+    const int nsegs = (rows + tb3_seg_rows - 1) / tb3_seg_rows;
+    g.seg_rows = g.seg_rows_tail = (rows + nsegs - 1) / nsegs;
+    g.n_big = (rows + g.seg_rows - 1) / g.seg_rows;
+    g.big_rows = rows;
+    g.n_tail = 0;
     return g;
   }
 
@@ -592,9 +653,14 @@ class Grid : public GridBase {
     int rows_min = slabs[0].rows;
     for (auto& s : slabs) rows_min = std::min(rows_min, s.rows);
     const bool want = (flags & LBM_GPU_KERNEL_TB2) != 0;
+    const bool want3 = (flags & LBM_GPU_KERNEL_TB3) != 0;
     const bool big = (kernel == LBM_GPU_KERNEL_VEC4);        // not taken by the persistent kernel
-    if (tb2_possible(rows_min) && (want || big)) enable_tb2();
+    if (want3 && !tb3_possible())
+      throw CudaError{"the three-step kernel needs fp32, nx a multiple of 4 and >= 32, the whole grid in one slab, "
+                      "and >= 12 rows"};
+    if (tb2_possible(rows_min) && (want || want3 || big)) enable_tb2();
     else if (want) throw CudaError{"the two-step kernel needs fp32, nx a multiple of 4 and >= 32, and >= 8 rows per slab"};
+    if (want3 || (big && tb3_possible() && tb3_pays())) enable_tb3();
   }
 
   // ------------------------------------------------------------- lattice input ----
@@ -736,7 +802,7 @@ class Grid : public GridBase {
       a.mask_dn = s.dn_gmask;
       a.plane_stride = plane_stride(s);
       a.nx = prm.nx; a.rows = s.rows; a.pitch = pitch; a.mask_pitch = mask_pitch; a.accel_row = s.accel_row;
-      a.deep = tb2 ? 1 : 0;
+      a.deep = tb2 ? 1 : 0;                // K10 reads the source lattice directly: K7's ghost rows are enough
       a.aw1 = prm.density * prm.accel / (real)9;      // d2q9-bgk.c:230-231
       a.aw2 = prm.density * prm.accel / (real)36;
       lbm::lbm_prepare<real><<<(std::max(prm.nx, mask_pitch) + 127) / 128, 128, 0, s.stream>>>(a);
@@ -789,6 +855,11 @@ class Grid : public GridBase {
   void launch_tb2(Slab<real>& s, const lbm::Tb2Args& ta, dim3 grid) {
     if constexpr (sizeof(real) == 4)
       launch_pdl(s, lbm::lbm_step2_tb<STRICT, MULTI>, ta, grid, dim3(tb2_threads), sizeof(lbm::Tb2Smem));
+  }
+  template <bool STRICT>
+  void launch_tb3(Slab<real>& s, const lbm::Tb2Args& ta, dim3 grid) {
+    if constexpr (sizeof(real) == 4)
+      launch_pdl(s, lbm::lbm_step3_tb<STRICT>, ta, grid, dim3(tb2_threads), sizeof(lbm::Tb3Smem));
   }
 
   void launch_cluster(int n_steps, bool strict) {
@@ -877,8 +948,9 @@ class Grid : public GridBase {
     a.aw2 = prm.density * prm.accel / (real)36;
   }
 
-  // one pass over every slab: one timestep (K1a/K1b/K1c), or two (K7) when `two`
-  void launch_pass(int t_in_segment, int pass_in_segment, bool two) {
+  // one pass over every slab: one timestep (K1a/K1b/K1c), two (K7) or three (K10)
+  void launch_pass(int t_in_segment, int pass_in_segment, int steps) {
+    const bool two = (steps == 2);
     const bool strict = (flags & LBM_GPU_STRICT) != 0;
     const int nslabs = (int)slabs.size();
     int vec, bx, by;
@@ -896,7 +968,27 @@ class Grid : public GridBase {
       }
       lbm::StepArgs<real> a;
       fill_step_args(a, s, t_in_segment);
-      if (two) {
+      if (steps == 3) {
+        if constexpr (sizeof(real) == 4) {
+          lbm::Tb2Args ta;
+          const Tb2Segments sg = tb3_segments(s.rows);
+          a.tiles_x = tb2_strips;
+          a.tiles_y = sg.n_big;
+          ta.s = a;
+          ta.ghost_mask = nullptr;
+          ta.av2 = a.av + kAvWords;
+          ta.av3 = a.av + 2 * kAvWords;
+          ta.wout = tb2_wout;
+          ta.span = tb2_span;
+          ta.seg_rows = sg.seg_rows;
+          ta.n_big = sg.n_big;
+          ta.big_rows = sg.big_rows;
+          ta.seg_rows_tail = sg.seg_rows_tail;
+          const dim3 grid((unsigned)((long long)tb2_strips * sg.n_big));
+          if (strict) launch_tb3<true>(s, ta, grid);
+          else        launch_tb3<false>(s, ta, grid);
+        }
+      } else if (two) {
         if constexpr (sizeof(real) == 4) {
           lbm::Tb2Args ta;
           const Tb2Segments sg = tb2_segments(s.rows);
@@ -908,6 +1000,7 @@ class Grid : public GridBase {
           ta.s = a;
           ta.ghost_mask = s.ghost_mask;
           ta.av2 = a.av + kAvWords;
+          ta.av3 = nullptr;
           ta.wout = tb2_wout;
           ta.span = tb2_span;
           ta.seg_rows = sg.seg_rows;
@@ -1009,13 +1102,13 @@ class Grid : public GridBase {
           passes_done += n_pairs;
         }
       }
-      if (n_steps & 1) launch_pass(n_steps - 1, 0, false);     // the odd last step: K1a
+      if (n_steps & 1) launch_pass(n_steps - 1, 0, 1);     // the odd last step: K1a
     } else {
       int t = 0, p = 0;
       while (t < n_steps) {
-        const bool two = tb2 && (n_steps - t >= 2);
-        launch_pass(t, p, two);
-        t += two ? 2 : 1;
+        const int steps = (tb3 && n_steps - t >= 3) ? 3 : (tb2 && n_steps - t >= 2) ? 2 : 1;
+        launch_pass(t, p, steps);
+        t += steps;
         p++;
       }
       if (use_flags) {
@@ -1493,6 +1586,9 @@ void ipc_connect_impl(Grid<float>& g, const IpcDesc& dn, const IpcDesc& up, bool
   s.up_gmask = (uint32_t*)(s.up_win + up.off_gmask);
   g.multi = true;
   g.use_flags = true;      // neighbours are other processes: device-side flags
+  if (g.flags & LBM_GPU_KERNEL_TB3) throw CudaError{"the three-step kernel needs the whole grid in one slab"};
+  g.tb3 = false;                   // a ring of slabs: K7 at most
+  if (g.kernel == LBM_GPU_KERNEL_TB3) g.kernel = LBM_GPU_KERNEL_VEC4;
   if (g.flags & LBM_GPU_KERNEL_TB2) {
     if (!ring_tb2) throw CudaError{"the two-step kernel needs lbm_gpu_ipc_connect_all and fp32, nx a multiple of 4 "
                                    "and >= 32, >= 8 rows on every rank"};

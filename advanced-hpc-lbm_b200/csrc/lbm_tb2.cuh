@@ -69,6 +69,7 @@ struct Tb2Args {
   int n_big;                       // ... of the first n_big segments, which cover rows [0, big_rows);
   int big_rows;                    // the segments behind them are seg_rows_tail rows tall: they get the highest
   int seg_rows_tail;               // block indices, so a launch ends with short blocks and the SMs drain together
+  unsigned long long* av3;         // K10 only: sums of sub-step 3
 };
 
 __device__ __forceinline__ void tb2_mbar_wait(unsigned long long* bar, const uint32_t parity) {
@@ -85,10 +86,16 @@ __device__ __forceinline__ void tb2_bulk_load(float* dst_smem, const float* src,
                ::"r"(smem_u32(dst_smem)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 
-// where plane k of local row `row` of the SOURCE state lives (row in [-2, rows + 2))
-__device__ __forceinline__ const float* tb2_row_ptr(const StepArgs<float>& a, const int k, const int row) {
-  if (row < 0) return a.ghost_s + (long long)((-1 - row) * 9 + k) * a.pitch;
-  if (row >= a.rows) return a.ghost_n + (long long)((row - a.rows) * 9 + k) * a.pitch;
+// where plane k of local row `row` of the SOURCE state lives (row in [-2, rows + 2)); PERIODIC:
+// the slab is the whole grid and rows beyond its ends are its own rows (row in [-rows, 2 rows))
+template <bool PERIODIC = false>
+__device__ __forceinline__ const float* tb2_row_ptr(const StepArgs<float>& a, const int k, int row) {
+  if (PERIODIC) {
+    row = (row < 0) ? row + a.rows : (row >= a.rows) ? row - a.rows : row;
+  } else {
+    if (row < 0) return a.ghost_s + (long long)((-1 - row) * 9 + k) * a.pitch;
+    if (row >= a.rows) return a.ghost_n + (long long)((row - a.rows) * 9 + k) * a.pitch;
+  }
   if (row == a.accel_row && k != 0 && k != 2 && k != 4) {
     const int idx = (k == 1) ? 0 : (k == 3) ? 1 : k - 3;       // side row order 1,3,5,6,7,8
     return a.side_src + (long long)idx * a.pitch;
@@ -101,7 +108,8 @@ __device__ __forceinline__ const float* tb2_row_ptr(const StepArgs<float>& a, co
 // in different warps first) works out where "its" plane-row lives and copies it, in as many
 // pieces as the periodic wrap in x cuts the span into (up to three when the span is the
 // whole width plus halo).  The bytes were announced before by tb2_expect.
-__device__ __forceinline__ void tb2_expect(Tb2Smem& sm, const int stage, const int span) {
+template <typename Smem>
+__device__ __forceinline__ void tb2_expect(Smem& sm, const int stage, const int span) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&sm.mbar[stage])),
                "r"((uint32_t)(9 * span * sizeof(float))) : "memory");
 }
@@ -110,12 +118,13 @@ __device__ __forceinline__ int tb2_plane_of_thread() {
   const int k = w + nwarps * lane;
   return (k < 9) ? k : -1;
 }
-__device__ __forceinline__ void tb2_issue(const StepArgs<float>& a, Tb2Smem& sm, const int stage, const int r,
+template <bool PERIODIC = false, typename Smem>
+__device__ __forceinline__ void tb2_issue(const StepArgs<float>& a, Smem& sm, const int stage, const int r,
                                           const int s0, const int span, const int k) {
   if (k < 0) return;
   unsigned long long* bar = &sm.mbar[stage];
   const int dy = (k == 2 || k == 5 || k == 6) ? -1 : (k == 4 || k == 7 || k == 8) ? 1 : 0;
-  const float* row = tb2_row_ptr(a, k, r + dy);
+  const float* row = tb2_row_ptr<PERIODIC>(a, k, r + dy);
   float* dst = &sm.in[stage][k][LBM_TB2_PAD];
   int col = s0, left = span;
   while (left > 0) {
@@ -149,6 +158,48 @@ __device__ __forceinline__ void tb2_ring_read_done(Tb2Smem& sm) {
 }
 __device__ __forceinline__ void tb2_put(float* row, const int c0, const float (&o)[4][9], const int k) {
   *reinterpret_cast<float4*>(row + LBM_TB2_PAD + c0) = make_float4(o[0][k], o[1][k], o[2][k], o[3][k]);
+}
+
+// a thread's quad of a finished row y goes to the destination lattice with 128-bit stores; the
+// slab's two edge rows at each end are also pushed into the neighbours' ghost rows, row ny-2
+// also (accelerated) into the side row.  `out` is accelerated in place on that row.
+template <bool STRICT>
+__device__ __forceinline__ void tb2_store_row(const StepArgs<float>& a, const int y, const int xg, float (&out)[4][9],
+                                              const uint32_t mbits) {
+  const long long PS = a.plane_stride;
+  float* d = a.dst + (long long)y * a.pitch + xg;
+#pragma unroll
+  for (int k = 0; k < 9; k++)
+    *reinterpret_cast<float4*>(d + k * PS) = make_float4(out[0][k], out[1][k], out[2][k], out[3][k]);
+  const bool first = (y == 0), second = (y == 1), last = (y == a.rows - 1), before_last = (y == a.rows - 2);
+  const bool cA = (y == a.accel_row);
+  if (first | second | last | before_last | cA) {        // block-uniform
+    if (cA) {
+#pragma unroll
+      for (int j = 0; j < 4; j++)
+        cell_accelerate<float, STRICT>(out[j][1], out[j][3], out[j][5], out[j][6], out[j][7], out[j][8],
+                                       (mbits >> j) & 1u, a.aw1, a.aw2);
+      const int ks[6] = {1, 3, 5, 6, 7, 8};
+#pragma unroll
+      for (int n = 0; n < 6; n++)
+        *reinterpret_cast<float4*>(a.side_dst + (long long)n * a.pitch + xg) =
+            make_float4(out[0][ks[n]], out[1][ks[n]], out[2][ks[n]], out[3][ks[n]]);
+    }
+#define LBM_TB2_PUSH(dst, depth, k)                                                             \
+  *reinterpret_cast<float4*>((dst) + (long long)((depth) * 9 + (k)) * a.pitch + xg) =          \
+      make_float4(out[0][k], out[1][k], out[2][k], out[3][k]);
+    if (first) {
+      LBM_TB2_PUSH(a.push_dn, 0, 4) LBM_TB2_PUSH(a.push_dn, 0, 7) LBM_TB2_PUSH(a.push_dn, 0, 8)
+      LBM_TB2_PUSH(a.push_dn, 0, 0) LBM_TB2_PUSH(a.push_dn, 0, 1) LBM_TB2_PUSH(a.push_dn, 0, 3)
+    }
+    if (last) {
+      LBM_TB2_PUSH(a.push_up, 0, 2) LBM_TB2_PUSH(a.push_up, 0, 5) LBM_TB2_PUSH(a.push_up, 0, 6)
+      LBM_TB2_PUSH(a.push_up, 0, 0) LBM_TB2_PUSH(a.push_up, 0, 1) LBM_TB2_PUSH(a.push_up, 0, 3)
+    }
+    if (second) { LBM_TB2_PUSH(a.push_dn, 1, 4) LBM_TB2_PUSH(a.push_dn, 1, 7) LBM_TB2_PUSH(a.push_dn, 1, 8) }
+    if (before_last) { LBM_TB2_PUSH(a.push_up, 1, 2) LBM_TB2_PUSH(a.push_up, 1, 5) LBM_TB2_PUSH(a.push_up, 1, 6) }
+#undef LBM_TB2_PUSH
+  }
 }
 
 // One tile = one strip x one segment, two timesteps.  `phases` holds the parity each staging
@@ -262,40 +313,7 @@ __device__ __forceinline__ void tb2_tile(const Tb2Args& ta, Tb2Smem& sm, const i
       if (owned) {
         q2 += q;
         bad2 |= bad;
-        const long long PS = a.plane_stride;
-        float* d = a.dst + (long long)y * a.pitch + xg;
-#pragma unroll
-        for (int k = 0; k < 9; k++)
-          *reinterpret_cast<float4*>(d + k * PS) = make_float4(out[0][k], out[1][k], out[2][k], out[3][k]);
-        const bool first = (y == 0), second = (y == 1), last = (y == a.rows - 1), before_last = (y == a.rows - 2);
-        const bool cA = (y == a.accel_row);
-        if (first | second | last | before_last | cA) {        // block-uniform
-          if (cA) {
-#pragma unroll
-            for (int j = 0; j < 4; j++)
-              cell_accelerate<float, STRICT>(out[j][1], out[j][3], out[j][5], out[j][6], out[j][7], out[j][8],
-                                             (mbits_prev >> j) & 1u, a.aw1, a.aw2);
-            const int ks[6] = {1, 3, 5, 6, 7, 8};
-#pragma unroll
-            for (int n = 0; n < 6; n++)
-              *reinterpret_cast<float4*>(a.side_dst + (long long)n * a.pitch + xg) =
-                  make_float4(out[0][ks[n]], out[1][ks[n]], out[2][ks[n]], out[3][ks[n]]);
-          }
-#define LBM_TB2_PUSH(dst, depth, k)                                                             \
-  *reinterpret_cast<float4*>((dst) + (long long)((depth) * 9 + (k)) * a.pitch + xg) =          \
-      make_float4(out[0][k], out[1][k], out[2][k], out[3][k]);
-          if (first) {
-            LBM_TB2_PUSH(a.push_dn, 0, 4) LBM_TB2_PUSH(a.push_dn, 0, 7) LBM_TB2_PUSH(a.push_dn, 0, 8)
-            LBM_TB2_PUSH(a.push_dn, 0, 0) LBM_TB2_PUSH(a.push_dn, 0, 1) LBM_TB2_PUSH(a.push_dn, 0, 3)
-          }
-          if (last) {
-            LBM_TB2_PUSH(a.push_up, 0, 2) LBM_TB2_PUSH(a.push_up, 0, 5) LBM_TB2_PUSH(a.push_up, 0, 6)
-            LBM_TB2_PUSH(a.push_up, 0, 0) LBM_TB2_PUSH(a.push_up, 0, 1) LBM_TB2_PUSH(a.push_up, 0, 3)
-          }
-          if (second) { LBM_TB2_PUSH(a.push_dn, 1, 4) LBM_TB2_PUSH(a.push_dn, 1, 7) LBM_TB2_PUSH(a.push_dn, 1, 8) }
-          if (before_last) { LBM_TB2_PUSH(a.push_up, 1, 2) LBM_TB2_PUSH(a.push_up, 1, 5) LBM_TB2_PUSH(a.push_up, 1, 6) }
-#undef LBM_TB2_PUSH
-        }
+        tb2_store_row<STRICT>(a, y, xg, out, mbits_prev);
       }
     }
     else {

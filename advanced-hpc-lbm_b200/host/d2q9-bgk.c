@@ -12,7 +12,7 @@
  *   LBM_PRECISION=f64      run the double-precision validation kernel (the golden files
  *                          in check/ were produced by a double build of the reference)
  *   LBM_STRICT=1           source operation order, no FMA contraction
- *   LBM_KERNEL=scalar|vec4|persistent|tma|cluster|tb2|pairs   force a kernel variant
+ *   LBM_KERNEL=scalar|vec4|persistent|tma|cluster|tb2|tb3|pairs   force a kernel variant
  *   LBM_SKIP_FINAL_STATE=1 do not write final_state.dat (huge synthetic grids: 16384^2
  *                          would be 24 GB of text)
  *   LBM_REPORT=1           print MLUPS / GB/s / device time after the contract lines
@@ -77,8 +77,9 @@ int main(int argc, char* argv[])
     else if (strcmp(kv, "tma") == 0) flags |= LBM_GPU_KERNEL_TMA;
     else if (strcmp(kv, "cluster") == 0) flags |= LBM_GPU_KERNEL_CLUSTER;
     else if (strcmp(kv, "tb2") == 0) flags |= LBM_GPU_KERNEL_TB2;
+    else if (strcmp(kv, "tb3") == 0) flags |= LBM_GPU_KERNEL_TB3;
     else if (strcmp(kv, "pairs") == 0) flags |= LBM_GPU_KERNEL_PAIRS;
-    else die("LBM_KERNEL must be scalar, vec4, persistent, tma, cluster, tb2 or pairs", __LINE__, __FILE__);
+    else die("LBM_KERNEL must be scalar, vec4, persistent, tma, cluster, tb2, tb3 or pairs", __LINE__, __FILE__);
   }
 
   /* Total/init time starts here: load values from file, build the device lattice */

@@ -86,6 +86,11 @@ typedef struct lbm_gpu lbm_gpu;   /* opaque handle: one lattice on one or more G
 #define LBM_GPU_KERNEL_PAIRS 2048u  /* force the small-grid persistent kernel that meets at a grid barrier once
                                       per TWO timesteps (single GPU, fp32, nx a multiple of 4 and <= 256); the
                                       default for such grids */
+#define LBM_GPU_KERNEL_TB3  4096u  /* force the three-timesteps-per-pass kernel (each distribution crosses
+                                      HBM once per THREE timesteps; fp32, nx a multiple of 4 and >= 32, the
+                                      whole grid on one GPU, at least 12 rows).  The default for such grids
+                                      that are large enough (otherwise LBM_GPU_KERNEL_TB2 is); the last one
+                                      or two steps of a run are done by the one- or two-step kernel */
 #define LBM_GPU_SYNC_EVENTS 1024u  /* lbm_gpu_create with n_gpus > 1: order the slabs with CUDA events
                                       (host-recorded, no device-side waiting) even when every slab has its
                                       own GPU; always used when slabs share a GPU */

@@ -20,6 +20,8 @@ VARIANTS = {
     "barrier0": ["-DLBM_BARRIER_MODE=0"],
     "tb2_t128": ["-DLBM_TB2_THREADS=128", "-DLBM_TB2_MIN_BLOCKS=3"],
     "tb2_t64": ["-DLBM_TB2_THREADS=64", "-DLBM_TB2_MIN_BLOCKS=6"],
+    "tb3_t64": ["-DLBM_TB2_THREADS=64", "-DLBM_TB3_MIN_BLOCKS=4"],     # K10, 64-thread strips (profiles/r03_k10.md)
+    "tb3_mb2": ["-DLBM_TB3_MIN_BLOCKS=2"],                              # K10, 186 registers, 6 warps per SM
 }
 if os.environ.get("LBM_VARIANTS"):
     VARIANTS = {k: v for k, v in VARIANTS.items() if k in os.environ["LBM_VARIANTS"].split(",")}

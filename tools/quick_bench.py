@@ -22,7 +22,7 @@ ap.add_argument("--f64", action="store_true")
 ap.add_argument("--sync-flags", action="store_true", help="in-process multi-GPU ordered by device flags")
 a = ap.parse_args()
 flags = {"auto": 0, "scalar": L.KERNEL_SCALAR, "vec4": L.KERNEL_VEC4, "tma": L.KERNEL_TMA, "persistent": L.KERNEL_PERSISTENT, "cluster": L.KERNEL_CLUSTER,
-         "tb2": L.KERNEL_TB2, "pairs": L.KERNEL_PAIRS}[a.kernel]
+         "tb2": L.KERNEL_TB2, "tb3": L.KERNEL_TB3, "pairs": L.KERNEL_PAIRS}[a.kernel]
 if a.sync_flags:
     flags |= L.SYNC_FLAGS
 t0 = time.time()
