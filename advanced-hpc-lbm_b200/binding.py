@@ -74,6 +74,7 @@ SYMBOLS = {
     "lbm_gpu_run": (C.c_int, [_P, C.c_int, _P]),
     "lbm_gpu_run_f64": (C.c_int, [_P, C.c_int, _P]),
     "lbm_gpu_run_sums": (C.c_int, [_P, C.c_int, _P]),
+    "lbm_gpu_run_batch": (C.c_int, [_P, C.c_int, C.c_int, _P]),
     "lbm_gpu_set_global_free_cells": (C.c_int, [_P, C.c_longlong]),
     "lbm_gpu_download": (C.c_int, [_P, _P]),
     "lbm_gpu_download_rows": (C.c_int, [_P, C.c_longlong, C.c_longlong, _P]),
@@ -319,3 +320,15 @@ class Lattice:
             self.close()
         except Exception:
             pass
+
+
+def run_batch(lattices, n_steps):
+    """Advance every Lattice of `lattices` by n_steps in one batch on the GPU (parameter
+    sweeps; lbm_gpu_run_batch).  Returns the av_vels of each, shape (n, n_steps) float32:
+    the same bits as lat.run(n_steps) on each in turn."""
+    lib = load_library()
+    lattices = list(lattices)
+    handles = (C.c_void_p * max(len(lattices), 1))(*[lat.h.value for lat in lattices])
+    av = np.empty((len(lattices), max(int(n_steps), 0)), dtype=np.float32)
+    _check(lib.lbm_gpu_run_batch(C.cast(handles, C.c_void_p), len(lattices), int(n_steps), _ptr(av)))
+    return av

@@ -1029,20 +1029,24 @@ class Grid : public GridBase {
     cur ^= 1;
   }
 
+  // room for the per-step sums of n_steps steps (the caller zeroes them)
+  void reserve_av(Slab<real>& s, int n_steps) {
+    if (s.av_cap >= (size_t)n_steps) return;
+    pool_free(s.av, s);
+    s.av = nullptr;
+    s.av_cap = std::max<size_t>((size_t)n_steps, 1024);
+    void* av = nullptr;
+    pool_alloc(&av, s.av_cap * (kAvWords + 2) * sizeof(unsigned long long), s);
+    s.av = (unsigned long long*)av;
+    s.av_compact = s.av + s.av_cap * kAvWords;      // {low, high} per step, filled after the run
+  }
+
   void run_segment(int n_steps, double* sums_out) {
     if (n_steps <= 0) return;
     const bool strict = (flags & LBM_GPU_STRICT) != 0;
     for (auto& s : slabs) {
       CK(cudaSetDevice(s.device));
-      if (s.av_cap < (size_t)n_steps) {
-        pool_free(s.av, s);
-        s.av = nullptr;
-        s.av_cap = std::max<size_t>((size_t)n_steps, 1024);
-        void* av = nullptr;
-        pool_alloc(&av, s.av_cap * (kAvWords + 2) * sizeof(unsigned long long), s);
-        s.av = (unsigned long long*)av;
-        s.av_compact = s.av + s.av_cap * kAvWords;      // {low, high} per step, filled after the run
-      }
+      reserve_av(s, n_steps);
       CK(cudaMemsetAsync(s.av, 0, (size_t)n_steps * kAvWords * sizeof(unsigned long long), s.stream));
     }
     for (auto& s : slabs) { CK(cudaSetDevice(s.device)); CK(cudaEventRecord(s.ev0, s.stream)); }
@@ -1137,28 +1141,31 @@ class Grid : public GridBase {
     steps_done += n_steps;
     if (use_flags) check_sync_errors();
     if (kernel == LBM_GPU_KERNEL_CLUSTER) prepare();      // side row + ghost rows of the new state
+    if (sums_out) read_sums(n_steps, sums_out);
+  }
 
-    if (sums_out) {
-      std::vector<unsigned long long> words((size_t)n_steps * 2);
-      std::vector<unsigned __int128> tot(n_steps, 0);
-      std::vector<char> bad(n_steps, 0);
-      for (auto& s : slabs) {
-        CK(cudaSetDevice(s.device));
-        lbm::lbm_compact_av<<<(n_steps + 255) / 256, 256, 0, s.stream>>>(s.av, s.av_compact, n_steps);
-        CK(cudaGetLastError());
-        launches++;
-        CK(cudaMemcpyAsync(words.data(), s.av_compact, words.size() * sizeof(unsigned long long),
-                           cudaMemcpyDeviceToHost, s.stream));
-        CK(cudaStreamSynchronize(s.stream));
-        for (int t = 0; t < n_steps; t++) {
-          const unsigned long long lo = words[2 * (size_t)t], hi = words[2 * (size_t)t + 1];
-          if (hi & LBM_NONFINITE_MARK) bad[t] = 1;
-          tot[t] += ((unsigned __int128)(hi & ~LBM_NONFINITE_MARK) << 32) + lo;
-        }
+  // The per-step sums of the last n_steps steps (device words -> exact 128-bit totals ->
+  // double; NaN for a step that met a non-finite cell).  After the steps have finished.
+  void read_sums(int n_steps, double* sums_out) {
+    std::vector<unsigned long long> words((size_t)n_steps * 2);
+    std::vector<unsigned __int128> tot(n_steps, 0);
+    std::vector<char> bad(n_steps, 0);
+    for (auto& s : slabs) {
+      CK(cudaSetDevice(s.device));
+      lbm::lbm_compact_av<<<(n_steps + 255) / 256, 256, 0, s.stream>>>(s.av, s.av_compact, n_steps);
+      CK(cudaGetLastError());
+      launches++;
+      CK(cudaMemcpyAsync(words.data(), s.av_compact, words.size() * sizeof(unsigned long long),
+                         cudaMemcpyDeviceToHost, s.stream));
+      CK(cudaStreamSynchronize(s.stream));
+      for (int t = 0; t < n_steps; t++) {
+        const unsigned long long lo = words[2 * (size_t)t], hi = words[2 * (size_t)t + 1];
+        if (hi & LBM_NONFINITE_MARK) bad[t] = 1;
+        tot[t] += ((unsigned __int128)(hi & ~LBM_NONFINITE_MARK) << 32) + lo;
       }
-      for (int t = 0; t < n_steps; t++)
-        sums_out[t] = bad[t] ? std::nan("") : (double)((long double)tot[t] / (long double)LBM_FIX_SCALE);
     }
+    for (int t = 0; t < n_steps; t++)
+      sums_out[t] = bad[t] ? std::nan("") : (double)((long double)tot[t] / (long double)LBM_FIX_SCALE);
   }
 
   // The flag protocol gave up (see boundary_wait): say why, in the reference's die() spirit.
@@ -1418,6 +1425,245 @@ int run_impl(lbm_gpu* h, int n_steps, real* av_out, double* sums_out, const char
   });
 }
 
+// ----------------------------------------------------------------- batches (K11) ----
+// lbm_gpu_run_batch: many K9 lattices of one shape advanced by one kernel, blockIdx.y = member.
+constexpr int kBatchMaxTileRows = 32;
+// Cost model of one K11 launch per pair of timesteps, fitted to the tile sweep at 128^2
+// (profiles/r04_batch.md): a fixed part (barrier, launch share) plus the larger of
+//   latency     loop iterations of a thread row x one dependent L2 round trip, which grows with
+//               the warps of a block that meet at its __syncthreads, and
+//   throughput  warp-iterations the busiest SM has to issue.
+constexpr double kBatchFixedNs = 2100.0, kBatchIterNs = 500.0, kBatchIterPerWarpNs = 70.0, kBatchWarpIterNs = 100.0;
+
+struct BatchShape {
+  int tile_rows = 0, thread_rows = 0, blocks_per_member = 0, members_per_launch = 0;
+  size_t smem = 0;
+};
+
+const void* batch_fn(bool strict) {
+  return strict ? (const void*)lbm::lbm_steps_pairs_batch<true> : (const void*)lbm::lbm_steps_pairs_batch<false>;
+}
+
+// Tile rows H and thread rows T of K11 for n members of nx x rows.  A launch holds as many
+// members as have all their blocks resident at once (cooperative launch); bigger batches take
+// several launches.  Every (H, T) whose blocks fit is scored with the cost model above and the
+// cheapest wins; ties go to fewer launches, then to taller tiles (fewer halo rows recomputed).
+BatchShape batch_shape(int device, int nx, int rows, bool strict, int n) {
+  struct Entry { int device, nx, rows, n; bool strict; BatchShape shape; };
+  static std::mutex mu;
+  static std::vector<Entry> cache;
+  std::lock_guard<std::mutex> lock(mu);
+  for (const Entry& e : cache)
+    if (e.device == device && e.nx == nx && e.rows == rows && e.n == n && e.strict == strict) return e.shape;
+  int sms = 0, coop = 0, max_smem = 0;
+  CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+  CK(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device));
+  CK(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+  if (!coop) throw CudaError{"cooperative launch is not available on this device"};
+  const void* fn = batch_fn(strict);
+  cudaFuncAttributes fa;
+  CK(cudaFuncGetAttributes(&fa, fn));
+  const int max_dyn = max_smem - (int)fa.sharedSizeBytes;     // the block's table entry is static shared memory
+  CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, max_dyn));
+  CK(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+  const int bx = (int)round_up(nx / 4, 32), wpr = bx / 32;
+  const int h_knob = getenv("LBM_BATCH_TILE_ROWS") ? atoi(getenv("LBM_BATCH_TILE_ROWS")) : 0;     // tuning knobs
+  const int t_knob = getenv("LBM_BATCH_THREAD_ROWS") ? atoi(getenv("LBM_BATCH_THREAD_ROWS")) : 0;
+  BatchShape best;
+  double best_cost = 0.0;
+  long long best_launches = 0;
+  for (int H = 1; H <= std::min(kBatchMaxTileRows, rows - 2); H++) {
+    if (h_knob > 0 && H != h_knob) continue;
+    const size_t smem = (size_t)(H + 2) * 9 * nx * sizeof(float);
+    if (smem > (size_t)max_dyn) break;
+    const int bpm = (rows + H - 1) / H;
+    for (int T = 1; T <= H + 2 && bx * T <= LBM_BATCH_MAX_THREADS; T++) {
+      if (t_knob > 0 && T != t_knob) continue;
+      int per_sm = 0;
+      CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, bx * T, smem));
+      const long long fit = (long long)per_sm * sms / bpm;
+      if (fit < 1) continue;
+      const long long launches = (n + fit - 1) / fit;
+      const long long members = (n + launches - 1) / launches;
+      const long long blocks_on_sm = (members * bpm + sms - 1) / sms;
+      const int iters = (H + 2 + T - 1) / T + (H + T - 1) / T;
+      const double latency = iters * (kBatchIterNs + kBatchIterPerWarpNs * T * wpr);
+      const double issue = (double)(blocks_on_sm * T * wpr * iters) * kBatchWarpIterNs;
+      const double cost = (double)launches * (kBatchFixedNs + std::max(latency, issue));
+      const bool better = best.tile_rows == 0 || cost < best_cost - 1e-6 ||
+                          (cost < best_cost + 1e-6 && (launches < best_launches ||
+                                                       (launches == best_launches && H > best.tile_rows)));
+      if (better) {
+        best.tile_rows = H;
+        best.thread_rows = T;
+        best.blocks_per_member = bpm;
+        best.members_per_launch = (int)members;
+        best.smem = smem;
+        best_cost = cost;
+        best_launches = launches;
+      }
+    }
+  }
+  if (best.tile_rows == 0) throw CudaError{"no tile shape of the batch kernel keeps one member's blocks resident"};
+  if (getenv("LBM_BATCH_VERBOSE") && getenv("LBM_BATCH_VERBOSE")[0] == '1')     // measurement aid
+    fprintf(stderr, "lbm_gpu_run_batch: %d x %d, %d members: tile_rows %d, thread_rows %d, %d members per launch\n",
+            nx, rows, n, best.tile_rows, best.thread_rows, best.members_per_launch);
+  cache.push_back({device, nx, rows, n, strict, best});
+  return best;
+}
+
+// One segment (at most kMaxSegmentSteps steps) of every member, in order on the first
+// member's stream; the other members' streams are ordered before and after it with events
+// (each single-slab member's step_ev[], which only multi-slab handles use otherwise).
+// Returns the device time; sums[i] (or NULL) receives member i's raw per-step sums.
+double run_batch_segment(const std::vector<Grid<float>*>& gs, const BatchShape& shape, int n_steps,
+                         const std::vector<double*>& sums) {
+  const int n = (int)gs.size();
+  Grid<float>& g0 = *gs[0];
+  Slab<float>& s0 = g0.slabs[0];
+  CK(cudaSetDevice(s0.device));
+  const cudaStream_t st = s0.stream;
+  for (Grid<float>* g : gs) g->reserve_av(g->slabs[0], n_steps);
+  for (int i = 1; i < n; i++) {
+    Slab<float>& s = gs[i]->slabs[0];
+    CK(cudaEventRecord(s.step_ev[0], s.stream));
+    CK(cudaStreamWaitEvent(st, s.step_ev[0], 0));
+  }
+  CK(cudaEventRecord(s0.ev0, st));
+  for (Grid<float>* g : gs) {
+    Slab<float>& s = g->slabs[0];
+    CK(cudaMemsetAsync(s.av, 0, (size_t)n_steps * kAvWords * sizeof(unsigned long long), st));
+  }
+  const int n_pairs = n_steps / 2;
+  if (n_pairs > 0) {
+    // the member table goes to the first member's staging buffer (idle during runs)
+    std::vector<lbm::BatchMember> table(n);
+    for (int i = 0; i < n; i++) {
+      Grid<float>& g = *gs[i];
+      Slab<float>& s = g.slabs[0];
+      lbm::StepArgs<float> a;
+      g.fill_step_args(a, s, 0);
+      lbm::BatchMember& m = table[i];
+      for (int b = 0; b < 2; b++) { m.lattice[b] = s.lattice[b]; m.side[b] = s.side[b]; }
+      m.window = (float*)s.win;
+      m.mask = s.mask;
+      m.av = s.av;
+      m.barrier = s.sync + kGridBarrier;
+      m.first_parity = g.cur;
+      m.omega = a.omega;
+      m.aw1 = a.aw1;
+      m.aw2 = a.aw2;
+      CK(cudaMemsetAsync(m.barrier, 0, sizeof(unsigned long long), st));
+    }
+    lbm::BatchMember* dtable = (lbm::BatchMember*)s0.staging;
+    CK(cudaMemcpyAsync(dtable, table.data(), table.size() * sizeof(lbm::BatchMember), cudaMemcpyHostToDevice, st));
+    lbm::BatchArgs ba;
+    memset(&ba, 0, sizeof ba);
+    g0.fill_step_args(ba.s, s0, 0);          // geometry; every pointer and constant is the member's
+    ba.n_pairs = n_pairs;
+    ba.tile_rows = shape.tile_rows;
+    const dim3 block((unsigned)round_up(g0.prm.nx / 4, 32), (unsigned)shape.thread_rows);
+    const bool strict = (g0.flags & LBM_GPU_STRICT) != 0;
+    for (int first = 0; first < n; first += shape.members_per_launch) {
+      const int count = std::min(shape.members_per_launch, n - first);
+      ba.members = dtable + first;
+      void* kargs[] = {(void*)&ba};
+      CK(cudaLaunchCooperativeKernel(batch_fn(strict), dim3((unsigned)shape.blocks_per_member, (unsigned)count), block,
+                                     kargs, shape.smem, st));
+    }
+    for (Grid<float>* g : gs) {
+      g->launches++;                          // the launch that held its blocks
+      g->cur = (g->cur + n_pairs) & 1;
+      g->passes_done += n_pairs;
+    }
+  }
+  if (n_steps & 1) {
+    // the odd last step: each member's one-step pass (K1a) on its own stream, as run_segment does
+    CK(cudaEventRecord(s0.step_ev[1], st));
+    for (int i = 0; i < n; i++) {
+      Slab<float>& s = gs[i]->slabs[0];
+      if (i > 0) CK(cudaStreamWaitEvent(s.stream, s0.step_ev[1], 0));
+      gs[i]->launch_pass(n_steps - 1, 0, 1);
+      if (i > 0) {
+        CK(cudaEventRecord(s.step_ev[1], s.stream));
+        CK(cudaStreamWaitEvent(st, s.step_ev[1], 0));
+      }
+    }
+  }
+  CK(cudaEventRecord(s0.ev1, st));
+  CK(cudaEventRecord(s0.step_ev[0], st));
+  for (int i = 1; i < n; i++) CK(cudaStreamWaitEvent(gs[i]->slabs[0].stream, s0.step_ev[0], 0));
+  CK(cudaStreamSynchronize(st));
+  float ms = 0.f;
+  CK(cudaEventElapsedTime(&ms, s0.ev0, s0.ev1));
+  for (int i = 0; i < n; i++) {
+    gs[i]->steps_done += n_steps;
+    if (sums[i]) gs[i]->read_sums(n_steps, sums[i]);
+  }
+  return ms;
+}
+
+int run_batch_impl(lbm_gpu* const* handles, int n, int n_steps, float* av_out) {
+  const char* fn = "lbm_gpu_run_batch";
+  if (!handles) return fail("%s: NULL handle array", fn);
+  if (n < 1) return fail("%s: need at least one member (n = %d)", fn, n);
+  if (n_steps < 0) return fail("%s: negative step count", fn);
+  std::vector<Grid<float>*> gs(n);
+  for (int i = 0; i < n; i++) {
+    if (!handles[i]) return fail("%s: member %d is a NULL handle", fn, i);
+    for (int j = 0; j < i; j++)
+      if (handles[j] == handles[i]) return fail("%s: members %d and %d are the same handle (duplicate)", fn, j, i);
+    GridBase* b = reinterpret_cast<GridBase*>(handles[i]);
+    if (b->is_f64()) return fail("%s: member %d is double precision; batches run fp32 lattices only", fn, i);
+    Grid<float>& g = *static_cast<Grid<float>*>(b);
+    if (g.slab_mode) return fail("%s: member %d is a slab handle (lbm_gpu_create_slab); members must be single-slab lattices", fn, i);
+    if (g.slabs.size() != 1)
+      return fail("%s: member %d is split into %d slabs; members must be single-slab lattices", fn, i, (int)g.slabs.size());
+    if (g.failed) return fail("%s: member %d is failed (an earlier run was abandoned)", fn, i);
+    if (g.kernel != LBM_GPU_KERNEL_PAIRS)
+      return fail("%s: member %d does not run the pairs kernel (LBM_GPU_KERNEL_PAIRS), the only one batched", fn, i);
+    gs[i] = &g;
+    const Grid<float>& g0 = *gs[0];
+    if (g.slabs[0].device != g0.slabs[0].device)
+      return fail("%s: member %d is on device %d and member 0 on device %d; members must share one device", fn, i,
+                  g.slabs[0].device, g0.slabs[0].device);
+    if (g.prm.nx != g0.prm.nx || g.prm.ny != g0.prm.ny)
+      return fail("%s: member %d is %d x %d and member 0 is %d x %d; members must have the same nx and ny", fn, i,
+                  g.prm.nx, g.prm.ny, g0.prm.nx, g0.prm.ny);
+    if ((g.flags & LBM_GPU_STRICT) != (g0.flags & LBM_GPU_STRICT))
+      return fail("%s: member %d and member 0 differ in LBM_GPU_STRICT; members must share it", fn, i);
+  }
+  try {
+    Grid<float>& g0 = *gs[0];
+    CK(cudaSetDevice(g0.slabs[0].device));
+    const BatchShape shape = batch_shape(g0.slabs[0].device, g0.prm.nx, g0.slabs[0].rows,
+                                         (g0.flags & LBM_GPU_STRICT) != 0, n);
+    std::vector<double> sums(av_out ? (size_t)n * n_steps : 0);
+    std::vector<double*> at(n, nullptr);
+    double ms = 0.0;
+    for (int done = 0; done < n_steps; done += kMaxSegmentSteps) {
+      const int seg = std::min(kMaxSegmentSteps, n_steps - done);
+      for (int i = 0; i < n && av_out; i++) at[i] = sums.data() + (size_t)i * n_steps + done;
+      ms += run_batch_segment(gs, shape, seg, at);
+    }
+    if (n_steps > 0)
+      for (Grid<float>* g : gs) {
+        g->last_run_ms = ms;
+        g->last_step_ms = ms / n_steps;
+      }
+    if (av_out)
+      for (int i = 0; i < n; i++) {
+        const double div = (double)gs[i]->divisor();
+        for (int t = 0; t < n_steps; t++) av_out[(size_t)i * n_steps + t] = (float)(sums[(size_t)i * n_steps + t] / div);
+      }
+  } catch (const CudaError& e) {
+    return fail("%s: %s", fn, e.what.c_str());
+  } catch (const std::exception& e) {
+    return fail("%s: %s", fn, e.what());
+  }
+  return 0;
+}
+
 }  // namespace
 
 // ======================================================================= C-ABI ====
@@ -1644,6 +1890,9 @@ int lbm_gpu_run(lbm_gpu* h, int n_steps, float* av_vels_out) {
 }
 int lbm_gpu_run_f64(lbm_gpu* h, int n_steps, double* av_vels_out) {
   return run_impl<double>(h, n_steps, av_vels_out, nullptr, "lbm_gpu_run_f64");
+}
+int lbm_gpu_run_batch(lbm_gpu* const* handles, int n, int n_steps, float* av_vels_out) {
+  return run_batch_impl(handles, n, n_steps, av_vels_out);
 }
 int lbm_gpu_run_sums(lbm_gpu* h, int n_steps, double* sums_out) {
   if (!h) return fail("lbm_gpu_run_sums: NULL handle");

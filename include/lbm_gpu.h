@@ -193,6 +193,22 @@ int lbm_gpu_run_sums(lbm_gpu* h, int n_steps, double* sums_out);
 int lbm_gpu_set_global_free_cells(lbm_gpu* h, long long free_cells);
 
 /*
+ * Parameter sweeps: advance n independent lattices by n_steps each, together on one GPU.
+ * Same result, bit for bit, as calling lbm_gpu_run(handles[i], n_steps, av_vels_out + i*n_steps)
+ * for i = 0..n-1 in turn; a small lattice leaves most of the GPU idle, so running many in
+ * one kernel costs little more than running one.  av_vels_out: n * n_steps floats,
+ * member-major, may be NULL.
+ * Members are ordinary handles from lbm_gpu_create.  They must share the device, nx, ny and
+ * the LBM_GPU_STRICT setting, and each must be fp32, a single slab, not failed, and run
+ * LBM_GPU_KERNEL_PAIRS (the default for fp32 grids with nx a multiple of 4 and <= 256).
+ * They may differ in density, accel, omega, obstacles, contents and history (steps done).
+ * Otherwise the call is refused before anything runs (no handle changes), as it is for
+ * n < 1, a NULL or duplicate handle, or n_steps < 0.  Afterwards each member is exactly
+ * where lbm_gpu_run would have left it; its last_run_device_ms is the whole batch's time.
+ */
+int lbm_gpu_run_batch(lbm_gpu* const* handles, int n, int n_steps, float* av_vels_out);
+
+/*
  * The reference keeps the lattice on the host, so calc_reynolds (d2q9-bgk.c:2893) and
  * write_values (d2q9-bgk.c:2918) read it directly.  Here the host asks for it:
  *   download        whole local lattice, AoS like t_speed (9 floats per cell)
