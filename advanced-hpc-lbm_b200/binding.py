@@ -29,6 +29,7 @@ KERNEL_TB2 = 512
 SYNC_EVENTS = 1024
 KERNEL_PAIRS = 2048
 KERNEL_TB3 = 4096
+STORE_F16 = 8192
 IPC_DESC_BYTES = 256
 
 

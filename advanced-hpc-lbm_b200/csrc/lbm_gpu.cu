@@ -9,6 +9,7 @@
 #include "lbm_tb2.cuh"
 #include "lbm_tb3.cuh"
 #include "lbm_pairs.cuh"
+#include "lbm_f16.cuh"
 
 #include <unistd.h>
 
@@ -177,6 +178,7 @@ class Grid : public GridBase {
   bool tb3 = false;            // three timesteps per pass (K10) wherever three steps remain (K7 for two, K1a for one)
   int tb3_seg_rows = 0;        // K10: rows per segment
   int pairs_tile_rows = 0;     // K9: rows per block
+  bool f16 = false;            // LBM_GPU_STORE_F16: the lattice buffers hold shifted binary16 (lbm_f16.cuh)
   bool failed = false;         // a neighbour never arrived: the lattice contents are void
   unsigned long long timeout_ns = 10000000000ULL;
   long long launches = 0;
@@ -269,7 +271,7 @@ class Grid : public GridBase {
   void alloc_slab(Slab<real>& s) {
     CK(cudaSetDevice(s.device));
     const long long plane = (long long)s.rows * pitch;
-    const size_t lat = (size_t)9 * plane * sizeof(real);
+    const size_t lat = (size_t)9 * plane * (f16 ? sizeof(__half) : sizeof(real));
     const size_t side = (size_t)6 * pitch * sizeof(real);
     const size_t maskb = (size_t)s.rows * mask_pitch * sizeof(uint32_t);
     size_t off = 0;
@@ -340,6 +342,17 @@ class Grid : public GridBase {
   real* win_section(char* win, int b, int d) const { return (real*)win + lbm::ghost_offset(pitch, b, d); }
 
   long long plane_stride(const Slab<real>& s) const { return (long long)s.rows * pitch; }
+
+  // LBM_GPU_STORE_F16: the binary16 view of a lattice buffer, and the shift of each speed
+  // (the rest state, computed as load_slab computes it)
+  __half* hlat(const Slab<real>& s, int b) const { return reinterpret_cast<__half*>(s.lattice[b]); }
+  lbm::RestShift rest() const {
+    lbm::RestShift r;
+    r.w0 = (float)(prm.density * (real)4 / (real)9);
+    r.w1 = (float)(prm.density / (real)9);
+    r.w2 = (float)(prm.density / (real)36);
+    return r;
+  }
 
   void setup_geometry(int nx) {
     pitch = (int)round_up(nx, 32);
@@ -488,17 +501,24 @@ class Grid : public GridBase {
     if constexpr (sizeof(real) == 4) {
       for (auto& s : slabs) {
         CK(cudaSetDevice(s.device));
+        if (f16) {
+          for (const void* fn : {(const void*)lbm::lbm_step2_tb_f16<false>, (const void*)lbm::lbm_step2_tb_f16<true>})
+            CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(lbm::Tb2hSmem)));
+          continue;
+        }
         for (const void* fn : {(const void*)lbm::lbm_step2_tb<false, false>, (const void*)lbm::lbm_step2_tb<false, true>,
                                (const void*)lbm::lbm_step2_tb<true, false>, (const void*)lbm::lbm_step2_tb<true, true>})
           CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(lbm::Tb2Smem)));
       }
-      if (prm.nx + 2 * LBM_TB2_PAD <= LBM_TB2_SPAN) {      // narrow grid: one strip, the whole width plus halo
+      // K7-f16 has a halo of 8 columns and owns multiples of 8 (16-byte bulk copies of binary16)
+      const int pad = f16 ? LBM_TB2H_PAD : LBM_TB2_PAD, max_wout = f16 ? LBM_TB2H_MAX_WOUT : LBM_TB2_MAX_WOUT;
+      if (prm.nx + 2 * pad <= LBM_TB2_SPAN) {      // narrow grid: one strip, the whole width plus halo
         tb2_strips = 1;
         tb2_wout = prm.nx;
-        tb2_span = prm.nx + 2 * LBM_TB2_PAD;
+        tb2_span = prm.nx + 2 * pad;
       } else {
-        tb2_strips = (prm.nx + LBM_TB2_MAX_WOUT - 1) / LBM_TB2_MAX_WOUT;
-        tb2_wout = (int)round_up((prm.nx + tb2_strips - 1) / tb2_strips, 4);
+        tb2_strips = (prm.nx + max_wout - 1) / max_wout;
+        tb2_wout = (int)round_up((prm.nx + tb2_strips - 1) / tb2_strips, f16 ? 8 : 4);
         tb2_span = LBM_TB2_SPAN;
       }
       tb2_threads = (int)round_up(tb2_span / 4, 32);
@@ -648,6 +668,16 @@ class Grid : public GridBase {
                                    "blocks are all resident"};
   }
 
+  // LBM_GPU_STORE_F16 (one slab, fp32): K7-f16 where K7's shape rules hold and the binary16 bulk copies
+  // can cut the rows (nx a multiple of 8), otherwise K1a-f16; LBM_GPU_KERNEL_VEC4 forces K1a-f16
+  void choose_f16() {
+    const bool tb2_ok = prm.nx % 8 == 0 && prm.nx >= 32 && slabs[0].rows >= kTb2MinRows;
+    if ((flags & LBM_GPU_KERNEL_TB2) && !tb2_ok)
+      throw CudaError{"the two-step kernel with LBM_GPU_STORE_F16 needs nx a multiple of 8 and >= 32, and >= 8 rows"};
+    kernel = LBM_GPU_KERNEL_VEC4;
+    if (tb2_ok && !(flags & LBM_GPU_KERNEL_VEC4)) enable_tb2();
+  }
+
   // single-process form: decide once all slabs exist
   void choose_tb2() {
     int rows_min = slabs[0].rows;
@@ -670,6 +700,8 @@ class Grid : public GridBase {
     const int nx = prm.nx;
     if (cells_aos) {
       upload_cells(s, cells_aos, cur);
+    } else if (f16) {
+      CK(cudaMemsetAsync(s.lattice[cur], 0, (size_t)9 * plane_stride(s) * sizeof(__half), s.stream));   // the rest state
     } else {
       const real w0 = prm.density * (real)4 / (real)9;     // d2q9-bgk.c:2802-2804
       const real w1 = prm.density / (real)9;
@@ -736,8 +768,12 @@ class Grid : public GridBase {
       const long long ncells = (long long)n * nx;
       CK(cudaMemcpyAsync(s.staging, (const char*)cells_aos + (size_t)r * row_bytes, (size_t)n * row_bytes,
                          cudaMemcpyHostToDevice, s.stream));
-      lbm::lbm_aos_to_soa<real><<<(unsigned)((ncells * 9 + 255) / 256), 256, 0, s.stream>>>(
-          (const real*)s.staging, s.lattice[cur], plane_stride(s), pitch, nx, r, ncells);
+      if (f16)
+        lbm::lbm_aos_to_soa<real, __half><<<(unsigned)((ncells * 9 + 255) / 256), 256, 0, s.stream>>>(
+            (const real*)s.staging, hlat(s, cur), plane_stride(s), pitch, nx, r, ncells, rest());
+      else
+        lbm::lbm_aos_to_soa<real><<<(unsigned)((ncells * 9 + 255) / 256), 256, 0, s.stream>>>(
+            (const real*)s.staging, s.lattice[cur], plane_stride(s), pitch, nx, r, ncells);
       CK(cudaGetLastError());
       launches++;
       CK(cudaStreamSynchronize(s.stream));
@@ -790,6 +826,17 @@ class Grid : public GridBase {
 
   void prepare() {
     if (!connected) throw CudaError{"lattice is not connected to its neighbours yet"};
+    if (f16) {            // one slab that holds the whole grid: no ghost rows, only the side row
+      Slab<real>& s = slabs[0];
+      CK(cudaSetDevice(s.device));
+      lbm::lbm_prepare_f16<<<(prm.nx + 127) / 128, 128, 0, s.stream>>>(
+          hlat(s, cur), (float*)s.side[cur], s.mask, plane_stride(s), prm.nx, pitch, mask_pitch, s.accel_row, rest(),
+          (float)(prm.density * prm.accel / (real)9), (float)(prm.density * prm.accel / (real)36));
+      CK(cudaGetLastError());
+      launches++;
+      CK(cudaStreamSynchronize(s.stream));
+      return;
+    }
     for (auto& s : slabs) {
       CK(cudaSetDevice(s.device));
       lbm::PrepareArgs<real> a;
@@ -949,7 +996,54 @@ class Grid : public GridBase {
   }
 
   // one pass over every slab: one timestep (K1a/K1b/K1c), two (K7) or three (K10)
+  // K1a-f16 (one step) or K7-f16 (two) on the single slab of a LBM_GPU_STORE_F16 lattice
+  void launch_pass_f16(int t_in_segment, int steps) {
+    if constexpr (sizeof(real) == 4) {
+      Slab<real>& s = slabs[0];
+      CK(cudaSetDevice(s.device));
+      lbm::F16Args a;
+      memset(&a, 0, sizeof a);
+      a.src = hlat(s, cur);
+      a.dst = hlat(s, cur ^ 1);
+      a.side_src = s.side[cur];
+      a.side_dst = s.side[cur ^ 1];
+      a.mask = s.mask;
+      a.av = s.av + (size_t)t_in_segment * kAvWords;
+      a.av2 = a.av + kAvWords;
+      a.plane_stride = plane_stride(s);
+      a.nx = prm.nx; a.rows = s.rows; a.pitch = pitch; a.mask_pitch = mask_pitch; a.accel_row = s.accel_row;
+      a.omega = prm.omega;
+      a.aw1 = prm.density * prm.accel / 9.f;          // d2q9-bgk.c:230-231
+      a.aw2 = prm.density * prm.accel / 36.f;
+      a.rest = rest();
+      const bool strict = (flags & LBM_GPU_STRICT) != 0;
+      if (steps == 2) {
+        const Tb2Segments sg = tb2_segments(s.rows);
+        a.tiles_x = tb2_strips;
+        a.tiles_y = sg.n_big + sg.n_tail;
+        a.wout = tb2_wout; a.span = tb2_span;
+        a.seg_rows = sg.seg_rows; a.n_big = sg.n_big; a.big_rows = sg.big_rows; a.seg_rows_tail = sg.seg_rows_tail;
+        const dim3 grid((unsigned)((long long)a.tiles_x * a.tiles_y));
+        if (strict) launch_pdl(s, lbm::lbm_step2_tb_f16<true>, a, grid, dim3(tb2_threads), sizeof(lbm::Tb2hSmem));
+        else        launch_pdl(s, lbm::lbm_step2_tb_f16<false>, a, grid, dim3(tb2_threads), sizeof(lbm::Tb2hSmem));
+      } else {
+        int vec, bx, by;
+        tile_shape(vec, bx, by);
+        a.tiles_x = ((prm.nx + 3) / 4 + bx - 1) / bx;
+        a.tiles_y = (s.rows + by - 1) / by;
+        const dim3 grid((unsigned)((long long)a.tiles_x * a.tiles_y)), block(bx, by);
+        if (strict) launch_pdl(s, lbm::lbm_step_vec4_f16<true>, a, grid, block, 0);
+        else        launch_pdl(s, lbm::lbm_step_vec4_f16<false>, a, grid, block, 0);
+      }
+      CK(cudaGetLastError());
+      launches++;
+    }
+    passes_done++;
+    cur ^= 1;
+  }
+
   void launch_pass(int t_in_segment, int pass_in_segment, int steps) {
+    if (f16) { launch_pass_f16(t_in_segment, steps); return; }
     const bool two = (steps == 2);
     const bool strict = (flags & LBM_GPU_STRICT) != 0;
     const int nslabs = (int)slabs.size();
@@ -1215,8 +1309,12 @@ class Grid : public GridBase {
       CK(cudaSetDevice(s.device));
       const int n = (int)std::min<long long>({(long long)chunk_rows, s.row0 + s.rows - g, row0 + nrows - g});
       const long long ncells = (long long)n * nx;
-      lbm::lbm_soa_to_aos<real><<<(unsigned)((ncells * 9 + 255) / 256), 256, 0, s.stream>>>(
-          s.lattice[cur], (real*)s.staging, plane_stride(s), pitch, nx, (int)(g - s.row0), ncells);
+      if (f16)
+        lbm::lbm_soa_to_aos<real, __half><<<(unsigned)((ncells * 9 + 255) / 256), 256, 0, s.stream>>>(
+            hlat(s, cur), (real*)s.staging, plane_stride(s), pitch, nx, (int)(g - s.row0), ncells, rest());
+      else
+        lbm::lbm_soa_to_aos<real><<<(unsigned)((ncells * 9 + 255) / 256), 256, 0, s.stream>>>(
+            s.lattice[cur], (real*)s.staging, plane_stride(s), pitch, nx, (int)(g - s.row0), ncells);
       CK(cudaGetLastError());
       launches++;
       CK(cudaMemcpyAsync((char*)out + (size_t)(g - row0) * row_bytes, s.staging, (size_t)n * row_bytes,
@@ -1254,9 +1352,14 @@ class Grid : public GridBase {
       real* d_u = u ? st + 2 * ncells : nullptr;
       real* d_p = p ? st + 3 * ncells : nullptr;
       if (i >= 2) CK(cudaStreamWaitEvent(s.stream, s.stage_drained[b], 0));
-      lbm::lbm_fields<real><<<(unsigned)((ncells + 255) / 256), 256, 0, s.stream>>>(
-          s.lattice[cur], s.mask, plane_stride(s), pitch, mask_pitch, nx, (int)(g - s.row0), n,
-          prm.density, d_ux, d_uy, d_u, d_p, nullptr);
+      if (f16)
+        lbm::lbm_fields<real, __half><<<(unsigned)((ncells + 255) / 256), 256, 0, s.stream>>>(
+            hlat(s, cur), s.mask, plane_stride(s), pitch, mask_pitch, nx, (int)(g - s.row0), n,
+            prm.density, d_ux, d_uy, d_u, d_p, nullptr, rest());
+      else
+        lbm::lbm_fields<real><<<(unsigned)((ncells + 255) / 256), 256, 0, s.stream>>>(
+            s.lattice[cur], s.mask, plane_stride(s), pitch, mask_pitch, nx, (int)(g - s.row0), n,
+            prm.density, d_ux, d_uy, d_u, d_p, nullptr);
       CK(cudaGetLastError());
       launches++;
       CK(cudaEventRecord(s.stage_filled[b], s.stream));
@@ -1284,9 +1387,14 @@ class Grid : public GridBase {
       unsigned long long* av = s.sync + kAvScratch;       // 128-byte aligned inside the sync block
       CK(cudaMemsetAsync(av, 0, kAvWords * sizeof(unsigned long long), s.stream));
       const long long ncells = (long long)s.rows * prm.nx;
-      lbm::lbm_fields<real><<<(unsigned)((ncells + 255) / 256), 256, 0, s.stream>>>(
-          s.lattice[cur], s.mask, plane_stride(s), pitch, mask_pitch, prm.nx, 0, s.rows, prm.density,
-          nullptr, nullptr, nullptr, nullptr, av);
+      if (f16)
+        lbm::lbm_fields<real, __half><<<(unsigned)((ncells + 255) / 256), 256, 0, s.stream>>>(
+            hlat(s, cur), s.mask, plane_stride(s), pitch, mask_pitch, prm.nx, 0, s.rows, prm.density,
+            nullptr, nullptr, nullptr, nullptr, av, rest());
+      else
+        lbm::lbm_fields<real><<<(unsigned)((ncells + 255) / 256), 256, 0, s.stream>>>(
+            s.lattice[cur], s.mask, plane_stride(s), pitch, mask_pitch, prm.nx, 0, s.rows, prm.density,
+            nullptr, nullptr, nullptr, nullptr, av);
       CK(cudaGetLastError());
       launches++;
       unsigned long long w[kAvWords];
@@ -1306,8 +1414,12 @@ class Grid : public GridBase {
       unsigned long long* out = s.sync + kScratch1;
       CK(cudaMemsetAsync(out, 0, 2 * sizeof(unsigned long long), s.stream));
       const long long ncells = (long long)s.rows * prm.nx;
-      lbm::lbm_digest<real><<<(unsigned)((ncells + 255) / 256), 256, 0, s.stream>>>(
-          s.lattice[cur], plane_stride(s), pitch, prm.nx, 0, s.rows, s.row0, out);
+      if (f16)
+        lbm::lbm_digest<real, __half><<<(unsigned)((ncells + 255) / 256), 256, 0, s.stream>>>(
+            hlat(s, cur), plane_stride(s), pitch, prm.nx, 0, s.rows, s.row0, out, rest());
+      else
+        lbm::lbm_digest<real><<<(unsigned)((ncells + 255) / 256), 256, 0, s.stream>>>(
+            s.lattice[cur], plane_stride(s), pitch, prm.nx, 0, s.rows, s.row0, out);
       CK(cudaGetLastError());
       launches++;
       unsigned long long w[2];
@@ -1342,6 +1454,15 @@ int create_impl(const typename ParamT<real>::type* params, const real* cells_aos
   if (params->nx < 1 || params->ny < 2) return fail("lbm_gpu_create: need nx >= 1 and ny >= 2 (got %d x %d)", params->nx, params->ny);
   if (n_gpus < 1) return fail("lbm_gpu_create: n_gpus must be >= 1");
   if (params->ny < n_gpus) return fail("lbm_gpu_create: fewer rows (%d) than GPUs (%d)", params->ny, n_gpus);
+  if (flags & LBM_GPU_STORE_F16) {
+    if (sizeof(real) != 4) return fail("lbm_gpu_create_f64: LBM_GPU_STORE_F16 is for fp32 lattices only");
+    if (n_gpus != 1) return fail("lbm_gpu_create: LBM_GPU_STORE_F16 needs n_gpus == 1 (got %d)", n_gpus);
+    const unsigned forced = LBM_GPU_KERNEL_SCALAR | LBM_GPU_KERNEL_TMA | LBM_GPU_KERNEL_PERSISTENT | LBM_GPU_KERNEL_CLUSTER |
+                            LBM_GPU_KERNEL_PAIRS | LBM_GPU_KERNEL_TB3;
+    if (flags & forced)
+      return fail("lbm_gpu_create: LBM_GPU_STORE_F16 runs LBM_GPU_KERNEL_VEC4 or LBM_GPU_KERNEL_TB2 only; "
+                  "another kernel was forced (flags 0x%x)", flags & forced);
+  }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) {
     cudaGetLastError();
@@ -1351,6 +1472,7 @@ int create_impl(const typename ParamT<real>::type* params, const real* cells_aos
   try {
     g->prm = *params;
     g->flags = flags;
+    g->f16 = (flags & LBM_GPU_STORE_F16) != 0;
     g->setup_geometry(params->nx);
     std::vector<long long> row0;
     std::vector<int> rows;
@@ -1372,9 +1494,13 @@ int create_impl(const typename ParamT<real>::type* params, const real* cells_aos
                    obstacles ? (const char*)obstacles + (size_t)s.row0 * obst_row_bytes : nullptr, 0);
     }
     g->connect_local();
-    g->choose_kernel();
-    g->choose_pairs();
-    g->choose_tb2();
+    if (g->f16) {
+      g->choose_f16();
+    } else {
+      g->choose_kernel();
+      g->choose_pairs();
+      g->choose_tb2();
+    }
     g->prepare();
   } catch (const CudaError& e) {
     return fail("lbm_gpu_create: %s", e.what.c_str());
@@ -1694,6 +1820,7 @@ int lbm_gpu_create_slab(const lbm_param* params, long long row0, long long nrows
   *out = nullptr;
   if (params->nx < 1 || params->ny < 2) return fail("lbm_gpu_create_slab: need nx >= 1 and ny >= 2");
   if (row0 < 0 || nrows < 1 || row0 + nrows > params->ny) return fail("lbm_gpu_create_slab: rows [%lld,%lld) outside the grid", row0, row0 + nrows);
+  if (flags & LBM_GPU_STORE_F16) return fail("lbm_gpu_create_slab: LBM_GPU_STORE_F16 is for lbm_gpu_create lattices only, not slab handles");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) {
     cudaGetLastError();
@@ -1731,6 +1858,7 @@ int lbm_gpu_ipc_export(lbm_gpu* h, void* desc) {
   if (!desc) return fail("lbm_gpu_ipc_export: NULL descriptor");
   return guarded<float>(h, "lbm_gpu_ipc_export", [&](Grid<float>& g) {
     if (g.slabs.size() != 1) throw CudaError{"only a one-slab handle can be exported"};
+    if (g.f16) throw CudaError{"a LBM_GPU_STORE_F16 lattice cannot be shared between processes"};
     Slab<float>& s = g.slabs[0];
     CK(cudaSetDevice(s.device));
     IpcDesc d;
@@ -1764,6 +1892,7 @@ namespace {
 // can run (and therefore will run) the two-step kernel
 void ipc_connect_impl(Grid<float>& g, const IpcDesc& dn, const IpcDesc& up, bool ring_tb2) {
   if (g.slabs.size() != 1) throw CudaError{"only a one-slab handle can be connected"};
+  if (g.f16) throw CudaError{"a LBM_GPU_STORE_F16 lattice cannot be shared between processes"};
   Slab<float>& s = g.slabs[0];
   CK(cudaSetDevice(s.device));
   const long long ny = g.prm.ny;

@@ -24,6 +24,7 @@
 //            (d2q9-bgk.c:229-260) without a separate kernel or a pre-pass.
 #pragma once
 #include <cuda.h>            // CUtensorMap (type only; the encoder is fetched at run time)
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -1215,6 +1216,22 @@ __global__ void lbm_prepare(const PrepareArgs<real> a) {
 // ------------------------------------------------------------------------------------
 // K4  setup / output kernels (not on the per-step path)
 // ------------------------------------------------------------------------------------
+// Stored lattice values.  An fp32 / fp64 lattice holds f itself.  A LBM_GPU_STORE_F16 lattice
+// holds the binary16 value of f_k - c_k, with c_k the rest-state value of speed k: encoded with
+// one fp32 subtract and a round to nearest even, decoded exactly and with one fp32 add.
+struct RestShift {
+  float w0, w1, w2;             // density*4/9, density/9, density/36 (as the rest state)
+  __host__ __device__ __forceinline__ float of(const int k) const { return k == 0 ? w0 : (k < 5 ? w1 : w2); }
+};
+__device__ __forceinline__ float f16_dec(const __half s, const float c) { return __fadd_rn(__half2float(s), c); }
+__device__ __forceinline__ __half f16_enc(const float f, const float c) { return __float2half_rn(__fsub_rn(f, c)); }
+template <typename real>
+__device__ __forceinline__ real stored_value(const real* p, int, const RestShift&) { return *p; }
+__device__ __forceinline__ float stored_value(const __half* p, const int k, const RestShift& r) { return f16_dec(*p, r.of(k)); }
+template <typename real>
+__device__ __forceinline__ void store_value(real* p, int, const real v, const RestShift&) { *p = v; }
+__device__ __forceinline__ void store_value(__half* p, const int k, const float v, const RestShift& r) { *p = f16_enc(v, r.of(k)); }
+
 // rest state, d2q9-bgk.c:2802-2823
 template <typename real>
 __global__ void lbm_init_rest(real* buf, long long plane_stride, int pitch, int nx, int rows,
@@ -1228,28 +1245,28 @@ __global__ void lbm_init_rest(real* buf, long long plane_stride, int pitch, int 
 
 // AoS rows (9 reals per cell, dense nx) -> SoA planes; `aos` holds nrows rows that go
 // to local rows [r0, r0+nrows)
-template <typename real>
-__global__ void lbm_aos_to_soa(const real* __restrict__ aos, real* __restrict__ buf, long long plane_stride,
-                               int pitch, int nx, int r0, long long ncells) {
+template <typename real, typename store = real>
+__global__ void lbm_aos_to_soa(const real* __restrict__ aos, store* __restrict__ buf, long long plane_stride,
+                               int pitch, int nx, int r0, long long ncells, RestShift rest = RestShift()) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= ncells * 9) return;
   const long long cell = i / 9;
   const int k = (int)(i - cell * 9);
   const long long row = cell / nx;
   const int x = (int)(cell - row * nx);
-  buf[k * plane_stride + (r0 + row) * pitch + x] = aos[i];
+  store_value(buf + k * plane_stride + (r0 + row) * pitch + x, k, aos[i], rest);
 }
 
-template <typename real>
-__global__ void lbm_soa_to_aos(const real* __restrict__ buf, real* __restrict__ aos, long long plane_stride,
-                               int pitch, int nx, int r0, long long ncells) {
+template <typename real, typename store = real>
+__global__ void lbm_soa_to_aos(const store* __restrict__ buf, real* __restrict__ aos, long long plane_stride,
+                               int pitch, int nx, int r0, long long ncells, RestShift rest = RestShift()) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= ncells * 9) return;
   const long long cell = i / 9;
   const int k = (int)(i - cell * 9);
   const long long row = cell / nx;
   const int x = (int)(cell - row * nx);
-  aos[i] = buf[k * plane_stride + (r0 + row) * pitch + x];
+  aos[i] = stored_value(buf + k * plane_stride + (r0 + row) * pitch + x, k, rest);
 }
 
 // int-per-cell obstacle rows -> bit mask rows; one warp packs 32 cells with a ballot.
@@ -1289,12 +1306,12 @@ __global__ void lbm_copy_mask_bits(const uint32_t* __restrict__ in, uint32_t* __
 // write_values' per-cell fields (d2q9-bgk.c:2937-2976) for local rows [r0, r0+nrows):
 // dense nx-wide outputs.  Also usable as av_velocity (d2q9-bgk.c:2665-2714) through
 // the |u| accumulator (warp_accumulate) when av != NULL.
-template <typename real>
-__global__ void lbm_fields(const real* __restrict__ buf, const uint32_t* __restrict__ mask,
+template <typename real, typename store = real>
+__global__ void lbm_fields(const store* __restrict__ buf, const uint32_t* __restrict__ mask,
                            long long plane_stride, int pitch, int mask_pitch, int nx, int r0, int nrows,
                            real density, real* __restrict__ ux_out, real* __restrict__ uy_out,
                            real* __restrict__ u_out, real* __restrict__ p_out,
-                           unsigned long long* av) {
+                           unsigned long long* av, RestShift rest = RestShift()) {
   const long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   unsigned long long q = 0ULL;
   if (n < (long long)nrows * nx) {
@@ -1304,7 +1321,7 @@ __global__ void lbm_fields(const real* __restrict__ buf, const uint32_t* __restr
     const bool obst = (mask[(long long)r * mask_pitch + (x >> 5)] >> (x & 31)) & 1u;
     real f[9];
 #pragma unroll
-    for (int k = 0; k < 9; k++) f[k] = buf[k * plane_stride + (long long)r * pitch + x];
+    for (int k = 0; k < 9; k++) f[k] = stored_value(buf + k * plane_stride + (long long)r * pitch + x, k, rest);
     real ux, uy, rho;
     real u = cell_macroscopic<real>(f, ux, uy, rho);
     const real c_sq = (real)1 / (real)3;
@@ -1329,9 +1346,10 @@ __global__ void lbm_fields(const real* __restrict__ buf, const uint32_t* __restr
 __device__ __forceinline__ unsigned long long bits_of(float f) { return (unsigned long long)__float_as_uint(f); }
 __device__ __forceinline__ unsigned long long bits_of(double f) { return (unsigned long long)__double_as_longlong(f); }
 
-template <typename real>
-__global__ void lbm_digest(const real* __restrict__ buf, long long plane_stride, int pitch, int nx, int r0,
-                           int nrows, long long global_row0, unsigned long long* out /* [mass, checksum] */) {
+template <typename real, typename store = real>
+__global__ void lbm_digest(const store* __restrict__ buf, long long plane_stride, int pitch, int nx, int r0,
+                           int nrows, long long global_row0, unsigned long long* out /* [mass, checksum] */,
+                           RestShift rest = RestShift()) {
   const long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   unsigned long long mass = 0ULL, sum = 0ULL;
   if (n < (long long)nrows * nx) {
@@ -1340,7 +1358,7 @@ __global__ void lbm_digest(const real* __restrict__ buf, long long plane_stride,
     const unsigned long long g = (unsigned long long)(global_row0 + row) * (unsigned long long)nx + (unsigned long long)x;
 #pragma unroll
     for (int k = 0; k < 9; k++) {
-      const real f = buf[k * plane_stride + (long long)(r0 + row) * pitch + x];
+      const real f = stored_value(buf + k * plane_stride + (long long)(r0 + row) * pitch + x, k, rest);
       mass += (unsigned long long)__double2ll_rn((double)f * 4294967296.0);
       const unsigned long long w = (g * 0x9E3779B97F4A7C15ULL + (unsigned long long)(k + 1) * 0xC2B2AE3D27D4EB4FULL) | 1ULL;
       sum += bits_of(f) * w;

@@ -11,6 +11,8 @@
  *   LBM_GPUS=N             split the rows over N GPUs (default 1)
  *   LBM_PRECISION=f64      run the double-precision validation kernel (the golden files
  *                          in check/ were produced by a double build of the reference)
+ *   LBM_PRECISION=f16      keep the lattice as shifted binary16 (LBM_GPU_STORE_F16: half the
+ *                          device memory, fp32 arithmetic, less accurate; single GPU only)
  *   LBM_STRICT=1           source operation order, no FMA contraction
  *   LBM_KERNEL=scalar|vec4|persistent|tma|cluster|tb2|tb3|pairs   force a kernel variant
  *   LBM_SKIP_FINAL_STATE=1 do not write final_state.dat (huge synthetic grids: 16384^2
@@ -68,6 +70,7 @@ int main(int argc, char* argv[])
   const int f64 = getenv("LBM_PRECISION") != NULL && strcmp(getenv("LBM_PRECISION"), "f64") == 0;
   const int n_gpus = getenv("LBM_GPUS") ? atoi(getenv("LBM_GPUS")) : 1;
   unsigned flags = LBM_GPU_OBST_BITS;
+  if (getenv("LBM_PRECISION") != NULL && strcmp(getenv("LBM_PRECISION"), "f16") == 0) flags |= LBM_GPU_STORE_F16;
   if (env_flag("LBM_STRICT")) flags |= LBM_GPU_STRICT;
   const char* kv = getenv("LBM_KERNEL");
   if (kv != NULL) {
@@ -164,7 +167,7 @@ int main(int argc, char* argv[])
     printf("{\"nx\": %d, \"ny\": %d, \"steps\": %d, \"gpus\": %d, \"precision\": \"%s\", \"kernel\": %d, "
            "\"init_s\": %.6f, \"compute_s\": %.6f, \"collate_s\": %.6f, \"device_compute_s\": %.6f, "
            "\"mlups_device\": %.1f, \"gbs_72B\": %.1f, \"free_cells\": %lld, \"kernel_launches\": %lld}\n",
-           nx, ny, iters, n_gpus, f64 ? "f64" : "f32", info.kernel, init_toc - init_tic, comp_toc - comp_tic,
+           nx, ny, iters, n_gpus, f64 ? "f64" : (flags & LBM_GPU_STORE_F16) ? "f16" : "f32", info.kernel, init_toc - init_tic, comp_toc - comp_tic,
            col_toc - col_tic, dev_s, dev_s > 0 ? updates / dev_s / 1e6 : 0.0, dev_s > 0 ? updates * 72.0 / dev_s / 1e9 : 0.0,
            info.free_cells, info.kernel_launches);
   } else if (env_flag("LBM_REPORT")) {

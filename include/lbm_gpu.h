@@ -94,6 +94,21 @@ typedef struct lbm_gpu lbm_gpu;   /* opaque handle: one lattice on one or more G
 #define LBM_GPU_SYNC_EVENTS 1024u  /* lbm_gpu_create with n_gpus > 1: order the slabs with CUDA events
                                       (host-recorded, no device-side waiting) even when every slab has its
                                       own GPU; always used when slabs share a GPU */
+/* Shifted binary16 lattice storage: half the bytes per cell (larger grids, fewer bytes per update)
+ * for some accuracy.  With c_k the rest-state value of speed k computed in fp32 as for the rest
+ * state (density*4/9, density/9, density/36), the lattice holds s_k = __float2half_rn(f_k - c_k)
+ * (one fp32 subtract, round to nearest even) and is read as f_k = __half2float(s_k) + c_k (one fp32
+ * add).  A timestep decodes, runs the ordinary fp32 step (accelerate row ny-2, pull, rebound or
+ * collide), and encodes.  Not rounded: the accelerated values of row ny-2 within a step, and the |u|
+ * that goes into av_vels (taken from the fp32 results before they are encoded).  The rest state
+ * encodes to zeros; download / final_fields / av_velocity / lbm_gpu_digest see the decoded fp32
+ * values; upload and create with cells_aos encode (and so round).  With LBM_GPU_STRICT the result is
+ * bit-exact against the fp32 reference arithmetic with the same encode/decode between steps.
+ * lbm_gpu_create only, fp32, n_gpus == 1; the only kernels that may be forced are
+ * LBM_GPU_KERNEL_VEC4 (one step per pass) and LBM_GPU_KERNEL_TB2 (two steps per pass, nx a multiple
+ * of 8 and >= 32, at least 8 rows; the default where it applies).  The accuracy of the shipped
+ * inputs is in INTEGRATION.md. */
+#define LBM_GPU_STORE_F16   8192u
 
 /* Information about a handle (lbm_gpu_get_info). */
 typedef struct {
