@@ -1298,10 +1298,20 @@ class Grid : public GridBase {
     throw CudaError{"row is not held by this process"};
   }
 
+  // Refuse a row range that leaves the rows held here before anything is enqueued, so that a
+  // refused call leaves no copy in flight into the caller's buffers or the staging buffer.
+  void check_rows(long long row0, long long nrows) {
+    long long held = 0;
+    for (auto& s : slabs) held += s.rows;
+    if (nrows > 0 && (row0 < slabs[0].row0 || row0 + nrows > slabs[0].row0 + held))
+      throw CudaError{"row range is not held by this process"};
+  }
+
   void download_rows(long long row0, long long nrows, real* out) {
     const int nx = prm.nx;
     const size_t row_bytes = (size_t)nx * 9 * sizeof(real);
     if (row_bytes > kStagingBytes) throw CudaError{"nx too large for the AoS staging buffer"};
+    check_rows(row0, nrows);
     const int chunk_rows = (int)std::max<size_t>(1, kStagingBytes / row_bytes);
     long long g = row0;
     while (g < row0 + nrows) {
@@ -1332,6 +1342,7 @@ class Grid : public GridBase {
     const size_t row_bytes = (size_t)nx * sizeof(real);
     const size_t half = kStagingBytes / 2;
     if (4 * row_bytes > half) throw CudaError{"nx too large for the fields staging buffer"};
+    check_rows(row0, nrows);
     const int chunk_rows = (int)(half / (4 * row_bytes));
     std::vector<Slab<real>*> used;
     long long g = row0;
@@ -1382,6 +1393,7 @@ class Grid : public GridBase {
 
   double av_velocity_sum() {
     unsigned __int128 tot = 0;
+    bool bad = false;
     for (auto& s : slabs) {
       CK(cudaSetDevice(s.device));
       unsigned long long* av = s.sync + kAvScratch;       // 128-byte aligned inside the sync block
@@ -1400,19 +1412,24 @@ class Grid : public GridBase {
       unsigned long long w[kAvWords];
       CK(cudaMemcpyAsync(w, av, sizeof w, cudaMemcpyDeviceToHost, s.stream));
       CK(cudaStreamSynchronize(s.stream));
-      for (int k = 0; k < LBM_AV_SLOTS; k++)
-        tot += ((unsigned __int128)w[LBM_AV_STRIDE * k + 1] << 32) + w[LBM_AV_STRIDE * k];
+      for (int k = 0; k < LBM_AV_SLOTS; k++) {
+        const unsigned long long hi = w[LBM_AV_STRIDE * k + 1];
+        if (hi & LBM_NONFINITE_MARK) bad = true;
+        tot += ((unsigned __int128)(hi & ~LBM_NONFINITE_MARK) << 32) + w[LBM_AV_STRIDE * k];
+      }
     }
+    if (bad) return std::nan("");                // a NaN or blown-up cell, as in read_sums
     return (double)((long double)tot / (long double)LBM_FIX_SCALE);
   }
 
   // exact digest of the rows held by this process (see lbm_digest)
   void digest(double* total_density, unsigned long long* checksum) {
     unsigned long long mass = 0, sum = 0;
+    bool bad = false;
     for (auto& s : slabs) {
       CK(cudaSetDevice(s.device));
-      unsigned long long* out = s.sync + kScratch1;
-      CK(cudaMemsetAsync(out, 0, 2 * sizeof(unsigned long long), s.stream));
+      unsigned long long* out = s.sync + kScratch0;         // kScratch0..2: mass, checksum, mark
+      CK(cudaMemsetAsync(out, 0, 3 * sizeof(unsigned long long), s.stream));
       const long long ncells = (long long)s.rows * prm.nx;
       if (f16)
         lbm::lbm_digest<real, __half><<<(unsigned)((ncells + 255) / 256), 256, 0, s.stream>>>(
@@ -1422,13 +1439,14 @@ class Grid : public GridBase {
             s.lattice[cur], plane_stride(s), pitch, prm.nx, 0, s.rows, s.row0, out);
       CK(cudaGetLastError());
       launches++;
-      unsigned long long w[2];
+      unsigned long long w[3];
       CK(cudaMemcpyAsync(w, out, sizeof w, cudaMemcpyDeviceToHost, s.stream));
       CK(cudaStreamSynchronize(s.stream));
       mass += w[0];
       sum += w[1];
+      bad = bad || w[2] != 0;
     }
-    if (total_density) *total_density = (double)(long long)mass / 4294967296.0;
+    if (total_density) *total_density = bad ? std::nan("") : (double)(long long)mass / 4294967296.0;
     if (checksum) *checksum = sum;
   }
 };

@@ -1305,7 +1305,9 @@ __global__ void lbm_copy_mask_bits(const uint32_t* __restrict__ in, uint32_t* __
 
 // write_values' per-cell fields (d2q9-bgk.c:2937-2976) for local rows [r0, r0+nrows):
 // dense nx-wide outputs.  Also usable as av_velocity (d2q9-bgk.c:2665-2714) through
-// the |u| accumulator (warp_accumulate) when av != NULL.
+// the |u| accumulator (warp_accumulate) when av != NULL; a fluid cell whose |u| is NaN or
+// not below LBM_SPEED_LIMIT adds nothing and sets LBM_NONFINITE_MARK in av[1], as the step
+// kernels do.
 template <typename real, typename store = real>
 __global__ void lbm_fields(const store* __restrict__ buf, const uint32_t* __restrict__ mask,
                            long long plane_stride, int pitch, int mask_pitch, int nx, int r0, int nrows,
@@ -1331,7 +1333,8 @@ __global__ void lbm_fields(const store* __restrict__ buf, const uint32_t* __rest
     if (uy_out) uy_out[n] = uy;
     if (u_out) u_out[n] = u;
     if (p_out) p_out[n] = pr;
-    q = to_fixed(u);
+    if (u < (real)LBM_SPEED_LIMIT) q = to_fixed(u);
+    else if (av) atomicOr(av + 1, LBM_NONFINITE_MARK);
   }
   if (av) warp_accumulate(q, av);
 }
@@ -1343,15 +1346,19 @@ __global__ void lbm_fields(const store* __restrict__ buf, const uint32_t* __rest
 //   checksum  sum of bit_pattern(f_k(cell)) * odd_weight(global cell index, k): equal for
 //             two lattices iff (up to 2^-64) every speed of every cell has the same bits,
 //             whatever the decomposition.  Full-size stand-in for a lattice comparison.
+// A value that is NaN, infinite or of magnitude 2^31 or more has no fixed-point mass: it adds
+// nothing to the mass and sets out[2], and the host reports total_density as NaN.
 __device__ __forceinline__ unsigned long long bits_of(float f) { return (unsigned long long)__float_as_uint(f); }
 __device__ __forceinline__ unsigned long long bits_of(double f) { return (unsigned long long)__double_as_longlong(f); }
 
 template <typename real, typename store = real>
 __global__ void lbm_digest(const store* __restrict__ buf, long long plane_stride, int pitch, int nx, int r0,
-                           int nrows, long long global_row0, unsigned long long* out /* [mass, checksum] */,
+                           int nrows, long long global_row0,
+                           unsigned long long* out /* [mass, checksum, non-finite mark] */,
                            RestShift rest = RestShift()) {
   const long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   unsigned long long mass = 0ULL, sum = 0ULL;
+  bool bad = false;
   if (n < (long long)nrows * nx) {
     const int row = (int)(n / nx);
     const int x = (int)(n - (long long)row * nx);
@@ -1359,7 +1366,8 @@ __global__ void lbm_digest(const store* __restrict__ buf, long long plane_stride
 #pragma unroll
     for (int k = 0; k < 9; k++) {
       const real f = stored_value(buf + k * plane_stride + (long long)(r0 + row) * pitch + x, k, rest);
-      mass += (unsigned long long)__double2ll_rn((double)f * 4294967296.0);
+      if (::fabs((double)f) < 2147483648.0) mass += (unsigned long long)__double2ll_rn((double)f * 4294967296.0);
+      else bad = true;
       const unsigned long long w = (g * 0x9E3779B97F4A7C15ULL + (unsigned long long)(k + 1) * 0xC2B2AE3D27D4EB4FULL) | 1ULL;
       sum += bits_of(f) * w;
     }
@@ -1373,6 +1381,7 @@ __global__ void lbm_digest(const store* __restrict__ buf, long long plane_stride
     if (mass) atomicAdd(out + 0, mass);
     if (sum) atomicAdd(out + 1, sum);
   }
+  if (bad) atomicOr(out + 2, 1ULL);
 }
 
 }  // namespace lbm

@@ -233,7 +233,11 @@ int lbm_gpu_run_batch(lbm_gpu* const* handles, int n, int n_steps, float* av_vel
  *                   row range, so a writer can stream huge grids slab by slab.  Any of
  *                   the four output pointers may be NULL.
  *   av_velocity     av_velocity() of the current lattice (d2q9-bgk.c:2665-2714) for
- *                   the Reynolds number line; sum over local rows / free cells.
+ *                   the Reynolds number line; sum over local rows / free cells.  NaN when
+ *                   a fluid cell's |u| is NaN (a NaN or zero-density cell) or not below 2,
+ *                   as lbm_gpu_run reports such a step.
+ * For download_rows and final_fields, nrows = 0 succeeds and writes nothing; a negative
+ * nrows, or rows not held by this process, is refused before anything is written.
  */
 int lbm_gpu_download(lbm_gpu* h, float* cells_aos_out);
 int lbm_gpu_download_rows(lbm_gpu* h, long long row0, long long nrows, float* cells_aos_out);
@@ -254,6 +258,8 @@ int lbm_gpu_av_velocity_f64(lbm_gpu* h, double* av_out);
  * Both are integer sums: independent of summation order and additive over slabs and
  * ranks, so two runs hold the same lattice iff their checksums agree -- the way to
  * compare lattices too large to download (16384 x 131072 is 77 GB).  Either may be NULL.
+ * A speed that is NaN, infinite or of magnitude 2^31 or more has no fixed-point value:
+ * total_density is then NaN, as the reference's sum would be; the checksum is unaffected.
  */
 int lbm_gpu_digest(lbm_gpu* h, double* total_density, unsigned long long* checksum);
 

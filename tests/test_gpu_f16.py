@@ -19,6 +19,7 @@ from hypothesis import HealthCheck, given, settings, strategies as st
 import lbm_b200 as L
 import oracle_f16 as H
 import oracle_lib as O
+import readout_ref as R
 
 pytestmark = pytest.mark.gpu
 D, A, W = 0.1, 0.005, 1.85
@@ -123,6 +124,8 @@ def test_upload_and_create_encode_as_numpy_does(nx, ny):
         assert bits_equal(u, ru) and bits_equal(p, rp)
         _, tot, n = O.av_velocity(want, obst)          # the oracle's double sum: the device sum is exact
         assert lat.av_velocity() == pytest.approx(tot / n, rel=1e-6)
+        assert lat.av_velocity() == R.host_average(R.fixed_u_sum(ru, obst), n, np.float32)
+        assert mass == R.digest_mass(got)
 
 
 def test_device_bytes_show_the_saving():

@@ -15,6 +15,7 @@ import pytest
 
 import lbm_b200 as L
 import oracle_lib as O
+import readout_ref as R
 
 pytestmark = pytest.mark.gpu
 
@@ -160,6 +161,7 @@ def test_final_fields_and_av_velocity():
         sub = lat.final_fields(row0=5, nrows=7)
         assert np.array_equal(sub[3], pr[5:12])
         assert abs(lat.av_velocity() - tot / n) <= 1e-7 * (tot / n)
+        assert lat.av_velocity() == R.host_average(R.fixed_u_sum(u, obst), n, np.float32)   # exact sum
         rows = lat.download_rows(4, 3)
         assert np.array_equal(rows, ref[4:7])
 
