@@ -62,6 +62,20 @@ struct CudaError {
 
 inline long long round_up(long long v, long long m) { return (v + m - 1) / m * m; }
 
+inline bool env_on(const char* name) { const char* e = getenv(name); return e && e[0] == '1'; }   // kill switches
+
+// The one LBM_GPU_KERNEL_* flag the caller forced, or 0; two or more are refused, by name.
+unsigned forced_kernel(unsigned flags) {
+  // LBM_GPU_KERNEL_<name> == 1 << index
+  static const char* const names[] = {nullptr, nullptr, "SCALAR", "TMA", "VEC4", nullptr, "PERSISTENT", nullptr, "CLUSTER", "TB2", nullptr, "PAIRS", "TB3"};
+  unsigned k = 0;
+  std::string msg = "more than one kernel forced, pass at most one of:";
+  for (int b = 0; b < 13; b++)
+    if (names[b] && (flags >> b & 1)) { k |= 1u << b; msg += std::string(" LBM_GPU_KERNEL_") + names[b]; }
+  if (k & (k - 1)) throw CudaError{msg};
+  return k;
+}
+
 constexpr int kPersistScalarBlocks = 296;      // measured, profiles/r01_small_grids.md
 constexpr long long kPersistMaxCells = 1280 * 1024;   // K5 up to here (1024^2: 109 GLUPS against 63 for K7); from 1280^2 on K7 wins (profiles/r02_kernel_variants.md)
 constexpr size_t kStagingBytes = 64u << 20;   // device staging for AoS<->SoA / mask / fields
@@ -158,7 +172,7 @@ class Grid : public GridBase {
   typedef typename ParamT<real>::type Param;
   Param prm;
   unsigned flags = 0;
-  int kernel = 0;
+  int kernel = 0;              // LBM_GPU_KERNEL_* that runs: set by select_kernel() only
   int persistent_vec = 4;      // cells per thread of the persistent kernel (4, or 1 for tiny grids)
   int cluster_ctas = 0;        // K6: CTAs of the cluster (16 or 8), 0 = not applicable
   int cluster_rows = 0;        // K6: rows per CTA
@@ -172,10 +186,8 @@ class Grid : public GridBase {
   long long steps_done = 0;
   long long passes_done = 0;   // kernel passes (one or two timesteps each): the unit of the flag protocol
   int cur = 0;                 // lattice buffer / window parity holding the current state (flips per pass)
-  bool tb2 = false;            // two timesteps per pass (K7) wherever two steps remain
   int tb2_strips = 0, tb2_wout = 0, tb2_seg_rows = 0, tb2_span = 0, tb2_threads = 0;
   int tb2_tail_rows = 16, tb2_tail_segs = 0;   // K7: height and number of the short segments that end a launch
-  bool tb3 = false;            // three timesteps per pass (K10) wherever three steps remain (K7 for two, K1a for one)
   int tb3_seg_rows = 0;        // K10: rows per segment
   int pairs_tile_rows = 0;     // K9: rows per block
   bool f16 = false;            // LBM_GPU_STORE_F16: the lattice buffers hold shifted binary16 (lbm_f16.cuh)
@@ -361,22 +373,10 @@ class Grid : public GridBase {
       const double ms = atof(e);
       if (ms > 0) timeout_ns = (unsigned long long)(ms * 1e6);
     }
-    if (flags & LBM_GPU_KERNEL_SCALAR) kernel = LBM_GPU_KERNEL_SCALAR;
-    else if (flags & LBM_GPU_KERNEL_VEC4) kernel = LBM_GPU_KERNEL_VEC4;
-    else if (flags & LBM_GPU_KERNEL_PERSISTENT) kernel = LBM_GPU_KERNEL_PERSISTENT;
-    else if (flags & (LBM_GPU_KERNEL_TB2 | LBM_GPU_KERNEL_TB3)) kernel = LBM_GPU_KERNEL_VEC4;   // decided in choose_tb2()
-    else if (flags & LBM_GPU_KERNEL_PAIRS) kernel = LBM_GPU_KERNEL_VEC4;       // decided in choose_pairs()
-    else if (flags & LBM_GPU_KERNEL_CLUSTER) kernel = LBM_GPU_KERNEL_VEC4;     // decided in choose_kernel()
-    else kernel = LBM_GPU_KERNEL_VEC4;                         // refined in choose_kernel()
-    if (flags & LBM_GPU_KERNEL_TMA) {
-      if (sizeof(real) != 4) throw CudaError{"the TMA kernel is built for single precision only"};
-      kernel = LBM_GPU_KERNEL_TMA;
-    }
   }
 
   // launch shape shared by the step kernels: blockDim (bx, by), tiles of bx*vec x by cells
-  void tile_shape(int& vec, int& bx, int& by) const {
-    vec = (kernel == LBM_GPU_KERNEL_SCALAR || (kernel == LBM_GPU_KERNEL_PERSISTENT && persistent_vec == 1)) ? 1 : 4;
+  void tile_shape(int vec, int& bx, int& by) const {
     const int nxv = (prm.nx + vec - 1) / vec;
     bx = (int)std::min<long long>(LBM_BLOCK_THREADS, round_up(nxv, 32));
     if (kernel == LBM_GPU_KERNEL_TMA) bx = LBM_BLOCK_THREADS;     // one row of LBM_TMA_TILE cells per block
@@ -399,8 +399,6 @@ class Grid : public GridBase {
     return coop ? per_sm * sms : 0;
   }
 
-  // After the slabs exist: grids small enough to be launch-latency bound (they live in
-  // L2) run all their steps in one persistent cooperative kernel.
   const void* cluster_fn() const {
     return (flags & LBM_GPU_STRICT) ? (const void*)lbm::lbm_steps_cluster<true> : (const void*)lbm::lbm_steps_cluster<false>;
   }
@@ -410,7 +408,6 @@ class Grid : public GridBase {
   bool cluster_fits() {
     if (sizeof(real) != 4 || slabs.size() != 1 || slab_mode) return false;
     Slab<real>& s = slabs[0];
-    CK(cudaSetDevice(s.device));
     int max_smem = 0;
     CK(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, s.device));
     for (int c : {16, 8}) {
@@ -444,60 +441,37 @@ class Grid : public GridBase {
     return false;
   }
 
-  void choose_kernel() {
-    const bool forced = flags & (LBM_GPU_KERNEL_SCALAR | LBM_GPU_KERNEL_VEC4 | LBM_GPU_KERNEL_PERSISTENT |
-                                 LBM_GPU_KERNEL_TMA | LBM_GPU_KERNEL_CLUSTER | LBM_GPU_KERNEL_TB2 |
-                                 LBM_GPU_KERNEL_PAIRS | LBM_GPU_KERNEL_TB3);
-    // K6 is opt-in only: 16 SMs doing all the arithmetic are no faster than K5 spreading it
-    // over the whole chip (profiles/r01_small_grids.md).
-    if (flags & LBM_GPU_KERNEL_CLUSTER) {
-      if (cluster_fits()) { kernel = LBM_GPU_KERNEL_CLUSTER; return; }
-      throw CudaError{"the cluster kernel needs a single-GPU fp32 lattice that fits in one cluster's shared memory"};
-    }
-    const bool want = (kernel == LBM_GPU_KERNEL_PERSISTENT);
-    if (!want && (forced || slabs.size() != 1 || slab_mode)) return;
-    if (slabs.size() != 1 || slab_mode) throw CudaError{"the persistent kernel handles a single slab only"};
-    CK(cudaSetDevice(slabs[0].device));
-    const int saved = kernel;
-    kernel = LBM_GPU_KERNEL_PERSISTENT;
-    auto tiles_for = [&](int pv) {
-      persistent_vec = pv;
-      int vec, bx, by;
-      tile_shape(vec, bx, by);
-      return (long long)(((prm.nx + vec - 1) / vec + bx - 1) / bx) * ((slabs[0].rows + by - 1) / by);
-    };
+  // K5 on the single slab: one or four cells per thread; false without cooperative launch
+  bool persistent_fits() {
     // tiny grids: one cell per thread (4x the threads on the step's dependent-latency chain)
     // as long as that does not put more than kPersistScalarBlocks blocks on the grid barrier
-    long long tiles = tiles_for(1);
+    int bx, by;
+    tile_shape(1, bx, by);
+    const long long tiles = (long long)((prm.nx + bx - 1) / bx) * ((slabs[0].rows + by - 1) / by);
+    persistent_vec = 1;
     int cap = persistent_capacity(slabs[0]);
     long long scalar_limit = std::min<long long>(cap, kPersistScalarBlocks);
     if (const char* e = getenv("LBM_PERSIST_VEC"))      // measurement knob of profiles/r01_small_grids.md
       scalar_limit = (atoi(e) == 1) ? cap : 0;
     if (tiles > scalar_limit) {
-      tiles = tiles_for(4);
+      persistent_vec = 4;
       cap = persistent_capacity(slabs[0]);
     }
-    if (cap < 1) {
-      if (want) throw CudaError{"cooperative launch is not available on this device"};
-      kernel = saved;
-    } else if (!want && (long long)prm.nx * slabs[0].rows > kPersistMaxCells) {
-      kernel = saved;             // beyond L2: bandwidth bound, one launch per pass is free
-    }
+    return cap >= 1;
   }
 
   // K7 (two timesteps per pass) needs fp32, a width the 16-byte bulk copies can cut (multiple
-  // of 4), slabs tall enough for two-row ghost zones, and no
+  // of 4; of 8 for binary16 rows), slabs tall enough for two-row ghost zones, and no other
   // kernel forced by the caller.  Every slab of the grid must come to the same answer: the
   // ghost-row pushes and the flag protocol count passes, not timesteps.
-  bool tb2_possible(int rows_min) const {
-    if (sizeof(real) != 4) return false;
-    if (flags & (LBM_GPU_KERNEL_SCALAR | LBM_GPU_KERNEL_VEC4 | LBM_GPU_KERNEL_PERSISTENT | LBM_GPU_KERNEL_TMA |
-                 LBM_GPU_KERNEL_CLUSTER | LBM_GPU_KERNEL_PAIRS)) return false;
-    if (getenv("LBM_GPU_NO_TB2") && getenv("LBM_GPU_NO_TB2")[0] == '1') return false;
-    return (prm.nx % 4 == 0) && prm.nx >= 32 && rows_min >= kTb2MinRows;
+  bool k7_fits(int rows_min) const {
+    const unsigned k = forced_kernel(flags);
+    if (k != 0 && k != LBM_GPU_KERNEL_TB2 && k != LBM_GPU_KERNEL_TB3) return false;
+    if (f16) return prm.nx % 8 == 0 && prm.nx >= 32 && rows_min >= kTb2MinRows;
+    return sizeof(real) == 4 && !env_on("LBM_GPU_NO_TB2") && prm.nx % 4 == 0 && prm.nx >= 32 && rows_min >= kTb2MinRows;
   }
 
-  void enable_tb2() {
+  void configure_tb2() {
     if constexpr (sizeof(real) == 4) {
       for (auto& s : slabs) {
         CK(cudaSetDevice(s.device));
@@ -522,11 +496,7 @@ class Grid : public GridBase {
         tb2_span = LBM_TB2_SPAN;
       }
       tb2_threads = (int)round_up(tb2_span / 4, 32);
-      // Segment height.  Every segment recomputes two rows of the first sub-step, so tall is
-      // cheap; but the blocks of a launch run in "waves" of the resident blocks and a last wave
-      // that is nearly empty leaves the SMs idle (16384 rows in 64-row segments: 19.03 waves).
-      // Score each height by (rows / (rows + 2)) x (waves / ceil(waves)) and take the best; grids
-      // with few blocks prefer short segments so that there are several waves at all.
+      // segment height: every segment recomputes two rows of the first sub-step, so tall is cheap
       int rows_max = 0;
       for (auto& s : slabs) rows_max = std::max(rows_max, s.rows);
       const double resident = (double)LBM_TB2_MIN_BLOCKS * sm_count();
@@ -539,8 +509,6 @@ class Grid : public GridBase {
       tb2_tail_segs = (int)((resident + tb2_strips - 1) / tb2_strips) + 1;
       if (const char* e = getenv("LBM_TB2_TAIL_ROWS")) tb2_tail_rows = atoi(e);                // tuning knob, 0 = off
       if (tb2_tail_rows < 2) tb2_tail_segs = 0;
-      tb2 = true;
-      kernel = LBM_GPU_KERNEL_TB2;
     }
   }
 
@@ -569,11 +537,10 @@ class Grid : public GridBase {
 
   // K10 (three timesteps per pass) on top of K7: one slab that holds the whole grid (its
   // rows beyond the ends are its own, so no three-deep ghost zones are needed), at least
-  // kTb3MinRows rows, and the K7 conditions.
-  bool tb3_possible() const {
-    return slabs.size() == 1 && slabs[0].rows == prm.ny && slabs[0].row0 == 0 && !(flags & LBM_GPU_KERNEL_TB2) &&
-           tb2_possible(slabs[0].rows) && slabs[0].rows >= kTb3MinRows &&
-           !(getenv("LBM_GPU_NO_TB3") && getenv("LBM_GPU_NO_TB3")[0] == '1');
+  // kTb3MinRows rows, fp32 storage, and the K7 conditions.
+  bool k10_fits() const {
+    return slabs.size() == 1 && slabs[0].rows == prm.ny && slabs[0].row0 == 0 && !f16 && k7_fits(slabs[0].rows) &&
+           slabs[0].rows >= kTb3MinRows && !env_on("LBM_GPU_NO_TB3");
   }
   // Default: K10 where it was measured faster than K7 (profiles/r03_size_sweep.log), i.e. where
   // its blocks fill enough waves of the SMs; with few waves the launch tail of K10's longer
@@ -582,7 +549,7 @@ class Grid : public GridBase {
     const double resident = (double)LBM_TB3_MIN_BLOCKS * sm_count();
     return tb_waves(slabs[0].rows, 64, resident) >= kTb3MinWaves;
   }
-  void enable_tb3() {
+  void configure_tb3() {
     if constexpr (sizeof(real) == 4) {
       Slab<real>& s = slabs[0];
       CK(cudaSetDevice(s.device));
@@ -591,8 +558,6 @@ class Grid : public GridBase {
       const double resident = (double)LBM_TB3_MIN_BLOCKS * sm_count();
       tb3_seg_rows = best_segment_rows(s.rows, resident, 4, 96);   // 96 rows measured best at 16384^2 (profiles/r03_k10.md)
       if (const char* e = getenv("LBM_TB3_SEG_ROWS")) tb3_seg_rows = std::max(1, atoi(e));   // tuning knob
-      tb3 = true;
-      kernel = LBM_GPU_KERNEL_TB3;
     }
   }
 
@@ -630,7 +595,8 @@ class Grid : public GridBase {
   }
 
   // K9 (two timesteps per grid barrier) for the small grids the persistent kernel K5 would
-  // take: single GPU, fp32, nx a multiple of 4 and at most 256, every block resident.
+  // take: single GPU, fp32, nx a multiple of 4 and at most 256, every block resident.  pairs_fit()
+  // checks them and sets the tile rows.
   const void* pairs_fn() const {
     if constexpr (sizeof(real) == 4)
       return (flags & LBM_GPU_STRICT) ? (const void*)lbm::lbm_steps_pairs<true> : (const void*)lbm::lbm_steps_pairs<false>;
@@ -639,59 +605,108 @@ class Grid : public GridBase {
   dim3 pairs_block() const { return dim3((unsigned)round_up(prm.nx / 4, 32), (unsigned)(pairs_tile_rows + 2)); }
   size_t pairs_smem() const { return (size_t)(pairs_tile_rows + 2) * 9 * prm.nx * sizeof(float); }
 
-  void choose_pairs() {
-    const bool want = (flags & LBM_GPU_KERNEL_PAIRS) != 0;
-    const bool small = (kernel == LBM_GPU_KERNEL_PERSISTENT) && !(flags & LBM_GPU_KERNEL_PERSISTENT);
-    static const bool off = getenv("LBM_GPU_NO_PAIRS") && getenv("LBM_GPU_NO_PAIRS")[0] == '1';
-    if (!want && (!small || off)) return;
-    bool ok = sizeof(real) == 4 && slabs.size() == 1 && !slab_mode && prm.nx % 4 == 0 && prm.nx >= 4 &&
-              prm.nx <= LBM_PAIRS_MAX_NX && slabs[0].rows >= 4;
-    if (ok) {
-      Slab<real>& s = slabs[0];
-      CK(cudaSetDevice(s.device));
-      int sms = 0, coop = 0, per_sm = 0;
-      CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s.device));
-      CK(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, s.device));
-      // one block per SM if the grid allows it: the fewest rows per block that still fits
-      pairs_tile_rows = std::min(LBM_PAIRS_MAX_TILE_ROWS, std::max(1, (s.rows + sms - 1) / sms));
-      if (const char* e = getenv("LBM_PAIRS_TILE_ROWS"))                      // tuning knob
-        pairs_tile_rows = std::min(LBM_PAIRS_MAX_TILE_ROWS, std::max(1, atoi(e)));
-      pairs_tile_rows = std::min(pairs_tile_rows, s.rows - 2);
-      const dim3 b = pairs_block();
-      ok = coop && cudaFuncSetAttribute(pairs_fn(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pairs_smem()) == cudaSuccess &&
-           cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pairs_fn(), (int)(b.x * b.y), pairs_smem()) == cudaSuccess &&
-           (long long)per_sm * sms >= (s.rows + pairs_tile_rows - 1) / pairs_tile_rows;
-      cudaGetLastError();
+  bool pairs_fit() {
+    if (!(sizeof(real) == 4 && slabs.size() == 1 && !slab_mode && prm.nx % 4 == 0 && prm.nx >= 4 &&
+          prm.nx <= LBM_PAIRS_MAX_NX && slabs[0].rows >= 4))
+      return false;
+    Slab<real>& s = slabs[0];
+    int sms = 0, coop = 0, per_sm = 0;
+    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s.device));
+    CK(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, s.device));
+    // one block per SM if the grid allows it: the fewest rows per block that still fits
+    pairs_tile_rows = std::min(LBM_PAIRS_MAX_TILE_ROWS, std::max(1, (s.rows + sms - 1) / sms));
+    if (const char* e = getenv("LBM_PAIRS_TILE_ROWS"))                      // tuning knob
+      pairs_tile_rows = std::min(LBM_PAIRS_MAX_TILE_ROWS, std::max(1, atoi(e)));
+    pairs_tile_rows = std::min(pairs_tile_rows, s.rows - 2);
+    const dim3 b = pairs_block();
+    const bool ok = coop && cudaFuncSetAttribute(pairs_fn(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pairs_smem()) == cudaSuccess &&
+                    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pairs_fn(), (int)(b.x * b.y), pairs_smem()) == cudaSuccess &&
+                    (long long)per_sm * sms >= (s.rows + pairs_tile_rows - 1) / pairs_tile_rows;
+    cudaGetLastError();
+    return ok;
+  }
+
+  // ------------------------------------------------------------ kernel choice ----
+  // Which kernel runs the lattice, and its launch configuration: the only code that sets
+  // `kernel`.  Runs before anything is allocated, and again when a slab handle joins a ring of
+  // processes (`ring_k7`: lbm_gpu_ipc_connect_all found that every rank can run K7):
+  //   0. refused on flags and shape alone: two kernels, TMA in fp64, binary16 outside one fp32
+  //      lbm_gpu_create slab or with a kernel other than VEC4 or TB2;
+  //   1. a forced kernel where its conditions hold, otherwise a refusal;
+  //   2. a ring: K7 where every rank can run it, otherwise K1a;
+  //   3. one lbm_gpu_create slab in L2 (kPersistMaxCells): K9 where it fits (unless LBM_GPU_NO_PAIRS), else K5;
+  //   4. K7 (K7-f16) where it fits, but not yet on a slab handle that holds part of the grid; K10
+  //      instead on the whole grid in one slab with enough waves of blocks (unless LBM_GPU_NO_TB3);
+  //   5. K1a (K1a-f16).
+  void select_kernel(bool ring = false, bool ring_k7 = false) {
+    const unsigned forced = forced_kernel(flags);
+    if (f16) {
+      if (slab_mode) throw CudaError{"LBM_GPU_STORE_F16 is for lbm_gpu_create lattices only, not slab handles"};
+      if (sizeof(real) != 4) throw CudaError{"LBM_GPU_STORE_F16 is for fp32 lattices only"};
+      if (slabs.size() != 1) throw CudaError{"LBM_GPU_STORE_F16 needs n_gpus == 1 (got " + std::to_string(slabs.size()) + ")"};
+      if (forced & ~(LBM_GPU_KERNEL_VEC4 | LBM_GPU_KERNEL_TB2)) {
+        char msg[160];
+        snprintf(msg, sizeof msg, "LBM_GPU_STORE_F16 runs LBM_GPU_KERNEL_VEC4 or LBM_GPU_KERNEL_TB2 only; "
+                 "another kernel was forced (flags 0x%x)", forced);
+        throw CudaError{msg};
+      }
     }
-    if (ok) kernel = LBM_GPU_KERNEL_PAIRS;
-    else if (want) throw CudaError{"the pairs kernel needs a single-GPU fp32 lattice with nx a multiple of 4 and <= 256 whose "
-                                   "blocks are all resident"};
-  }
-
-  // LBM_GPU_STORE_F16 (one slab, fp32): K7-f16 where K7's shape rules hold and the binary16 bulk copies
-  // can cut the rows (nx a multiple of 8), otherwise K1a-f16; LBM_GPU_KERNEL_VEC4 forces K1a-f16
-  void choose_f16() {
-    const bool tb2_ok = prm.nx % 8 == 0 && prm.nx >= 32 && slabs[0].rows >= kTb2MinRows;
-    if ((flags & LBM_GPU_KERNEL_TB2) && !tb2_ok)
-      throw CudaError{"the two-step kernel with LBM_GPU_STORE_F16 needs nx a multiple of 8 and >= 32, and >= 8 rows"};
-    kernel = LBM_GPU_KERNEL_VEC4;
-    if (tb2_ok && !(flags & LBM_GPU_KERNEL_VEC4)) enable_tb2();
-  }
-
-  // single-process form: decide once all slabs exist
-  void choose_tb2() {
+    if (forced == LBM_GPU_KERNEL_TMA && sizeof(real) != 4) throw CudaError{"the TMA kernel is built for single precision only"};
+    const bool one_slab = slabs.size() == 1 && !slab_mode;
+    const bool partial = slab_mode && slabs[0].rows != prm.ny;
     int rows_min = slabs[0].rows;
     for (auto& s : slabs) rows_min = std::min(rows_min, s.rows);
-    const bool want = (flags & LBM_GPU_KERNEL_TB2) != 0;
-    const bool want3 = (flags & LBM_GPU_KERNEL_TB3) != 0;
-    const bool big = (kernel == LBM_GPU_KERNEL_VEC4);        // not taken by the persistent kernel
-    if (want3 && !tb3_possible())
-      throw CudaError{"the three-step kernel needs fp32, nx a multiple of 4 and >= 32, the whole grid in one slab, "
-                      "and >= 12 rows"};
-    if (tb2_possible(rows_min) && (want || want3 || big)) enable_tb2();
-    else if (want) throw CudaError{"the two-step kernel needs fp32, nx a multiple of 4 and >= 32, and >= 8 rows per slab"};
-    if (want3 || (big && tb3_possible() && tb3_pays())) enable_tb3();
+    CK(cudaSetDevice(slabs[0].device));
+    bool k7 = false;
+    switch (forced) {
+      case 0:
+        if (!ring && !f16 && one_slab && (long long)prm.nx * slabs[0].rows <= kPersistMaxCells && persistent_fits()) {
+          kernel = (!env_on("LBM_GPU_NO_PAIRS") && pairs_fit()) ? LBM_GPU_KERNEL_PAIRS : LBM_GPU_KERNEL_PERSISTENT;
+          return;
+        }
+        k7 = ring ? ring_k7 : !partial && k7_fits(rows_min);
+        break;
+      case LBM_GPU_KERNEL_PERSISTENT:
+        if (!one_slab) throw CudaError{"the persistent kernel handles a single slab only"};
+        if (!persistent_fits()) throw CudaError{"cooperative launch is not available on this device"};
+        break;
+      // K6 is opt-in only: 16 SMs doing all the arithmetic are no faster than K5 spreading it
+      // over the whole chip (profiles/r01_small_grids.md).
+      case LBM_GPU_KERNEL_CLUSTER:
+        if (!cluster_fits()) throw CudaError{"the cluster kernel needs a single-GPU fp32 lattice that fits in one cluster's shared memory"};
+        break;
+      case LBM_GPU_KERNEL_PAIRS:
+        if (!pairs_fit()) throw CudaError{"the pairs kernel needs a single-GPU fp32 lattice with nx a multiple of 4 and <= 256 whose blocks are all resident"};
+        break;
+      case LBM_GPU_KERNEL_TB2:
+        if (ring && !ring_k7)
+          throw CudaError{"the two-step kernel needs lbm_gpu_ipc_connect_all and fp32, nx a multiple of 4 and >= 32, "
+                          ">= 8 rows on every rank"};
+        if (!ring && !partial && !k7_fits(rows_min))
+          throw CudaError{f16 ? "the two-step kernel with LBM_GPU_STORE_F16 needs nx a multiple of 8 and >= 32, and >= 8 rows"
+                              : "the two-step kernel needs fp32, nx a multiple of 4 and >= 32, and >= 8 rows per slab"};
+        k7 = ring || !partial;
+        break;
+      case LBM_GPU_KERNEL_TB3:
+        if (ring) throw CudaError{"the three-step kernel needs the whole grid in one slab"};
+        if (!k10_fits()) throw CudaError{"the three-step kernel needs fp32, nx a multiple of 4 and >= 32, the whole grid in one slab, and >= 12 rows"};
+        k7 = true;
+        break;
+    }
+    if (!k7) {
+      kernel = (forced && forced != LBM_GPU_KERNEL_TB2) ? forced : LBM_GPU_KERNEL_VEC4;
+      return;
+    }
+    configure_tb2();
+    kernel = LBM_GPU_KERNEL_TB2;
+    if (forced == LBM_GPU_KERNEL_TB3 || (!forced && !ring && k10_fits() && tb3_pays())) {
+      configure_tb3();
+      kernel = LBM_GPU_KERNEL_TB3;
+    }
   }
+
+  // timesteps of the kernel's longest pass: K10 three, K7 and K7-f16 two, the others one
+  int max_pass_steps() const { return kernel == LBM_GPU_KERNEL_TB3 ? 3 : kernel == LBM_GPU_KERNEL_TB2 ? 2 : 1; }
 
   // ------------------------------------------------------------- lattice input ----
   // cells: AoS rows for this slab (or NULL -> rest state); obstacles: rows for this slab
@@ -849,7 +864,7 @@ class Grid : public GridBase {
       a.mask_dn = s.dn_gmask;
       a.plane_stride = plane_stride(s);
       a.nx = prm.nx; a.rows = s.rows; a.pitch = pitch; a.mask_pitch = mask_pitch; a.accel_row = s.accel_row;
-      a.deep = tb2 ? 1 : 0;                // K10 reads the source lattice directly: K7's ghost rows are enough
+      a.deep = max_pass_steps() > 1 ? 1 : 0;   // K10 reads the source lattice directly: K7's ghost rows are enough
       a.aw1 = prm.density * prm.accel / (real)9;      // d2q9-bgk.c:230-231
       a.aw2 = prm.density * prm.accel / (real)36;
       lbm::lbm_prepare<real><<<(std::max(prm.nx, mask_pitch) + 127) / 128, 128, 0, s.stream>>>(a);
@@ -1027,8 +1042,8 @@ class Grid : public GridBase {
         if (strict) launch_pdl(s, lbm::lbm_step2_tb_f16<true>, a, grid, dim3(tb2_threads), sizeof(lbm::Tb2hSmem));
         else        launch_pdl(s, lbm::lbm_step2_tb_f16<false>, a, grid, dim3(tb2_threads), sizeof(lbm::Tb2hSmem));
       } else {
-        int vec, bx, by;
-        tile_shape(vec, bx, by);
+        int bx, by;
+        tile_shape(4, bx, by);
         a.tiles_x = ((prm.nx + 3) / 4 + bx - 1) / bx;
         a.tiles_y = (s.rows + by - 1) / by;
         const dim3 grid((unsigned)((long long)a.tiles_x * a.tiles_y)), block(bx, by);
@@ -1044,10 +1059,10 @@ class Grid : public GridBase {
 
   void launch_pass(int t_in_segment, int pass_in_segment, int steps) {
     if (f16) { launch_pass_f16(t_in_segment, steps); return; }
-    const bool two = (steps == 2);
     const bool strict = (flags & LBM_GPU_STRICT) != 0;
     const int nslabs = (int)slabs.size();
-    int vec, bx, by;
+    const int vec = (kernel == LBM_GPU_KERNEL_SCALAR) ? 1 : 4;
+    int bx, by;
     tile_shape(vec, bx, by);
     const int nxv = (prm.nx + vec - 1) / vec;
     for (int si = 0; si < nslabs; si++) {
@@ -1082,7 +1097,7 @@ class Grid : public GridBase {
           if (strict) launch_tb3<true>(s, ta, grid);
           else        launch_tb3<false>(s, ta, grid);
         }
-      } else if (two) {
+      } else if (steps == 2) {
         if constexpr (sizeof(real) == 4) {
           lbm::Tb2Args ta;
           const Tb2Segments sg = tb2_segments(s.rows);
@@ -1108,8 +1123,8 @@ class Grid : public GridBase {
       } else {
         a.tiles_x = (nxv + bx - 1) / bx;
         a.tiles_y = (s.rows + by - 1) / by;
-        a.deep = tb2 ? 1 : 0;                 // a lone step between two-step passes keeps their ghost rows filled
-        a.edge_tiles = tb2 ? (2 + by - 1) / by : 1;   // the tile rows that hold the slab's two edge rows
+        a.deep = max_pass_steps() > 1 ? 1 : 0;     // a lone step between multi-step passes keeps their ghost rows filled
+        a.edge_tiles = a.deep ? (2 + by - 1) / by : 1;   // the tile rows that hold the slab's two edge rows   // the tile rows that hold the slab's two edge rows
         const dim3 grid((unsigned)((long long)a.tiles_x * a.tiles_y));
         const dim3 block(bx, by);
         if (strict) { if (use_flags) launch_step<true, true>(s, a, grid, block, cur); else launch_step<true, false>(s, a, grid, block, cur); }
@@ -1149,7 +1164,8 @@ class Grid : public GridBase {
       launch_cluster(n_steps, strict);
       cur = (cur + n_steps) & 1;
     } else if (kernel == LBM_GPU_KERNEL_PERSISTENT) {
-      int vec, bx, by;
+      const int vec = persistent_vec;
+      int bx, by;
       tile_shape(vec, bx, by);
       const int nxv = (prm.nx + vec - 1) / vec;
       Slab<real>& s = slabs[0];
@@ -1204,7 +1220,7 @@ class Grid : public GridBase {
     } else {
       int t = 0, p = 0;
       while (t < n_steps) {
-        const int steps = (tb3 && n_steps - t >= 3) ? 3 : (tb2 && n_steps - t >= 2) ? 2 : 1;
+        const int steps = std::min(max_pass_steps(), n_steps - t);
         launch_pass(t, p, steps);
         t += steps;
         p++;
@@ -1472,15 +1488,6 @@ int create_impl(const typename ParamT<real>::type* params, const real* cells_aos
   if (params->nx < 1 || params->ny < 2) return fail("lbm_gpu_create: need nx >= 1 and ny >= 2 (got %d x %d)", params->nx, params->ny);
   if (n_gpus < 1) return fail("lbm_gpu_create: n_gpus must be >= 1");
   if (params->ny < n_gpus) return fail("lbm_gpu_create: fewer rows (%d) than GPUs (%d)", params->ny, n_gpus);
-  if (flags & LBM_GPU_STORE_F16) {
-    if (sizeof(real) != 4) return fail("lbm_gpu_create_f64: LBM_GPU_STORE_F16 is for fp32 lattices only");
-    if (n_gpus != 1) return fail("lbm_gpu_create: LBM_GPU_STORE_F16 needs n_gpus == 1 (got %d)", n_gpus);
-    const unsigned forced = LBM_GPU_KERNEL_SCALAR | LBM_GPU_KERNEL_TMA | LBM_GPU_KERNEL_PERSISTENT | LBM_GPU_KERNEL_CLUSTER |
-                            LBM_GPU_KERNEL_PAIRS | LBM_GPU_KERNEL_TB3;
-    if (flags & forced)
-      return fail("lbm_gpu_create: LBM_GPU_STORE_F16 runs LBM_GPU_KERNEL_VEC4 or LBM_GPU_KERNEL_TB2 only; "
-                  "another kernel was forced (flags 0x%x)", flags & forced);
-  }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) {
     cudaGetLastError();
@@ -1496,8 +1503,6 @@ int create_impl(const typename ParamT<real>::type* params, const real* cells_aos
     std::vector<int> rows;
     split_rows(params->ny, n_gpus, row0, rows);
     g->slabs.resize(n_gpus);
-    const size_t cell_row = (size_t)params->nx * 9;
-    const size_t obst_row_bytes = (flags & LBM_GPU_OBST_BITS) ? (size_t)((params->nx + 31) / 32) * 4 : (size_t)params->nx * 4;
     for (int i = 0; i < n_gpus; i++) {
       Slab<real>& s = g->slabs[i];
       s.device = device_ids ? device_ids[i] : i;
@@ -1506,19 +1511,17 @@ int create_impl(const typename ParamT<real>::type* params, const real* cells_aos
       s.rows = rows[i];
       const long long ar = (long long)params->ny - 2;
       s.accel_row = (ar >= s.row0 && ar < s.row0 + s.rows) ? (int)(ar - s.row0) : LBM_NO_ROW;
+    }
+    g->select_kernel();
+    const size_t cell_row = (size_t)params->nx * 9;
+    const size_t obst_row_bytes = (flags & LBM_GPU_OBST_BITS) ? (size_t)((params->nx + 31) / 32) * 4 : (size_t)params->nx * 4;
+    for (Slab<real>& s : g->slabs) {
       g->alloc_slab(s);
       if (g->kernel == LBM_GPU_KERNEL_TMA) g->make_tensor_maps(s);
       g->load_slab(s, cells_aos ? cells_aos + (size_t)s.row0 * cell_row : nullptr,
                    obstacles ? (const char*)obstacles + (size_t)s.row0 * obst_row_bytes : nullptr, 0);
     }
     g->connect_local();
-    if (g->f16) {
-      g->choose_f16();
-    } else {
-      g->choose_kernel();
-      g->choose_pairs();
-      g->choose_tb2();
-    }
     g->prepare();
   } catch (const CudaError& e) {
     return fail("lbm_gpu_create: %s", e.what.c_str());
@@ -1838,7 +1841,6 @@ int lbm_gpu_create_slab(const lbm_param* params, long long row0, long long nrows
   *out = nullptr;
   if (params->nx < 1 || params->ny < 2) return fail("lbm_gpu_create_slab: need nx >= 1 and ny >= 2");
   if (row0 < 0 || nrows < 1 || row0 + nrows > params->ny) return fail("lbm_gpu_create_slab: rows [%lld,%lld) outside the grid", row0, row0 + nrows);
-  if (flags & LBM_GPU_STORE_F16) return fail("lbm_gpu_create_slab: LBM_GPU_STORE_F16 is for lbm_gpu_create lattices only, not slab handles");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) {
     cudaGetLastError();
@@ -1849,6 +1851,7 @@ int lbm_gpu_create_slab(const lbm_param* params, long long row0, long long nrows
   try {
     g->prm = *params;
     g->flags = flags;
+    g->f16 = (flags & LBM_GPU_STORE_F16) != 0;
     g->slab_mode = true;
     g->setup_geometry(params->nx);
     g->slabs.resize(1);
@@ -1858,11 +1861,11 @@ int lbm_gpu_create_slab(const lbm_param* params, long long row0, long long nrows
     s.rows = (int)nrows;
     const long long ar = (long long)params->ny - 2;
     s.accel_row = (ar >= row0 && ar < row0 + nrows) ? (int)(ar - row0) : LBM_NO_ROW;
+    g->select_kernel();
     g->alloc_slab(s);
     if (g->kernel == LBM_GPU_KERNEL_TMA) g->make_tensor_maps(s);
     g->load_slab(s, cells_aos_rows, obstacles_rows, 0);
-    if (g->kernel == LBM_GPU_KERNEL_PERSISTENT) throw CudaError{"the persistent kernel handles a single slab only"};
-    if (nrows == params->ny) { g->connect_local(); g->choose_tb2(); g->prepare(); }   // whole grid in one slab
+    if (nrows == params->ny) { g->connect_local(); g->prepare(); }   // whole grid in one slab
   } catch (const CudaError& e) {
     return fail("lbm_gpu_create_slab: %s", e.what.c_str());
   } catch (const std::exception& e) {
@@ -1895,7 +1898,7 @@ int lbm_gpu_ipc_export(lbm_gpu* h, void* desc) {
     d.passes_done = (unsigned long long)g.passes_done;
     d.local_free_cells = s.free_cells;
     d.cur = g.cur;
-    d.tb2_ok = g.tb2_possible(s.rows) ? 1 : 0;
+    d.tb2_ok = g.k7_fits(s.rows) ? 1 : 0;
     CK(cudaIpcGetMemHandle(&d.handle, s.win));
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, s.device));
@@ -1906,9 +1909,9 @@ int lbm_gpu_ipc_export(lbm_gpu* h, void* desc) {
 }
 
 namespace {
-// wire a one-slab handle to the slabs below and above it; `ring_tb2`: every slab of the ring
+// wire a one-slab handle to the slabs below and above it; `ring_k7`: every slab of the ring
 // can run (and therefore will run) the two-step kernel
-void ipc_connect_impl(Grid<float>& g, const IpcDesc& dn, const IpcDesc& up, bool ring_tb2) {
+void ipc_connect_impl(Grid<float>& g, const IpcDesc& dn, const IpcDesc& up, bool ring_k7) {
   if (g.slabs.size() != 1) throw CudaError{"only a one-slab handle can be connected"};
   if (g.f16) throw CudaError{"a LBM_GPU_STORE_F16 lattice cannot be shared between processes"};
   Slab<float>& s = g.slabs[0];
@@ -1979,14 +1982,7 @@ void ipc_connect_impl(Grid<float>& g, const IpcDesc& dn, const IpcDesc& up, bool
   s.up_gmask = (uint32_t*)(s.up_win + up.off_gmask);
   g.multi = true;
   g.use_flags = true;      // neighbours are other processes: device-side flags
-  if (g.flags & LBM_GPU_KERNEL_TB3) throw CudaError{"the three-step kernel needs the whole grid in one slab"};
-  g.tb3 = false;                   // a ring of slabs: K7 at most
-  if (g.kernel == LBM_GPU_KERNEL_TB3) g.kernel = LBM_GPU_KERNEL_VEC4;
-  if (g.flags & LBM_GPU_KERNEL_TB2) {
-    if (!ring_tb2) throw CudaError{"the two-step kernel needs lbm_gpu_ipc_connect_all and fp32, nx a multiple of 4 "
-                                   "and >= 32, >= 8 rows on every rank"};
-  }
-  if (ring_tb2) g.enable_tb2();
+  g.select_kernel(true, ring_k7);
   g.connected = true;
 }
 }  // namespace
@@ -2011,19 +2007,19 @@ int lbm_gpu_ipc_connect_all(lbm_gpu* h, const void* descs, int n) {
     const long long ny = g.prm.ny;
     long long rows_total = 0, free_total = 0;
     int below = -1, above = -1;
-    bool all_tb2 = true;
+    bool all_k7 = true;
     for (int i = 0; i < n; i++) {
       const IpcDesc& d = all[i];
       if (d.magic != kIpcMagic) throw CudaError{"bad descriptor in the list"};
       rows_total += d.rows;
       free_total += d.local_free_cells;
-      all_tb2 = all_tb2 && d.tb2_ok && d.rows >= kTb2MinRows;
+      all_k7 = all_k7 && d.tb2_ok;
       if ((d.row0 + d.rows) % ny == s.row0 % ny) below = i;
       if ((s.row0 + s.rows) % ny == d.row0 % ny) above = i;
     }
     if (rows_total != ny) throw CudaError{"the descriptors do not cover the grid's rows exactly once"};
     if (below < 0 || above < 0) throw CudaError{"no descriptor holds the rows next to this slab"};
-    ipc_connect_impl(g, all[below], all[above], all_tb2);
+    ipc_connect_impl(g, all[below], all[above], all_k7);
     g.global_free_cells = free_total;
   });
 }

@@ -55,7 +55,7 @@ typedef struct {
 
 typedef struct lbm_gpu lbm_gpu;   /* opaque handle: one lattice on one or more GPUs */
 
-/* lbm_gpu_create flags */
+/* lbm_gpu_create flags.  At most one LBM_GPU_KERNEL_* flag: a create that forces two is refused. */
 #define LBM_GPU_DEFAULT        0u
 #define LBM_GPU_STRICT         1u  /* source operation order, no FMA contraction: bit-exact
                                       against a -O2 -ffp-contract=off build of the reference */
@@ -115,7 +115,8 @@ typedef struct {
   int       nx, ny;
   int       n_gpus;            /* slabs held by THIS process */
   int       is_f64;
-  int       kernel;            /* LBM_GPU_KERNEL_* actually selected */
+  int       kernel;            /* LBM_GPU_KERNEL_* that runs the next lbm_gpu_run (chosen at create,
+                                  again at lbm_gpu_ipc_connect / _connect_all) */
   int       pitch;             /* elements per stored lattice row */
   long long free_cells;        /* non-obstacle cells of the WHOLE grid (if known) or of the local rows */
   long long local_free_cells;  /* non-obstacle cells of the rows held by this process */
@@ -159,8 +160,10 @@ int lbm_gpu_create_f64(const lbm_param_f64* params, const double* cells_aos, con
  *      descriptors of ALL ranks and call lbm_gpu_ipc_connect_all(): the library then finds
  *      its two neighbours itself, learns the whole grid's free-cell count (so lbm_gpu_run
  *      returns true averages without lbm_gpu_set_global_free_cells) and, knowing every
- *      slab's height, may select the two-timesteps-per-pass kernel, a decision all ranks
- *      must share (with the two-descriptor form the one-step kernel is kept),
+ *      slab's height, selects the two-timesteps-per-pass kernel where every rank can run
+ *      it, a decision all ranks must share.  Otherwise, and always with the two-descriptor
+ *      form, a ring runs the one-step kernel (unless another was forced), also on a slab
+ *      that holds the whole grid and took a multi-step kernel at create,
  *   4. pass a host barrier over all ranks, then lbm_gpu_ipc_prepare(), then a second
  *      host barrier -- after which lbm_gpu_run() may be called (same n_steps on
  *      every rank).
