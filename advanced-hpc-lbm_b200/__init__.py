@@ -7,13 +7,13 @@ the tests and the benchmark driver.  The directory name contains hyphens, so imp
 it with importlib.import_module("advanced-hpc-lbm_b200") or through the root-level
 shim `lbm_b200`.
 """
-from .binding import (IPC_DESC_BYTES, KERNEL_CLUSTER, KERNEL_PAIRS, KERNEL_PERSISTENT, KERNEL_SCALAR, KERNEL_TB2, KERNEL_TB3, KERNEL_TMA, KERNEL_VEC4, LIB_PATH, OBST_BITS, POOL, STORE_F16, STRICT,
+from .binding import (FIELDS_F16, FIELDS_F32, IPC_DESC_BYTES, KERNEL_CLUSTER, KERNEL_PAIRS, KERNEL_PERSISTENT, KERNEL_SCALAR, KERNEL_TB2, KERNEL_TB3, KERNEL_TMA, KERNEL_VEC4, LIB_PATH, OBST_BITS, POOL, STORE_F16, STRICT,
                       SYNC_EVENTS, SYNC_FLAGS,
                       SYMBOLS, Info, Lattice, LbmError, Param, ParamF64, PinnedArray, lattice_checksum, load_library,
                       pack_obstacle_bits, run_batch)
 from .slabs import split_rows, ring_neighbours
 
-__all__ = ["IPC_DESC_BYTES", "KERNEL_CLUSTER", "KERNEL_PAIRS", "KERNEL_PERSISTENT", "KERNEL_SCALAR", "KERNEL_TB2", "KERNEL_TB3", "KERNEL_TMA", "KERNEL_VEC4", "LIB_PATH", "OBST_BITS", "POOL", "STORE_F16", "STRICT",
+__all__ = ["FIELDS_F16", "FIELDS_F32", "IPC_DESC_BYTES", "KERNEL_CLUSTER", "KERNEL_PAIRS", "KERNEL_PERSISTENT", "KERNEL_SCALAR", "KERNEL_TB2", "KERNEL_TB3", "KERNEL_TMA", "KERNEL_VEC4", "LIB_PATH", "OBST_BITS", "POOL", "STORE_F16", "STRICT",
            "SYNC_EVENTS", "SYNC_FLAGS",
            "SYMBOLS", "Info", "Lattice", "LbmError", "Param", "ParamF64", "PinnedArray", "lattice_checksum", "load_library",
            "pack_obstacle_bits", "run_batch", "split_rows", "ring_neighbours"]

@@ -31,6 +31,9 @@ KERNEL_PAIRS = 2048
 KERNEL_TB3 = 4096
 STORE_F16 = 8192
 IPC_DESC_BYTES = 256
+# lbm_gpu_coarse_fields formats
+FIELDS_F32 = 0
+FIELDS_F16 = 1
 
 
 class LbmError(RuntimeError):
@@ -81,6 +84,7 @@ SYMBOLS = {
     "lbm_gpu_download_rows": (C.c_int, [_P, C.c_longlong, C.c_longlong, _P]),
     "lbm_gpu_final_fields": (C.c_int, [_P, C.c_longlong, C.c_longlong, _P, _P, _P, _P]),
     "lbm_gpu_av_velocity": (C.c_int, [_P, _P]),
+    "lbm_gpu_coarse_fields": (C.c_int, [_P, C.c_int, C.c_uint, C.c_longlong, C.c_longlong, _P, _P, _P, _P]),
     "lbm_gpu_download_f64": (C.c_int, [_P, _P]),
     "lbm_gpu_final_fields_f64": (C.c_int, [_P, C.c_longlong, C.c_longlong, _P, _P, _P, _P]),
     "lbm_gpu_av_velocity_f64": (C.c_int, [_P, _P]),
@@ -283,6 +287,29 @@ class Lattice:
             out = [np.empty((nrows, self.nx), dtype=self.dtype) for _ in range(4)]
         fn = self.lib.lbm_gpu_final_fields_f64 if self.f64 else self.lib.lbm_gpu_final_fields
         _check(fn(self.h, int(row0), int(nrows), *[_ptr(o) for o in out]))
+        return tuple(out)
+
+    def coarse_rows(self, factor):
+        """(crow0, ncrows): the coarse rows of `factor` whose fine rows this handle holds entirely."""
+        ncy = -(-self.ny // factor)
+        end = self.row0 + self.rows
+        first = -(-self.row0 // factor)
+        last = ncy if end == self.ny else end // factor
+        return first, max(0, last - first)
+
+    def coarse_fields(self, factor, f16=False, crow0=None, ncrows=None, out=None):
+        """Block means over factor x factor cells of (u_x, u_y, |u|, pressure), computed on the GPU
+        (lbm_gpu_coarse_fields): four arrays of shape (ncrows, ceil(nx / factor)), float32, or with
+        f16 float16 holding the pressure shifted by p0 = float32(density) * float32(1/3) (decode
+        it as float32(h) + p0).  By default every coarse row this handle holds entirely."""
+        d0, dn = self.coarse_rows(factor)
+        crow0 = d0 if crow0 is None else crow0
+        ncrows = dn if ncrows is None else ncrows
+        if out is None:
+            ncx = -(-self.nx // factor)
+            out = [np.empty((max(ncrows, 0), ncx), dtype=np.float16 if f16 else np.float32) for _ in range(4)]
+        _check(self.lib.lbm_gpu_coarse_fields(self.h, int(factor), FIELDS_F16 if f16 else FIELDS_F32, int(crow0),
+                                              int(ncrows), *[_ptr(o) for o in out]))
         return tuple(out)
 
     def av_velocity(self):

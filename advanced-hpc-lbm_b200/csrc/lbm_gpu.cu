@@ -22,6 +22,7 @@
 #include <exception>
 #include <memory>
 #include <mutex>
+#include <numeric>
 #include <string>
 #include <vector>
 
@@ -1407,6 +1408,136 @@ class Grid : public GridBase {
     }
   }
 
+  // Block means of the fields (lbm_gpu_coarse_fields; the arithmetic is in lbm_coarse_fields).
+  // Coarse rows that lie wholly in one slab go through the staging buffer as final_fields'
+  // rows do: chunk by chunk into one half (kernel stream), copied out from the other (copy
+  // stream), one synchronisation per call.  A coarse row cut by a boundary between two slabs
+  // of this process (at most one per boundary) comes after them: each slab's integer sums are
+  // copied back and added here, and the host computes the same means the kernel would.
+  template <typename out_t>
+  void launch_coarse(Slab<real>& s, int factor, int nc, long long J0, int n, out_t* const (&d)[4],
+                     unsigned long long* raw) {
+    const int ncx = (prm.nx + factor - 1) / factor;
+    const dim3 grid((unsigned)((ncx + nc - 1) / nc), (unsigned)n);
+    const unsigned threads = (unsigned)round_up((nc * factor + 3) / 4, 32);
+    const size_t smem = factor == 1 ? 0 : (size_t)nc * (4 * sizeof(unsigned long long) + sizeof(unsigned));
+    if (f16)
+      lbm::lbm_coarse_fields<__half, out_t><<<grid, threads, smem, s.stream>>>(
+          hlat(s, cur), s.mask, plane_stride(s), pitch, mask_pitch, prm.nx, prm.ny, s.row0, s.rows, factor, nc, ncx,
+          J0, (float)prm.density, rest(), d[0], d[1], d[2], d[3], raw);
+    else
+      lbm::lbm_coarse_fields<float, out_t><<<grid, threads, smem, s.stream>>>(
+          (const float*)s.lattice[cur], s.mask, plane_stride(s), pitch, mask_pitch, prm.nx, prm.ny, s.row0, s.rows,
+          factor, nc, ncx, J0, (float)prm.density, rest(), d[0], d[1], d[2], d[3], raw);
+    CK(cudaGetLastError());
+    launches++;
+  }
+
+  void coarse_fields(int factor, bool half_out, long long crow0, long long ncrows, void* const (&out)[4]) {
+    const int nx = prm.nx;
+    const long long ny = prm.ny;
+    const int ncx = (nx + factor - 1) / factor;
+    const long long ncy = (ny + factor - 1) / factor;
+    if (ncrows == 0) return;
+    if (crow0 < 0 || crow0 + ncrows > ncy)
+      throw CudaError{"coarse rows [" + std::to_string(crow0) + ", " + std::to_string(crow0 + ncrows) +
+                      ") are not all in the grid's " + std::to_string(ncy) + " coarse rows"};
+    long long held = 0;
+    for (auto& s : slabs) held += s.rows;
+    const long long h0 = slabs[0].row0, h1 = h0 + held;
+    const long long first = crow0 * factor < h0 ? crow0 : (std::min((crow0 + ncrows) * factor, ny) > h1 ? std::max(crow0, h1 / factor) : -1);
+    if (first >= 0) {
+      char b[256];
+      snprintf(b, sizeof b, "coarse row %lld needs global rows [%lld, %lld), and this process holds rows [%lld, %lld)",
+               first, first * factor, std::min(first * factor + factor, ny), h0, h1);
+      throw CudaError{b};
+    }
+    if (factor == 1 && !half_out) {                   // the per-cell fields themselves
+      final_fields(crow0, ncrows, (real*)out[0], (real*)out[1], (real*)out[2], (real*)out[3]);
+      return;
+    }
+    const size_t es = half_out ? sizeof(__half) : sizeof(float);
+    const size_t half = kStagingBytes / 2;
+    const size_t row_bytes = 4 * (size_t)ncx * es;
+    if (row_bytes > half || (slabs.size() > 1 && (size_t)ncx * lbm::kCoarseRawWords * 8 > kStagingBytes))
+      throw CudaError{"nx too large for the coarse fields staging buffer"};
+    // coarse columns per block: nc * factor <= kCoarseSpan and a multiple of 4 (aligned quads)
+    int nc = lbm::kCoarseSpan / factor;
+    nc -= nc % (4 / std::gcd(factor, 4));
+    nc = std::min(nc, ncx);
+    const int chunk = (int)std::min<size_t>(half / row_bytes, 65535);
+    std::vector<Slab<real>*> used;
+    std::vector<long long> cut;
+    long long J = crow0;
+    int i = 0;
+    while (J < crow0 + ncrows) {
+      Slab<real>& s = slab_of_row(J * factor);
+      const long long s_end = s.row0 + s.rows;
+      if (std::min(J * factor + factor, ny) > s_end) { cut.push_back(J++); continue; }
+      const long long whole_end = s_end == ny ? ncy : s_end / factor;     // first coarse row not wholly in s
+      const int n = (int)std::min<long long>({(long long)chunk, whole_end - J, crow0 + ncrows - J});
+      CK(cudaSetDevice(s.device));
+      if (used.empty() || used.back() != &s) {
+        used.push_back(&s);
+        i = 0;
+      }
+      const int b = i & 1;
+      char* st = (char*)s.staging + (size_t)b * half;
+      const size_t plane = (size_t)n * ncx * es;
+      void* d[4];
+      for (int k = 0; k < 4; k++) d[k] = out[k] ? st + k * plane : nullptr;
+      if (i >= 2) CK(cudaStreamWaitEvent(s.stream, s.stage_drained[b], 0));
+      if (half_out) {
+        __half* const dh[4] = {(__half*)d[0], (__half*)d[1], (__half*)d[2], (__half*)d[3]};
+        launch_coarse<__half>(s, factor, nc, J, n, dh, nullptr);
+      } else {
+        float* const df[4] = {(float*)d[0], (float*)d[1], (float*)d[2], (float*)d[3]};
+        launch_coarse<float>(s, factor, nc, J, n, df, nullptr);
+      }
+      CK(cudaEventRecord(s.stage_filled[b], s.stream));
+      CK(cudaStreamWaitEvent(s.copy_stream, s.stage_filled[b], 0));
+      const size_t off = (size_t)(J - crow0) * ncx * es;
+      for (int k = 0; k < 4; k++)
+        if (out[k]) CK(cudaMemcpyAsync((char*)out[k] + off, d[k], plane, cudaMemcpyDeviceToHost, s.copy_stream));
+      CK(cudaEventRecord(s.stage_drained[b], s.copy_stream));
+      J += n;
+      i++;
+    }
+    for (Slab<real>* s : used) {
+      CK(cudaSetDevice(s->device));
+      CK(cudaStreamSynchronize(s->copy_stream));
+      CK(cudaStreamSynchronize(s->stream));
+    }
+    if (cut.empty()) return;
+    const float p0 = (float)prm.density * (1.0f / 3.0f);
+    std::vector<unsigned long long> tot(ncx * lbm::kCoarseRawWords), part(tot.size());
+    for (const long long Jc : cut) {
+      const long long g0 = Jc * factor, g1 = std::min(g0 + factor, ny);
+      std::fill(tot.begin(), tot.end(), 0ULL);
+      for (auto& s : slabs) {
+        if (s.row0 >= g1 || s.row0 + s.rows <= g0) continue;
+        CK(cudaSetDevice(s.device));
+        float* const none[4] = {nullptr, nullptr, nullptr, nullptr};
+        launch_coarse<float>(s, factor, nc, Jc, 1, none, (unsigned long long*)s.staging);
+        CK(cudaMemcpyAsync(part.data(), s.staging, part.size() * 8, cudaMemcpyDeviceToHost, s.stream));
+        CK(cudaStreamSynchronize(s.stream));
+        for (size_t w = 0; w < tot.size(); w++)
+          tot[w] = (w % lbm::kCoarseRawWords == 4) ? (tot[w] | part[w]) : tot[w] + part[w];
+      }
+      for (int C = 0; C < ncx; C++) {
+        const unsigned long long* w = &tot[(size_t)C * lbm::kCoarseRawWords];
+        const double cells = (double)((g1 - g0) * (long long)std::min(factor, nx - C * factor));
+        const size_t o = (size_t)(Jc - crow0) * ncx + C;
+        for (int k = 0; k < 4; k++) {
+          if (!out[k]) continue;
+          const float m = ((w[4] >> k) & 1) ? std::nanf("") : (float)((double)(long long)w[k] * 0x1p-32 / cells);
+          if (half_out) ((__half*)out[k])[o] = __float2half_rn(k == 3 ? m - p0 : m);
+          else ((float*)out[k])[o] = m;
+        }
+      }
+    }
+  }
+
   double av_velocity_sum() {
     unsigned __int128 tot = 0;
     bool bad = false;
@@ -2080,6 +2211,20 @@ int lbm_gpu_final_fields(lbm_gpu* h, long long row0, long long nrows, float* ux,
 int lbm_gpu_final_fields_f64(lbm_gpu* h, long long row0, long long nrows, double* ux, double* uy, double* u, double* p) {
   if (nrows < 0) return fail("lbm_gpu_final_fields_f64: bad argument");
   return guarded<double>(h, "lbm_gpu_final_fields_f64", [&](Grid<double>& g) { g.final_fields(row0, nrows, ux, uy, u, p); });
+}
+
+int lbm_gpu_coarse_fields(lbm_gpu* h, int factor, unsigned format, long long crow0, long long ncrows,
+                          void* ux, void* uy, void* u, void* p) {
+  if (factor < 1 || factor > 256) return fail("lbm_gpu_coarse_fields: factor %d is not in 1..256", factor);
+  if (format != LBM_GPU_FIELDS_F32 && format != LBM_GPU_FIELDS_F16)
+    return fail("lbm_gpu_coarse_fields: unknown format %u", format);
+  if (ncrows < 0) return fail("lbm_gpu_coarse_fields: negative ncrows");
+  if (h && reinterpret_cast<GridBase*>(h)->is_f64())
+    return fail("lbm_gpu_coarse_fields: double-precision handles are not served (use lbm_gpu_final_fields_f64)");
+  return guarded<float>(h, "lbm_gpu_coarse_fields", [&](Grid<float>& g) {
+    void* const out[4] = {ux, uy, u, p};
+    g.coarse_fields(factor, format == LBM_GPU_FIELDS_F16, crow0, ncrows, out);
+  });
 }
 
 int lbm_gpu_av_velocity(lbm_gpu* h, float* av_out) {

@@ -1339,6 +1339,165 @@ __global__ void lbm_fields(const store* __restrict__ buf, const uint32_t* __rest
   if (av) warp_accumulate(q, av);
 }
 
+// Block means of lbm_fields' values (lbm_gpu_coarse_fields, include/lbm_gpu.h).  The grid is cut
+// into factor x factor blocks from global cell (0,0).  blockIdx.y is one band, coarse row
+// J0 + blockIdx.y, restricted to the rows [s_row0, s_row0 + s_rows) this slab holds; blockIdx.x
+// is a run of `nc` coarse columns.  nc * factor is a multiple of 4, so thread t's column quad,
+// starting at x = C0 * factor + 4t, is aligned for one 128-bit load per plane (64-bit for
+// binary16); the thread walks down the band.  Each cell's (u_x, u_y, |u|, pressure) is
+// lbm_fields' value bit for bit and enters its block's sum as round_half_even(v * 2^32) in int64:
+// integer sums are exact in any order, so the threads' sums meet per coarse column in shared
+// memory with atomics, for any factor.  With factor >= 2 a quad touches at most two coarse
+// columns: the first `split` of its columns belong to the first.  A value that is not finite or
+// of magnitude kCoarseLimit or more marks its field of the block instead; below that bound a
+// 256 x 256 block's sum stays under 2^63.
+//   raw == nullptr  every band lies wholly in this slab: the block writes the means, fp32 or
+//                   binary16 (pressure shifted by p0, the obstacle pressure), ncx per output row;
+//   raw != nullptr  partial sums of a band cut by a slab boundary, kCoarseRawWords per block
+//                   (four sums, then the mark bits), for the host to add across slabs.
+// factor == 1 (binary16 output only): each cell's values are converted directly, no sums.
+constexpr float kCoarseLimit = 32768.0f;             // 2^15
+constexpr int kCoarseSpan = 1024;                    // columns per block, at most
+constexpr int kCoarseThreads = kCoarseSpan / 4;
+constexpr int kCoarseRawWords = 5;
+
+__device__ __forceinline__ void load_quad(const float* p, int, const RestShift&, float (&v)[4]) {
+  const float4 q = *reinterpret_cast<const float4*>(p);
+  v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+}
+__device__ __forceinline__ void load_quad(const __half* p, const int k, const RestShift& r, float (&v)[4]) {
+  const uint2 q = *reinterpret_cast<const uint2*>(p);
+  const __half2 a = *reinterpret_cast<const __half2*>(&q.x), b = *reinterpret_cast<const __half2*>(&q.y);
+  const float c = r.of(k);
+  v[0] = f16_dec(__low2half(a), c); v[1] = f16_dec(__high2half(a), c);
+  v[2] = f16_dec(__low2half(b), c); v[3] = f16_dec(__high2half(b), c);
+}
+// an output value; binary16 outputs hold v - shift (0 for the velocities, p0 for the pressure)
+__device__ __forceinline__ void put_field(float* o, const float v, float) { *o = v; }
+__device__ __forceinline__ void put_field(__half* o, const float v, const float shift) { *o = __float2half_rn(__fsub_rn(v, shift)); }
+
+__device__ __forceinline__ void add_fixed(unsigned long long& acc, unsigned& mark, const unsigned bit, const float v) {
+  if (::fabsf(v) < kCoarseLimit) acc += (unsigned long long)__float2ll_rn(__fmul_rn(v, 4294967296.0f));
+  else mark |= bit;                                  // NaN lands here too
+}
+
+template <typename store, typename out_t>
+__global__ void __launch_bounds__(kCoarseThreads)
+lbm_coarse_fields(const store* __restrict__ buf, const uint32_t* __restrict__ mask, long long plane_stride,
+                  int pitch, int mask_pitch, int nx, int ny, long long s_row0, int s_rows, int factor, int nc,
+                  int ncx, long long J0, float density, RestShift rest, out_t* __restrict__ ux_out,
+                  out_t* __restrict__ uy_out, out_t* __restrict__ u_out, out_t* __restrict__ p_out,
+                  unsigned long long* __restrict__ raw) {
+  extern __shared__ unsigned long long coarse_sm[];  // nc x 4 sums, then nc mark words
+  typedef Ops<float, true> M;
+  const float c_sq = 1.0f / 3.0f;
+  const float p0 = M::mul(density, c_sq);
+  const long long g0 = (J0 + blockIdx.y) * factor, g1 = ::min(g0 + factor, (long long)ny);   // global rows
+  const int r0 = (int)(::max(g0, s_row0) - s_row0);                                           // local rows
+  const int r1 = (int)(::min(g1, s_row0 + s_rows) - s_row0);
+  const int C0 = blockIdx.x * nc;
+  const int ncb = ::min(nc, ncx - C0);
+  const int xend = ::min((C0 + ncb) * factor, nx);
+  const int x4 = C0 * factor + 4 * (int)threadIdx.x;
+  const int nvalid = ::min(4, xend - x4);
+  const long long orow = (long long)blockIdx.y * ncx;
+
+  if (factor == 1) {
+    if (nvalid <= 0) return;
+    float f[9][4];
+#pragma unroll
+    for (int k = 0; k < 9; k++) load_quad(buf + k * plane_stride + (long long)r0 * pitch + x4, k, rest, f[k]);
+    const uint32_t ob = mask[(long long)r0 * mask_pitch + (x4 >> 5)] >> (x4 & 31);
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+      if (j >= nvalid) break;
+      float cell[9];
+#pragma unroll
+      for (int k = 0; k < 9; k++) cell[k] = f[k][j];
+      float ux, uy, rho;
+      float u = cell_macroscopic<float>(cell, ux, uy, rho);
+      float pr = M::mul(rho, c_sq);
+      if ((ob >> j) & 1u) { ux = 0; uy = 0; u = 0; pr = p0; }
+      const long long o = orow + x4 + j;
+      if (ux_out) put_field(ux_out + o, ux, 0.0f);
+      if (uy_out) put_field(uy_out + o, uy, 0.0f);
+      if (u_out) put_field(u_out + o, u, 0.0f);
+      if (p_out) put_field(p_out + o, pr, p0);
+    }
+    return;
+  }
+
+  unsigned long long* sums = coarse_sm;
+  unsigned* marks = reinterpret_cast<unsigned*>(coarse_sm + 4 * nc);
+  for (int i = threadIdx.x; i < 4 * nc; i += blockDim.x) sums[i] = 0ULL;
+  for (int i = threadIdx.x; i < nc; i += blockDim.x) marks[i] = 0u;
+  __syncthreads();
+  if (nvalid > 0) {
+    const int lo = x4 / factor;                      // coarse column of the quad's first column
+    const int split = ::min(4, (lo + 1) * factor - x4);
+    unsigned long long a0[4] = {0ULL, 0ULL, 0ULL, 0ULL}, a1[4] = {0ULL, 0ULL, 0ULL, 0ULL};
+    unsigned mark = 0u;                              // bit 4 * (second column) + field
+    for (int r = r0; r < r1; r++) {
+      float f[9][4];
+#pragma unroll
+      for (int k = 0; k < 9; k++) load_quad(buf + k * plane_stride + (long long)r * pitch + x4, k, rest, f[k]);
+      const uint32_t ob = mask[(long long)r * mask_pitch + (x4 >> 5)] >> (x4 & 31);
+#pragma unroll
+      for (int j = 0; j < 4; j++) {
+        if (j >= nvalid) break;
+        float cell[9];
+#pragma unroll
+        for (int k = 0; k < 9; k++) cell[k] = f[k][j];
+        float ux, uy, rho;
+        float u = cell_macroscopic<float>(cell, ux, uy, rho);
+        float pr = M::mul(rho, c_sq);
+        if ((ob >> j) & 1u) { ux = 0; uy = 0; u = 0; pr = p0; }
+        if (j < split) {
+          add_fixed(a0[0], mark, 1u, ux); add_fixed(a0[1], mark, 2u, uy);
+          add_fixed(a0[2], mark, 4u, u); add_fixed(a0[3], mark, 8u, pr);
+        } else {
+          add_fixed(a1[0], mark, 16u, ux); add_fixed(a1[1], mark, 32u, uy);
+          add_fixed(a1[2], mark, 64u, u); add_fixed(a1[3], mark, 128u, pr);
+        }
+      }
+    }
+    const int c = lo - C0;
+#pragma unroll
+    for (int i = 0; i < 4; i++)
+      if (a0[i]) atomicAdd(sums + 4 * c + i, a0[i]);
+    if (mark & 15u) atomicOr(marks + c, mark & 15u);
+    if (split < nvalid) {
+#pragma unroll
+      for (int i = 0; i < 4; i++)
+        if (a1[i]) atomicAdd(sums + 4 * (c + 1) + i, a1[i]);
+      if (mark >> 4) atomicOr(marks + c + 1, mark >> 4);
+    }
+  }
+  __syncthreads();
+  for (int c = threadIdx.x; c < ncb; c += blockDim.x) {
+    const int C = C0 + c;
+    const unsigned m = marks[c];
+    if (raw) {
+      unsigned long long* w = raw + (orow + C) * kCoarseRawWords;
+#pragma unroll
+      for (int i = 0; i < 4; i++) w[i] = sums[4 * c + i];
+      w[4] = m;
+      continue;
+    }
+    const double cells = (double)((g1 - g0) * (long long)::min(factor, nx - C * factor));
+    float mean[4];
+#pragma unroll
+    for (int i = 0; i < 4; i++)
+      mean[i] = ((m >> i) & 1u) ? __int_as_float(0x7fffffff)
+                                : __double2float_rn(__ddiv_rn(__dmul_rn(__ll2double_rn((long long)sums[4 * c + i]),
+                                                                        0x1p-32), cells));
+    if (ux_out) put_field(ux_out + orow + C, mean[0], 0.0f);
+    if (uy_out) put_field(uy_out + orow + C, mean[1], 0.0f);
+    if (u_out) put_field(u_out + orow + C, mean[2], 0.0f);
+    if (p_out) put_field(p_out + orow + C, mean[3], p0);
+  }
+}
+
 // Digest of the lattice rows [r0, r0+nrows): two wrapping 64-bit integer sums, so they
 // are exact, order-independent and additive over slabs / ranks.
 //   mass      sum over cells and speeds of round(f * 2^32): total_density of the reference

@@ -248,6 +248,48 @@ int lbm_gpu_final_fields(lbm_gpu* h, long long row0, long long nrows,
                          float* u_x, float* u_y, float* u, float* pressure);
 int lbm_gpu_av_velocity(lbm_gpu* h, float* av_out);
 
+/*
+ * Block-averaged fields, computed on the device so that only the coarse picture crosses PCIe
+ * (a snapshot of a grid too large to read out cell by cell, or a time series of one).
+ * The grid is cut into factor x factor blocks from cell (0,0): ncx = ceil(nx/factor) blocks per
+ * coarse row, ceil(ny/factor) coarse rows; coarse row J covers global rows [J*factor,
+ * min(J*factor + factor, ny)), and the blocks at the right and top edges are smaller.  Each
+ * non-NULL output receives ncrows x ncx values, row-major, of coarse rows [crow0, crow0+ncrows).
+ *
+ * The value of a block is the mean over ALL its cells (obstacle cells included, with the
+ * 0, 0, 0, density/3 that final_fields reports for them) of lbm_gpu_final_fields' per-cell values,
+ * bit for bit; for u_x and u_y that is the superficial (volume-averaged) velocity, so the coarse
+ * field carries the flux of the fine one.  The arithmetic is exact and the same for any slab
+ * split: each cell value v adds round_half_even(v * 2^32) to an int64 sum S, and the mean is
+ * (float)((double)S * 2^-32 / cells), computed in double and rounded once to fp32.  A block in
+ * which a value is NaN, infinite or of magnitude 2^15 or more reports NaN for that field (below
+ * that bound the sum of a 256 x 256 block stays under 2^63).
+ *
+ *   LBM_GPU_FIELDS_F32  float outputs: the mean.
+ *   LBM_GPU_FIELDS_F16  binary16 outputs (uint16_t bit patterns), half the bytes: u_x, u_y and |u|
+ *                       hold __float2half_rn(mean); pressure is shifted, as the lattice is under
+ *                       LBM_GPU_STORE_F16, because it varies by ~1e-4 relative around density/3
+ *                       and binary16 keeps 11 bits: it holds __float2half_rn(mean - p0), the
+ *                       subtraction in fp32, with p0 = (float)density * (1.0f/3.0f) the obstacle
+ *                       pressure of final_fields.  Decode it as __half2float(h) + p0.
+ * factor == 1:  with F16 each cell's own values are converted (pressure shifted): the
+ * full-resolution read-out at half the size, with no fixed-point step; with F32 the call is
+ * lbm_gpu_final_fields.
+ *
+ * factor 1..256.  A handle with several slabs in this process adds the integer sums of a
+ * coarse row cut by a slab boundary on the host, so the result equals one slab's bit for bit.
+ * A slab handle (one process per GPU) serves the coarse rows whose fine rows it holds entirely;
+ * a request for any other coarse row is refused with a message that names it.  Refused before
+ * anything is enqueued or written: factor out of range, an unknown format, ncrows < 0, coarse
+ * rows beyond the grid or not held, and double-precision handles (use
+ * lbm_gpu_final_fields_f64).  ncrows = 0 succeeds and writes nothing.  The lattice, steps_done
+ * and the kernel choice are not touched, so run(a); coarse_fields; run(b) equals run(a+b).
+ */
+#define LBM_GPU_FIELDS_F32 0u
+#define LBM_GPU_FIELDS_F16 1u
+int lbm_gpu_coarse_fields(lbm_gpu* h, int factor, unsigned format, long long crow0, long long ncrows,
+                          void* u_x, void* u_y, void* u, void* pressure);
+
 int lbm_gpu_download_f64(lbm_gpu* h, double* cells_aos_out);
 int lbm_gpu_final_fields_f64(lbm_gpu* h, long long row0, long long nrows,
                              double* u_x, double* u_y, double* u, double* pressure);
