@@ -8,8 +8,9 @@
 //
 // Step t inside the kernel (same per-cell arithmetic as every other kernel -- cell_update,
 // cell_accelerate -- so the results are bit-identical):
-//   every thread pulls the nine values of each of its cells from buffer `cur` (own band, or
-//   the band of the CTA below/above via DSMEM), collides, adds |u| to the step's sum and
+//   every thread pulls the nine values of each of its cells (default build: of each of its
+//   x-aligned quads of cells) from buffer `cur` (own band, or the band of the CTA
+//   below/above via DSMEM), collides, adds |u| to the step's sum and
 //   stores the result into its own band of buffer `cur ^ 1`; row ny-2 is stored WITH the
 //   next step's accelerate_flow applied (d2q9-bgk.c:229-260), except after the last step;
 //   cluster barrier; the buffers swap roles.
@@ -83,9 +84,9 @@ lbm_steps_cluster(const __grid_constant__ ClusterArgs a) {
     const float* rd_above = above + cur * buffer;
     unsigned long long* av_step = a.av + (size_t)t * (LBM_AV_STRIDE * LBM_AV_SLOTS);
     const bool last_step = (t == a.n_steps - 1);
-    unsigned long long q = 0ULL;
-    for (int c = tid; c < my_cells; c += LBM_CLUSTER_THREADS) {
-      const int yl = c / nx, x = c - yl * nx, y = y0 + yl;
+    // one cell: collide, store into buffer `wr`, return |u| (0 for an obstacle cell)
+    auto update = [&](const int yl, const int x) -> float {
+      const int c = yl * nx + x, y = y0 + yl;
       const int xw = (x == 0) ? nx - 1 : x - 1;
       const int xe = (x + 1 == nx) ? 0 : x + 1;
       const float* c_row = rd + yl * nx;
@@ -103,13 +104,36 @@ lbm_steps_cluster(const __grid_constant__ ClusterArgs a) {
       p[7] = n_row[7 * plane + xe];
       p[8] = n_row[8 * plane + xw];
       const float s = cell_update<float, STRICT>(p, obst, a.omega, o);
-      q += to_fixed(s);
-      if (!(s < (float)LBM_SPEED_LIMIT)) atomicOr(av_step + 1, LBM_NONFINITE_MARK);
       if (y == accel_y && !last_step)
         cell_accelerate<float, true>(o[1], o[3], o[5], o[6], o[7], o[8], obst, a.aw1, a.aw2);
 #pragma unroll
       for (int k = 0; k < 9; k++) wr[k * plane + c] = o[k];
+      return s;
+    };
+    unsigned long long q = 0ULL;
+    bool bad = false;
+    if (STRICT) {
+      for (int c = tid; c < my_cells; c += LBM_CLUSTER_THREADS) {
+        const int yl = c / nx;
+        const float s = update(yl, c - yl * nx);
+        q += to_fixed(s);
+        bad |= !(s < (float)LBM_SPEED_LIMIT);
+      }
+    } else {
+      // the default build adds |u| over the x-aligned quads of the other kernels, in their
+      // float order (quad_sum_fixed), so that every kernel gives the same av_vels bits
+      const int quads_x = (nx + 3) / 4;
+      for (int i = tid; i < my_rows * quads_x; i += LBM_CLUSTER_THREADS) {
+        const int yl = i / quads_x, x0 = 4 * (i - yl * quads_x);
+        float s[4];
+#pragma unroll
+        for (int j = 0; j < 4; j++) s[j] = (x0 + j < nx) ? update(yl, x0 + j) : 0.0f;
+        bool b;
+        q += quad_sum_fixed<float>(s[0], s[1], s[2], s[3], b);
+        bad |= b;
+      }
     }
+    if (bad) atomicOr(av_step + 1, LBM_NONFINITE_MARK);
     block_accumulate(q, av_step);
     cluster.sync();
     cur ^= 1;

@@ -223,7 +223,9 @@ __device__ __forceinline__ double speed_of(double usq) { return ::sqrt(usq); }
 // A cell whose |u| is NaN or beyond any physical value (the lattice has blown up; the speed
 // of sound is 0.577) cannot be represented in the fixed-point sum: the step's high word gets
 // this bit and the host reports that step's average as NaN, which is what the reference's
-// float sum would give a few steps later at the latest.  The bound also keeps every
+// float sum would give a few steps later at the latest.  Every kernel, in both builds, tests
+// each fluid cell's |u| against it on its own (quad_sum_fixed, scalar_tile, K6), and so does
+// the av_velocity read-out, so one lattice gives one NaN pattern.  The bound also keeps every
 // per-thread partial sum (up to 4 cells x 256 rows) below 2^64; partial sums are split
 // into 32-bit halves before they are added across threads.
 #define LBM_SPEED_LIMIT 2.0
@@ -327,12 +329,16 @@ template <> struct QuadConsts<double, false> {
   __device__ __forceinline__ explicit QuadConsts(double om) : k(om) {}
 };
 
+// Every cell is held to LBM_SPEED_LIMIT on its own, as in the strict build and in av_velocity:
+// a bound on the quad's sum would let one cell of up to four times the limit through.  The
+// compares are written so that a NaN speed fails them (fmaxf would drop it).  With each speed
+// below 2 the quad's sum stays below 8, which is the headroom the fixed-point sum relies on.
 template <typename real>
 __device__ __forceinline__ unsigned long long quad_sum_fixed(real s0, real s1, real s2, real s3, bool& bad) {
   typedef Ops<real, true> M;
-  const real s = M::add(M::add(s0, s1), M::add(s2, s3));
-  bad = !(s < (real)(4.0 * LBM_SPEED_LIMIT));     // the bound of four cells
-  return to_fixed(s);
+  const real L = (real)LBM_SPEED_LIMIT;
+  bad = !(s0 < L && s1 < L && s2 < L && s3 < L);
+  return to_fixed(M::add(M::add(s0, s1), M::add(s2, s3)));
 }
 
 template <typename real, bool STRICT>
@@ -1030,18 +1036,17 @@ __device__ __forceinline__ unsigned long long scalar_tile(const StepArgs<real>& 
   // |u| sum: the strict build converts every cell exactly; the default build adds the four
   // cells of an aligned quad as floats in the order of the vectorised kernels (quad_update),
   // so that every kernel variant returns the same av_vels bits.
+  // Both builds hold every cell to LBM_SPEED_LIMIT on its own (see quad_sum_fixed).
   unsigned long long q;
-  bool bad;
+  const bool bad = !(s < (real)LBM_SPEED_LIMIT);
   if (STRICT) {
     q = to_fixed(s);
-    bad = !(s < (real)LBM_SPEED_LIMIT);
   } else {
     typedef Ops<real, true> M;
     real t = M::add(s, __shfl_xor_sync(0xffffffffu, s, 1));
     t = M::add(t, __shfl_xor_sync(0xffffffffu, t, 2));
     const bool lead = (threadIdx.x & 3) == 0;
     q = lead ? to_fixed(t) : 0ULL;
-    bad = lead && !(t < (real)(4.0 * LBM_SPEED_LIMIT));
   }
   if (active && bad) atomicOr(a.av + 1, LBM_NONFINITE_MARK);
   return q;
