@@ -110,7 +110,7 @@ enum SyncWord { kFlagFromBelow = 0, kFlagFromAbove = 1, kBoundaryDone = 2, kScra
                 kAvScratch = 16 /* kAvWords words */, kSyncWords = 16 + 128 };
 constexpr int kTb2MinRows = 8;                             // per slab, for the two-step kernel
 constexpr int kTb3MinRows = 12;                            // for the three-step kernel (one slab)
-constexpr double kTb3MinWaves = 4.0;                       // K10 by default from this many waves of its blocks on
+constexpr double kTb3MinWaves = 2.0;                       // K10 by default from this many waves of its blocks on
 constexpr int kAvWords = LBM_AV_STRIDE * LBM_AV_SLOTS;     // words of one step's |u| sums (1 KiB)
 constexpr int kMaxSegmentSteps = 1 << 16;                  // 64 MiB of sums per run segment
 
@@ -543,9 +543,10 @@ class Grid : public GridBase {
     return slabs.size() == 1 && slabs[0].rows == prm.ny && slabs[0].row0 == 0 && !f16 && k7_fits(slabs[0].rows) &&
            slabs[0].rows >= kTb3MinRows && !env_on("LBM_GPU_NO_TB3");
   }
-  // Default: K10 where it was measured faster than K7 (profiles/r03_size_sweep.log), i.e. where
-  // its blocks fill enough waves of the SMs; with few waves the launch tail of K10's longer
-  // blocks costs more than the bytes it saves.
+  // Default: K10 where its blocks fill at least two waves of the SMs.  At four blocks per SM it
+  // measured faster than K7 on every size swept (1.15 x at 16384 x 2048, 2.4 waves;
+  // profiles/r07_k10_four_blocks.md); below two waves (4096^2: 1.2) K7 stays, where the launch
+  // tail of K10's longer blocks weighs most.
   bool tb3_pays() const {
     const double resident = (double)LBM_TB3_MIN_BLOCKS * sm_count();
     return tb_waves(slabs[0].rows, 64, resident) >= kTb3MinWaves;
@@ -557,7 +558,9 @@ class Grid : public GridBase {
       for (const void* fn : {(const void*)lbm::lbm_step3_tb<false>, (const void*)lbm::lbm_step3_tb<true>})
         CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(lbm::Tb3Smem)));
       const double resident = (double)LBM_TB3_MIN_BLOCKS * sm_count();
-      tb3_seg_rows = best_segment_rows(s.rows, resident, 4, 96);   // 96 rows measured best at 16384^2 (profiles/r03_k10.md)
+      // at 16384^2 80-112 rows are within 0.7 % of each other, 64 and 128 1.5 % slower; the score
+      // picks 88 (profiles/r07_k10_four_blocks.md)
+      tb3_seg_rows = best_segment_rows(s.rows, resident, 4, 96);
       if (const char* e = getenv("LBM_TB3_SEG_ROWS")) tb3_seg_rows = std::max(1, atoi(e));   // tuning knob
     }
   }
@@ -2312,5 +2315,18 @@ void lbm_gpu_destroy(lbm_gpu* h) {
   if (!h) return;
   delete reinterpret_cast<GridBase*>(h);
 }
+
+#ifdef LBM_EXPERIMENTS
+// -DLBM_EXPERIMENTS builds only: K10's staging-wait and tile cycles on the current device since
+// the last call (lbm::tb3_exp_cycles), then cleared
+int lbm_gpu_exp_tb3_cycles(unsigned long long out[2]) {
+  static const unsigned long long zero[2] = {0ULL, 0ULL};
+  if (cudaDeviceSynchronize() != cudaSuccess ||
+      cudaMemcpyFromSymbol(out, lbm::tb3_exp_cycles, sizeof zero) != cudaSuccess ||
+      cudaMemcpyToSymbol(lbm::tb3_exp_cycles, zero, sizeof zero) != cudaSuccess)
+    return fail("lbm_gpu_exp_tb3_cycles: %s", cudaGetErrorString(cudaGetLastError()));
+  return 0;
+}
+#endif
 
 }  // extern "C"

@@ -10,19 +10,25 @@
 // no three-deep ghost zones; it still pushes K7's two-deep ghost rows, so that a K7 pass (two
 // steps left) or a K1a step (one left) can follow it.  Several slabs run K7.
 //
-// Decomposition: K7's strips, segments and bulk-copy staging (two rows ahead, mbarrier
-// completion).  Iteration i of a segment [R0, R1), source row r = R0 - 2 + i:
+// Decomposition: K7's strips and segments, bulk-copy staging with mbarrier completion.
+// Iteration i of a segment [R0, R1), source row r = R0 - 2 + i:
 //   1. sub-step 1 on row r from the staged input -> ring level 1;
 //   2. sub-step 2 on row r-1 from ring level 1  -> ring level 2      (i >= 2);
 //   3. sub-step 3 on row r-2 from ring level 2  -> HBM, 128-bit stores (i >= 4).
 // Sub-step 1 covers rows R0-2 .. R1+1, sub-step 2 R0-1 .. R1, sub-step 3 R0 .. R1-1; sub-step k
 // is valid on span columns [k, span-k), which contain the owned columns [4, span-4).
 //
+// Staging is one stage deep: the copies of row r+1 are issued right after the first block
+// barrier of iteration i (everyone has read row r by then) and land while sub-steps 2 and 3
+// run.  A second stage would hide more copy latency but costs 9 plane-rows, and without them
+// a fourth block fits on the SM: 12 warps instead of 9 hide the shared-memory and barrier
+// latency this kernel is bound by (profiles/r07_k10_four_blocks.md).
+//
 // The ring is lean: planes 0, 2 and 4 are pulled from the thread's own columns, so they stay
 // in registers (plane 4 of row r is used in the same iteration, plane 0 of row r-1 is carried
 // one iteration, plane 2 of rows r-2 and r-1 two).  Only the six x-shifted planes go through
-// shared memory: 12 plane-rows per level instead of 17, and 18 + 2 x 12 plane-rows of 1568 B
-// (65.9 KB) let three blocks (9 warps) share an SM.
+// shared memory: 12 plane-rows per level instead of 17.  With plane 0 of level 2 (2 rows)
+// that is 9 + 2 x 12 + 2 = 35 plane-rows of 1568 B (53.6 KB): four blocks (12 warps) share an SM.
 //
 // Ordering: two block barriers per iteration, one after each ring level is written.  Each
 // also orders the reads of the previous iteration before the writes of this one (WAR), so no
@@ -36,7 +42,13 @@
 namespace lbm {
 
 #ifndef LBM_TB3_MIN_BLOCKS
-#define LBM_TB3_MIN_BLOCKS (LBM_TB2_THREADS <= 64 ? 4 : LBM_TB2_THREADS <= 96 ? 3 : 2)
+#define LBM_TB3_MIN_BLOCKS (LBM_TB2_THREADS <= 96 ? 4 : 2)
+#endif
+
+#ifdef LBM_EXPERIMENTS
+// clock64() cycles K10 spends waiting for staged rows [0] and in its tiles [1], summed over the
+// warps (lane 0 of each); read and cleared by lbm_gpu_exp_tb3_cycles (tools/build_variants.py)
+__device__ unsigned long long tb3_exp_cycles[2];
 #endif
 
 struct Tb3Level {                       // one level of the ring: the x-shifted planes of sub-step-k rows
@@ -45,14 +57,15 @@ struct Tb3Level {                       // one level of the ring: the x-shifted 
   float r78[2][LBM_TB2_ROWF];           // planes 7,8 of this iteration's row
 };
 struct Tb3Smem {
-  float in[2][9][LBM_TB2_ROWF];         // two stages of pulled plane-rows (bulk copy destination)
+  float in[1][9][LBM_TB2_ROWF];         // one stage of pulled plane-rows (bulk copy destination; the stage
+                                        // index keeps K7's tb2_expect / tb2_issue usable)
   Tb3Level lv[2];                       // sub-step-1 rows, sub-step-2 rows
   float p0[2][LBM_TB2_ROWF];            // plane 0 of the sub-step-2 rows of this and the previous iteration
-                                        // (in shared memory, not registers: 9 warps per SM leave 168 each)
-  unsigned long long mbar[2];           // "stage filled"
+                                        // (in shared memory, not registers: 12 warps per SM leave 168 each)
+  unsigned long long mbar[1];           // "stage filled"
 };
-constexpr int kTb3PlaneRows = 18 + 2 * 12 + 2;
-static_assert(sizeof(Tb3Smem) == kTb3PlaneRows * LBM_TB2_ROWF * sizeof(float) + 16, "ring layout");
+constexpr int kTb3PlaneRows = 9 + 2 * 12 + 2;
+static_assert(sizeof(Tb3Smem) == kTb3PlaneRows * LBM_TB2_ROWF * sizeof(float) + 8, "ring layout");
 // per block: the dynamic layout, block_accumulate's 512 B of static scratch, 1 KB reserved by the SM
 static_assert((sizeof(Tb3Smem) + 512 + 1024) * LBM_TB3_MIN_BLOCKS <= 228 * 1024,
               "LBM_TB3_MIN_BLOCKS blocks of shared memory per SM");
@@ -66,7 +79,6 @@ __device__ __forceinline__ void tb3_init_smem(Tb3Smem& sm, const int span) {
   }
   if (tid == 0) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&sm.mbar[0])) : "memory");
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&sm.mbar[1])) : "memory");
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
 }
@@ -133,9 +145,8 @@ __device__ __forceinline__ void tb3_tile(const Tb2Args& ta, Tb3Smem& sm, const i
                      (X0 + c0 - LBM_TB2_PAD < a.nx);
 
   const int my_plane = tb2_plane_of_thread();
-  if (tid == 0) { tb2_expect(sm, 0, ta.span); tb2_expect(sm, 1, ta.span); }
-#pragma unroll 1
-  for (int k = 0; k < 2; k++) tb2_issue<true>(a, sm, k, R0 - 2 + k, S0, ta.span, my_plane);
+  if (tid == 0) tb2_expect(sm, 0, ta.span);
+  tb2_issue<true>(a, sm, 0, R0 - 2, S0, ta.span, my_plane);
 
   const QuadConsts<float, STRICT> qc(a.omega);
   const int mword_idx = xg >> 5, mshift = xg & 31;
@@ -145,21 +156,30 @@ __device__ __forceinline__ void tb3_tile(const Tb2Args& ta, Tb3Smem& sm, const i
   };
   uint32_t m1 = mask_bits(R0 - 2), m2 = 0u, m3 = 0u;   // masks of the rows of sub-steps 1, 2, 3
   Tb3Carry c1, c2;                                      // levels 1 and 2 (level 2 keeps plane 0 in sm.p0)
-  uint32_t phases = 0u;
+  uint32_t phase = 0u;                                  // parity the staging barrier completes next
+#ifdef LBM_EXPERIMENTS
+  const long long t_tile = clock64();
+  long long t_wait = 0;
+#endif
 
 #pragma unroll 1
   for (int i = 0; i < n_it; i++) {
-    const int st = i & 1;
     const int r = R0 - 2 + i;
     const uint32_t m_next = (i + 1 < n_it) ? mask_bits(r + 1) : 0u;
     float in[4][9], out[4][9];
     bool b;
-    // ---------------- sub-step 1 on row r: pulled values are staged in sm.in[st] ----------------
-    tb2_mbar_wait(&sm.mbar[st], (phases >> st) & 1u);
-    phases ^= 1u << st;
-    if (tid == 0 && i + 2 < n_it) tb2_expect(sm, st, ta.span);      // the refill of this stage, issued after the barrier below
+    // ---------------- sub-step 1 on row r: pulled values are staged in sm.in[0] -----------------
+#ifdef LBM_EXPERIMENTS
+    const long long t0 = clock64();
+    tb2_mbar_wait(&sm.mbar[0], phase);
+    t_wait += clock64() - t0;
+#else
+    tb2_mbar_wait(&sm.mbar[0], phase);
+#endif
+    phase ^= 1u;
+    if (tid == 0 && i + 1 < n_it) tb2_expect(sm, 0, ta.span);       // the refill with row r+1, issued after the barrier below
     {
-      const float(*row)[LBM_TB2_ROWF] = sm.in[st];
+      const float(*row)[LBM_TB2_ROWF] = sm.in[0];
       tb2_get(row[0], c0, in[0][0], in[1][0], in[2][0], in[3][0]);
       tb2_get(row[2], c0, in[0][2], in[1][2], in[2][2], in[3][2]);
       tb2_get(row[4], c0, in[0][4], in[1][4], in[2][4], in[3][4]);
@@ -177,8 +197,8 @@ __device__ __forceinline__ void tb3_tile(const Tb2Args& ta, Tb3Smem& sm, const i
     float p4[4];
 #pragma unroll
     for (int j = 0; j < 4; j++) p4[j] = out[j][4];
-    __syncthreads();          // level-1 row r is complete; stage `st` has been read by everyone
-    if (i + 2 < n_it) tb2_issue<true>(a, sm, st, r + 2, S0, ta.span, my_plane);
+    __syncthreads();          // level-1 row r is complete; the stage has been read by everyone
+    if (i + 1 < n_it) tb2_issue<true>(a, sm, 0, r + 1, S0, ta.span, my_plane);
 
     if (i >= 2) {
       // ---------------- sub-step 2 on row y = r - 1 from level-1 rows y-1, y, y+1 --------------
@@ -216,6 +236,12 @@ __device__ __forceinline__ void tb3_tile(const Tb2Args& ta, Tb3Smem& sm, const i
     m2 = m1;
     m1 = m_next;
   }
+#ifdef LBM_EXPERIMENTS
+  if ((tid & 31) == 0) {
+    atomicAdd(&tb3_exp_cycles[0], (unsigned long long)t_wait);
+    atomicAdd(&tb3_exp_cycles[1], (unsigned long long)(clock64() - t_tile));
+  }
+#endif
 }
 
 // ------------------------------------------------------------------------------------

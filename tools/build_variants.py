@@ -22,6 +22,7 @@ VARIANTS = {
     "tb2_t64": ["-DLBM_TB2_THREADS=64", "-DLBM_TB2_MIN_BLOCKS=6"],
     "tb3_t64": ["-DLBM_TB2_THREADS=64", "-DLBM_TB3_MIN_BLOCKS=4"],     # K10, 64-thread strips (profiles/r03_k10.md)
     "tb3_mb2": ["-DLBM_TB3_MIN_BLOCKS=2"],                              # K10, 186 registers, 6 warps per SM
+    "tb3_wait": ["-DLBM_EXPERIMENTS"],    # K10's staging-wait share of its cycles (run with --kernel tb3), r07
 }
 if os.environ.get("LBM_VARIANTS"):
     VARIANTS = {k: v for k, v in VARIANTS.items() if k in os.environ["LBM_VARIANTS"].split(",")}

@@ -1,6 +1,7 @@
 #!/usr/bin/env python3
 """Quick device-time probe of the step kernel (development tool, not the bench contract)."""
 import argparse
+import ctypes
 import os
 import sys
 import time
@@ -32,11 +33,19 @@ t1 = time.time()
 lat = L.Lattice(a.nx, a.ny, 0.1, 0.005, 1.85, obstacles=bits, bits=True, flags=flags, n_gpus=a.gpus, f64=a.f64)
 t2 = time.time()
 print("mask %.2fs create %.2fs free_cells %d" % (t1 - t0, t2 - t1, lat.info().free_cells), flush=True)
+# K10's staging-wait counters, in -DLBM_EXPERIMENTS builds (tools/build_variants.py tb3_wait) only
+exp_cycles = getattr(L.load_library(), "lbm_gpu_exp_tb3_cycles", None)
+cyc = (ctypes.c_ulonglong * 2)()
 lat.run_timed(3)
+if exp_cycles:
+    exp_cycles(cyc)
 for r in range(a.reps):
     ms = lat.run_timed(a.steps)
     mlups = a.nx * a.ny * a.steps / ms / 1e3
-    print("kernel=%s %dx%d gpus=%d steps=%d: %.3f ms/step  %.0f MLUPS  %.0f GB/s (x72B; x144B if f64)" %
-          (a.kernel, a.nx, a.ny, a.gpus, a.steps, ms / a.steps, mlups, mlups * 72e-3), flush=True)
+    wait = ""
+    if exp_cycles and exp_cycles(cyc) == 0 and cyc[1]:
+        wait = "  K10 staging wait %.2f %% of its cycles" % (100.0 * cyc[0] / cyc[1])
+    print("kernel=%s %dx%d gpus=%d steps=%d: %.3f ms/step  %.0f MLUPS  %.0f GB/s (x72B; x144B if f64)%s" %
+          (a.kernel, a.nx, a.ny, a.gpus, a.steps, ms / a.steps, mlups, mlups * 72e-3, wait), flush=True)
 av = lat.run(5)
 print("av_vels", av)
