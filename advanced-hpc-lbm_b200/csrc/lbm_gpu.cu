@@ -111,6 +111,7 @@ enum SyncWord { kFlagFromBelow = 0, kFlagFromAbove = 1, kBoundaryDone = 2, kScra
 constexpr int kTb2MinRows = 8;                             // per slab, for the two-step kernel
 constexpr int kTb3MinRows = 12;                            // for the three-step kernel (one slab)
 constexpr double kTb3MinWaves = 2.0;                       // K10 by default from this many waves of its blocks on
+constexpr int kTb3OverlapSegRows = 192;                    // K10 segment height when passes overlap
 constexpr int kAvWords = LBM_AV_STRIDE * LBM_AV_SLOTS;     // words of one step's |u| sums (1 KiB)
 constexpr int kMaxSegmentSteps = 1 << 16;                  // 64 MiB of sums per run segment
 
@@ -190,6 +191,8 @@ class Grid : public GridBase {
   int tb2_strips = 0, tb2_wout = 0, tb2_seg_rows = 0, tb2_span = 0, tb2_threads = 0;
   int tb2_tail_rows = 16, tb2_tail_segs = 0;   // K7: height and number of the short segments that end a launch
   int tb3_seg_rows = 0;        // K10: rows per segment
+  bool tb3_overlap = false;    // K10: consecutive passes overlap, ordered per tile (lbm_tb3.cuh)
+  uint32_t* tb3_done = nullptr;   // K10: per tile, the passes it has completed (tb3_overlap only)
   int pairs_tile_rows = 0;     // K9: rows per block
   bool f16 = false;            // LBM_GPU_STORE_F16: the lattice buffers hold shifted binary16 (lbm_f16.cuh)
   bool failed = false;         // a neighbour never arrived: the lattice contents are void
@@ -222,6 +225,7 @@ class Grid : public GridBase {
         if (s.step_ev[i]) cudaEventDestroy(s.step_ev[i]);
       if (s.stream) cudaStreamDestroy(s.stream);
     }
+    if (tb3_done) { cudaSetDevice(slabs[0].device); cudaFree(tb3_done); }
   }
 
   // LBM_GPU_POOL: the lattice and the staging buffer come from the device's stream-ordered
@@ -558,11 +562,42 @@ class Grid : public GridBase {
       for (const void* fn : {(const void*)lbm::lbm_step3_tb<false>, (const void*)lbm::lbm_step3_tb<true>})
         CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(lbm::Tb3Smem)));
       const double resident = (double)LBM_TB3_MIN_BLOCKS * sm_count();
-      // at 16384^2 80-112 rows are within 0.7 % of each other, 64 and 128 1.5 % slower; the score
-      // picks 88 (profiles/r07_k10_four_blocks.md)
-      tb3_seg_rows = best_segment_rows(s.rows, resident, 4, 96);
+      // Passes that do not overlap end in a tail: the wave score picks 88 rows at 16384^2, where
+      // 80-112 rows are within 0.7 % of each other (profiles/r07_k10_four_blocks.md).  Overlapped
+      // passes have no tail between them, so taller segments pay less halo: 192 rows measured
+      // 2.3 % faster than 88 at 16384^2 (profiles/r08_k10_overlap.md); the wave score stays for
+      // launches of fewer than two waves at that height.
+      const bool overlap = use_pdl() && !env_on("LBM_GPU_NO_TB3_OVERLAP");
+      tb3_seg_rows = (overlap && tb_waves(s.rows, kTb3OverlapSegRows, resident) >= 2.0)
+                         ? kTb3OverlapSegRows : best_segment_rows(s.rows, resident, 4, 96);
       if (const char* e = getenv("LBM_TB3_SEG_ROWS")) tb3_seg_rows = std::max(1, atoi(e));   // tuning knob
+      tb3_overlap = overlap && tb3_overlap_fits(s.rows);
+      if (tb3_overlap && !tb3_done) {
+        const size_t bytes = (size_t)tb2_strips * tb3_segments(s.rows).n_big * sizeof(uint32_t);
+        CK(cudaMalloc((void**)&tb3_done, bytes));
+        // No reset is needed later (upload, a K7 or K1a pass in between): the first K10 pass after
+        // anything else waits for the whole previous grid and then publishes every tile.
+        CK(cudaMemset(tb3_done, 0, bytes));
+      }
     }
+  }
+  // Overlapped K10 passes order a tile after the 3 x 3 neighbourhood of its tile in the previous
+  // pass.  That neighbourhood holds every tile whose cells it reads (rows R0-3 .. R1+2, the
+  // staged columns) and, the relation being symmetric, every tile that reads the cells it
+  // writes, if no tile reads beyond the strips and segments next to it: false for segments of
+  // fewer than three rows, or a last strip narrower than the halo.
+  bool tb3_overlap_fits(int rows) const {
+    const Tb2Segments g = tb3_segments(rows);
+    auto near = [](int a, int b, int n) { const int d = (a - b + n) % n; return d <= 1 || d == n - 1; };
+    for (int seg = 0; seg < g.n_big; seg++) {
+      const int r0 = seg * g.seg_rows, r1 = std::min(r0 + g.seg_rows, rows);
+      for (int r = r0 - 3; r < r1 + 3; r++)
+        if (!near(((r % rows) + rows) % rows / g.seg_rows, seg, g.n_big)) return false;
+    }
+    for (int strip = 0; strip < tb2_strips; strip++)
+      for (int c = strip * tb2_wout - LBM_TB2_PAD; c < strip * tb2_wout - LBM_TB2_PAD + tb2_span; c++)
+        if (!near(((c % prm.nx) + prm.nx) % prm.nx / tb2_wout, strip, tb2_strips)) return false;
+    return true;
   }
 
   // segments of a slab for K7: n_big segments of equal height, then (tall slabs) n_tail short
@@ -1097,6 +1132,9 @@ class Grid : public GridBase {
           ta.n_big = sg.n_big;
           ta.big_rows = sg.big_rows;
           ta.seg_rows_tail = sg.seg_rows_tail;
+          ta.tile_done = tb3_overlap ? tb3_done : nullptr;
+          // a K10 pass is preceded in its run segment by K10 passes only (a shorter last pass comes last)
+          ta.wait_tiles = tb3_overlap && pass_in_segment > 0;
           const dim3 grid((unsigned)((long long)tb2_strips * sg.n_big));
           if (strict) launch_tb3<true>(s, ta, grid);
           else        launch_tb3<false>(s, ta, grid);
@@ -1253,8 +1291,8 @@ class Grid : public GridBase {
     last_run_ms = ms_max;
     last_step_ms = ms_max / n_steps;
     steps_done += n_steps;
-    if (use_flags) check_sync_errors();
-    if (kernel == LBM_GPU_KERNEL_CLUSTER) prepare();      // side row + ghost rows of the new state
+    if (use_flags || (kernel == LBM_GPU_KERNEL_TB3 && tb3_overlap)) check_sync_errors();
+    if (kernel == LBM_GPU_KERNEL_CLUSTER) prepare();     // side row + ghost rows of the new state
     if (sums_out) read_sums(n_steps, sums_out);
   }
 
@@ -1293,7 +1331,10 @@ class Grid : public GridBase {
       failed = true;
       const unsigned long long why = w[1] >> 56, pass = w[1] & 0xffffffffffffffULL;
       char msg[256];
-      if (why == LBM_SYNC_TIMEOUT)
+      if (why == LBM_SYNC_TILE_TIMEOUT)
+        snprintf(msg, sizeof msg, "three-step kernel: a tile of pass %llu did not complete within %.1f s; run abandoned",
+                 pass - 1, (double)timeout_ns * 1e-9);
+      else if (why == LBM_SYNC_TIMEOUT)
         snprintf(msg, sizeof msg, "rows [%lld,%lld): a neighbouring slab did not complete pass %llu within %.1f s "
                  "(its process died, or it was asked for a different number of steps); run abandoned",
                  s.row0, s.row0 + s.rows, pass, (double)timeout_ns * 1e-9);
@@ -2325,6 +2366,19 @@ int lbm_gpu_exp_tb3_cycles(unsigned long long out[2]) {
       cudaMemcpyFromSymbol(out, lbm::tb3_exp_cycles, sizeof zero) != cudaSuccess ||
       cudaMemcpyToSymbol(lbm::tb3_exp_cycles, zero, sizeof zero) != cudaSuccess)
     return fail("lbm_gpu_exp_tb3_cycles: %s", cudaGetErrorString(cudaGetLastError()));
+  return 0;
+}
+// ... and K10's block times since the last call (lbm::tb3_exp_blocks: earliest start, latest
+// end, sum of block durations, in ns), then cleared; out[3] = resident K10 blocks of the device
+int lbm_gpu_exp_tb3_blocks(unsigned long long out[4]) {
+  static const unsigned long long clear[3] = {~0ULL, 0ULL, 0ULL};
+  int dev = 0, sms = 0;
+  if (cudaDeviceSynchronize() != cudaSuccess || cudaGetDevice(&dev) != cudaSuccess ||
+      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
+      cudaMemcpyFromSymbol(out, lbm::tb3_exp_blocks, sizeof clear) != cudaSuccess ||
+      cudaMemcpyToSymbol(lbm::tb3_exp_blocks, clear, sizeof clear) != cudaSuccess)
+    return fail("lbm_gpu_exp_tb3_blocks: %s", cudaGetErrorString(cudaGetLastError()));
+  out[3] = (unsigned long long)LBM_TB3_MIN_BLOCKS * sms;
   return 0;
 }
 #endif

@@ -623,6 +623,7 @@ __device__ __forceinline__ unsigned long long global_timer_ns() {
 // error codes left in the sync block for the host (kSyncError)
 #define LBM_SYNC_TIMEOUT 1ULL
 #define LBM_SYNC_ABORTED 2ULL
+#define LBM_SYNC_TILE_TIMEOUT 3ULL    /* K10: a neighbour tile of the previous pass never completed */
 
 // Wait until both neighbours have completed `pass` passes.  The wait is bounded: when a
 // neighbour does not arrive within timeout_ns (its process died, or it was asked for a

@@ -70,6 +70,9 @@ struct Tb2Args {
   int big_rows;                    // the segments behind them are seg_rows_tail rows tall: they get the highest
   int seg_rows_tail;               // block indices, so a launch ends with short blocks and the SMs drain together
   unsigned long long* av3;         // K10 only: sums of sub-step 3
+  uint32_t* tile_done;             // K10 only: per tile, the passes it has completed; null = passes do not overlap
+  int wait_tiles;                  // K10 only: the launch before this one was a K10 pass of the same lattice and
+                                   // segmentation, so a block waits for its nine neighbour tiles, not the whole grid
 };
 
 __device__ __forceinline__ void tb2_mbar_wait(unsigned long long* bar, const uint32_t parity) {

@@ -49,6 +49,10 @@ namespace lbm {
 // clock64() cycles K10 spends waiting for staged rows [0] and in its tiles [1], summed over the
 // warps (lane 0 of each); read and cleared by lbm_gpu_exp_tb3_cycles (tools/build_variants.py)
 __device__ unsigned long long tb3_exp_cycles[2];
+// %globaltimer of K10's blocks: earliest start [0], latest end [1], sum of block durations [2]
+// (start = the previous pass's data is available, end = the tile is published); read and
+// cleared by lbm_gpu_exp_tb3_blocks
+__device__ unsigned long long tb3_exp_blocks[3] = {~0ULL, 0ULL, 0ULL};
 #endif
 
 struct Tb3Level {                       // one level of the ring: the x-shifted planes of sub-step-k rows
@@ -244,20 +248,93 @@ __device__ __forceinline__ void tb3_tile(const Tb2Args& ta, Tb3Smem& sm, const i
 #endif
 }
 
+// Blocks take the segments middle-out (m, m-1, m+1, m-2, ...; m = tiles_y / 2), so the last
+// blocks of a pass are segments 0 and tiles_y-1 and their neighbours: the first blocks of the next
+// pass, around m, do not wait for the last ones of this pass.  The order changes no result.
+__device__ __forceinline__ int tb3_seg_of_slot(const int slot, const int tiles_y) {
+  return (slot & 1) ? tiles_y / 2 - (slot + 1) / 2 : tiles_y / 2 + slot / 2;
+}
+__device__ __forceinline__ int tb3_slot_of_seg(const int seg, const int tiles_y) {
+  return (seg >= tiles_y / 2) ? 2 * (seg - tiles_y / 2) : 2 * (tiles_y / 2 - seg) - 1;
+}
+
+__device__ __forceinline__ uint32_t ld_acquire_gpu_u32(const uint32_t* p) {
+  uint32_t v;
+  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+
+// Overlapped passes: thread 0 waits until the 3 x 3 neighbourhood of tile (strip, seg), periodic
+// in x and y, has completed the previous pass: its words count passes completed, so they must
+// reach a.pass (signed difference, so wrap-around is harmless; a word starts at 0, which no pass
+// after the first can mistake for its predecessor).  The host allows the overlap only where that
+// neighbourhood holds every tile that reads a cell this tile writes, and every tile that writes a
+// cell this tile reads (Grid::tb3_overlap_fits).  The wait is bounded like boundary_wait: on a time-out, or when
+// another block gave up, the block records why, raises the abort word and carries on; the run's
+// results are void and lbm_gpu_run reports it.
+__device__ __forceinline__ void tb3_wait_tiles(const Tb2Args& ta, const int strip, const int seg) {
+  const StepArgs<float>& a = ta.s;
+  const uint32_t done = (uint32_t)a.pass;
+  const unsigned long long t0 = global_timer_ns();
+  unsigned ns = 32;
+#pragma unroll 1
+  for (int dy = -1; dy <= 1; dy++) {
+    if ((dy == -1 && a.tiles_y < 2) || (dy == 1 && a.tiles_y < 3)) continue;    // fewer than three segments
+    const int y = (seg + dy + a.tiles_y) % a.tiles_y;
+#pragma unroll 1
+    for (int dx = -1; dx <= 1; dx++) {
+      if ((dx == -1 && a.tiles_x < 2) || (dx == 1 && a.tiles_x < 3)) continue;  // ... or strips
+      const uint32_t* f = ta.tile_done + (size_t)tb3_slot_of_seg(y, a.tiles_y) * a.tiles_x + (strip + dx + a.tiles_x) % a.tiles_x;
+      while ((int)(ld_acquire_gpu_u32(f) - done) < 0) {
+        if (ld_acquire_sys(a.abort_word) != 0ULL) return;
+        if (global_timer_ns() - t0 > a.timeout_ns) {
+          atomicCAS(a.abort_word + 1, 0ULL, (LBM_SYNC_TILE_TIMEOUT << 56) | (a.pass & 0xffffffffffffffULL));
+          st_release_sys(a.abort_word, 1ULL);
+          return;
+        }
+        __nanosleep(ns);
+        ns = min(2u * ns, 1024u);
+      }
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------
 // K10  lbm_step3_tb: one launch = three timesteps of a slab that holds the whole grid
 // ------------------------------------------------------------------------------------
+// Consecutive K10 passes overlap (ta.tile_done set): every block triggers the next launch as soon
+// as it is resident, and publishes the number of passes its tile has completed after its last
+// global write.  A block
+// of a pass that follows a K10 pass (ta.wait_tiles) waits for its nine neighbour tiles of that
+// pass instead of the whole grid.  Deadlock freedom: the next grid launches only once every block
+// of this one has triggered, i.e. is resident or finished, so every tile a waiting block depends
+// on already holds an SM or is done; the oldest pass in flight waits for nothing that is not.
+// A kernel after K10 that calls cudaGridDependencySynchronize (K7, K1a) still waits for the
+// whole grid to complete and flush, as does anything launched without programmatic
+// serialization.
+// The words of ta.tile_done are indexed by block, not by tile: the epilogue then needs nothing
+// the row loop has to keep in registers.
 template <bool STRICT>
 __global__ void __launch_bounds__(LBM_TB2_THREADS, LBM_TB3_MIN_BLOCKS)
 lbm_step3_tb(const __grid_constant__ Tb2Args ta) {
   extern __shared__ __align__(128) unsigned char tb3_smem_raw[];
   Tb3Smem& sm = *reinterpret_cast<Tb3Smem*>(tb3_smem_raw);
   const StepArgs<float>& a = ta.s;
-  int strip, seg;
-  tile_of_block(a.tiles_x, a.tiles_y, 1, strip, seg);
+  const int slot = (int)(blockIdx.x / (unsigned)a.tiles_x);
+  const int strip = (int)blockIdx.x - slot * a.tiles_x;
+  const int seg = tb3_seg_of_slot(slot, a.tiles_y);
   tb3_init_smem(sm, ta.span);
-  cudaGridDependencySynchronize();           // PDL: the previous pass's writes are visible from here on
+  if (ta.tile_done) cudaTriggerProgrammaticLaunchCompletion();
+  if (ta.wait_tiles) {
+    if (threadIdx.x == 0) tb3_wait_tiles(ta, strip, seg);
+  } else {
+    cudaGridDependencySynchronize();         // PDL: the previous pass's writes are visible from here on
+  }
   __syncthreads();
+  if (ta.wait_tiles) asm volatile("fence.proxy.async.global;" ::: "memory");   // the staging copies are async-proxy reads
+#ifdef LBM_EXPERIMENTS
+  const unsigned long long t_start = global_timer_ns();
+#endif
   unsigned long long q[3] = {0ULL, 0ULL, 0ULL};
   bool bad[3] = {false, false, false};
   tb3_tile<STRICT>(ta, sm, strip, seg, q, bad);
@@ -269,6 +346,25 @@ lbm_step3_tb(const __grid_constant__ Tb2Args ta) {
   block_accumulate(q[1], ta.av2);
   __syncthreads();
   block_accumulate(q[2], ta.av3);
+  if (ta.tile_done) {
+    // every store of the tile, its ghost-row pushes and its sums are made visible before the
+    // tile is published (stores of this pass may be read by bulk copies of the next)
+    asm volatile("fence.proxy.async.global;" ::: "memory");
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      __threadfence();
+      asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(ta.tile_done + blockIdx.x),
+                   "r"((uint32_t)a.pass + 1u) : "memory");
+    }
+  }
+#ifdef LBM_EXPERIMENTS
+  if (threadIdx.x == 0) {
+    const unsigned long long t_end = global_timer_ns();
+    atomicMin(&tb3_exp_blocks[0], t_start);
+    atomicMax(&tb3_exp_blocks[1], t_end);
+    atomicAdd(&tb3_exp_blocks[2], t_end - t_start);
+  }
+#endif
 }
 
 }  // namespace lbm

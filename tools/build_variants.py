@@ -22,7 +22,9 @@ VARIANTS = {
     "tb2_t64": ["-DLBM_TB2_THREADS=64", "-DLBM_TB2_MIN_BLOCKS=6"],
     "tb3_t64": ["-DLBM_TB2_THREADS=64", "-DLBM_TB3_MIN_BLOCKS=4"],     # K10, 64-thread strips (profiles/r03_k10.md)
     "tb3_mb2": ["-DLBM_TB3_MIN_BLOCKS=2"],                              # K10, 186 registers, 6 warps per SM
-    "tb3_wait": ["-DLBM_EXPERIMENTS"],    # K10's staging-wait share of its cycles (run with --kernel tb3), r07
+    # K10's staging-wait share of its cycles (r07) and the busy fraction of its block slots (r08; run with
+    # --kernel tb3, and LBM_GPU_NO_TB3_OVERLAP=1 for passes that do not overlap)
+    "tb3_wait": ["-DLBM_EXPERIMENTS"],
 }
 if os.environ.get("LBM_VARIANTS"):
     VARIANTS = {k: v for k, v in VARIANTS.items() if k in os.environ["LBM_VARIANTS"].split(",")}

@@ -36,15 +36,22 @@ print("mask %.2fs create %.2fs free_cells %d" % (t1 - t0, t2 - t1, lat.info().fr
 # K10's staging-wait counters, in -DLBM_EXPERIMENTS builds (tools/build_variants.py tb3_wait) only
 exp_cycles = getattr(L.load_library(), "lbm_gpu_exp_tb3_cycles", None)
 cyc = (ctypes.c_ulonglong * 2)()
+# ... and K10's block times: busy fraction = sum of block times / (resident blocks x span of the run)
+exp_blocks = getattr(L.load_library(), "lbm_gpu_exp_tb3_blocks", None)
+blk = (ctypes.c_ulonglong * 4)()
 lat.run_timed(3)
 if exp_cycles:
     exp_cycles(cyc)
+    exp_blocks(blk)
 for r in range(a.reps):
     ms = lat.run_timed(a.steps)
     mlups = a.nx * a.ny * a.steps / ms / 1e3
     wait = ""
     if exp_cycles and exp_cycles(cyc) == 0 and cyc[1]:
         wait = "  K10 staging wait %.2f %% of its cycles" % (100.0 * cyc[0] / cyc[1])
+    if exp_blocks and exp_blocks(blk) == 0 and blk[2]:
+        span = blk[1] - blk[0]
+        wait += "  K10 busy %.2f %% of %d slots over %.3f ms" % (100.0 * blk[2] / (blk[3] * span), blk[3], span * 1e-6)
     print("kernel=%s %dx%d gpus=%d steps=%d: %.3f ms/step  %.0f MLUPS  %.0f GB/s (x72B; x144B if f64)%s" %
           (a.kernel, a.nx, a.ny, a.gpus, a.steps, ms / a.steps, mlups, mlups * 72e-3, wait), flush=True)
 av = lat.run(5)
