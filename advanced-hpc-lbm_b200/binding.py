@@ -91,6 +91,8 @@ SYMBOLS = {
     "lbm_gpu_digest": (C.c_int, [_P, C.POINTER(C.c_double), C.POINTER(C.c_ulonglong)]),
     "lbm_gpu_upload": (C.c_int, [_P, _P]),
     "lbm_gpu_upload_f64": (C.c_int, [_P, _P]),
+    "lbm_gpu_save_rows": (C.c_int, [_P, C.c_longlong, C.c_longlong, _P]),
+    "lbm_gpu_load_rows": (C.c_int, [_P, C.c_longlong, C.c_longlong, _P]),
     "lbm_gpu_get_info": (C.c_int, [_P, C.POINTER(Info)]),
     "lbm_gpu_destroy": (None, [_P]),
     "lbm_gpu_host_alloc": (C.c_int, [C.c_size_t, C.POINTER(_P)]),
@@ -202,6 +204,7 @@ class Lattice:
                 assert obstacles.size == rows * self.nx
         self.rows = rows
         self.row0 = 0 if slab is None else int(slab[0])
+        self.f16 = bool(flags & STORE_F16)
         dev = None
         if device_ids is not None:
             dev = np.ascontiguousarray(device_ids, dtype=np.int32)
@@ -278,6 +281,31 @@ class Lattice:
         assert cells.size == self.rows * self.nx * 9
         fn = self.lib.lbm_gpu_upload_f64 if self.f64 else self.lib.lbm_gpu_upload
         _check(fn(self.h, _ptr(cells)))
+
+    @property
+    def record_dtype(self):
+        """Element type of save_rows / load_rows: the handle's stored type (binary16 as uint16 bits)."""
+        return np.float64 if self.f64 else (np.uint16 if self.f16 else np.float32)
+
+    def save_rows(self, row0=None, nrows=None):
+        """Rows [row0, row0 + nrows) of the stored lattice, (nrows, nx, 9) of record_dtype, bit for bit
+        (lbm_gpu_save_rows).  By default every row this handle holds."""
+        row0 = self.row0 if row0 is None else int(row0)
+        nrows = self.row0 + self.rows - row0 if nrows is None else int(nrows)
+        out = np.empty((max(nrows, 0), self.nx, 9), dtype=self.record_dtype)
+        _check(self.lib.lbm_gpu_save_rows(self.h, row0, nrows, _ptr(out)))
+        return out
+
+    def load_rows(self, row0, arr):
+        """Put rows saved by save_rows back from row0 on (lbm_gpu_load_rows).  A slab handle that holds
+        part of the grid must pass barrier / ipc_prepare / barrier with the other ranks before it runs."""
+        arr = np.asarray(arr)
+        if arr.dtype != self.record_dtype:
+            raise LbmError("load_rows: records of this lattice are %s, got %s" % (np.dtype(self.record_dtype), arr.dtype))
+        if arr.ndim != 3 or arr.shape[1:] != (self.nx, 9):
+            raise LbmError("load_rows: need shape (nrows, %d, 9), got %s" % (self.nx, arr.shape))
+        arr = np.ascontiguousarray(arr)
+        _check(self.lib.lbm_gpu_load_rows(self.h, int(row0), arr.shape[0], _ptr(arr)))
 
     def final_fields(self, row0=None, nrows=None, out=None):
         """(u_x, u_y, |u|, pressure) as write_values computes them (d2q9-bgk.c:2937-2976)."""

@@ -196,6 +196,7 @@ class Grid : public GridBase {
   int pairs_tile_rows = 0;     // K9: rows per block
   bool f16 = false;            // LBM_GPU_STORE_F16: the lattice buffers hold shifted binary16 (lbm_f16.cuh)
   bool failed = false;         // a neighbour never arrived: the lattice contents are void
+  bool loaded_unprepared = false;   // a slab handle took rows from lbm_gpu_load_rows: lbm_gpu_ipc_prepare must come first
   unsigned long long timeout_ns = 10000000000ULL;
   long long launches = 0;
   double last_run_ms = 0.0, last_step_ms = 0.0;
@@ -911,6 +912,7 @@ class Grid : public GridBase {
       launches++;
     }
     for (auto& s : slabs) { CK(cudaSetDevice(s.device)); CK(cudaStreamSynchronize(s.stream)); }
+    loaded_unprepared = false;
   }
 
   // -------------------------------------------------------------------- run ----
@@ -1002,6 +1004,9 @@ class Grid : public GridBase {
     if (!connected) throw CudaError{"lattice is not connected to its neighbours yet"};
     if (failed) throw CudaError{"an earlier run of this lattice was abandoned (a neighbouring slab never arrived); "
                                 "its contents are void"};
+    if (loaded_unprepared)
+      throw CudaError{"rows were loaded into this slab handle with lbm_gpu_load_rows and its neighbours' ghost rows are "
+                      "stale: pass a host barrier over all ranks, lbm_gpu_ipc_prepare, and a second barrier first"};
     double ms = 0.0;
     const int total = n_steps;
     for (int done = 0; done < total; done += kMaxSegmentSteps) {
@@ -1393,6 +1398,88 @@ class Grid : public GridBase {
       CK(cudaStreamSynchronize(s.stream));
       g += n;
     }
+  }
+
+  // lbm_gpu_save_rows / lbm_gpu_load_rows: the stored lattice as cell-major records of 9 stored
+  // elements (lbm_pack_rows, lbm_unpack_rows), nothing decoded or rounded
+  size_t rec_bytes() const { return f16 ? sizeof(__half) : sizeof(real); }
+
+  template <typename T>
+  void launch_rec(bool save, Slab<real>& s, void* st, int r, int n) {
+    const long long ncells = (long long)n * prm.nx;
+    const dim3 grid((unsigned)((ncells + lbm::kRecCells - 1) / lbm::kRecCells));
+    T* planes = reinterpret_cast<T*>(s.lattice[cur]);
+    T* rec = static_cast<T*>(st);
+    const bool vec = prm.nx % (int)(16 / sizeof(T)) == 0;
+    if (save && vec)  lbm::lbm_pack_rows<T, true><<<grid, lbm::kRecThreads, 0, s.stream>>>(planes, rec, plane_stride(s), pitch, prm.nx, r, ncells);
+    if (save && !vec) lbm::lbm_pack_rows<T, false><<<grid, lbm::kRecThreads, 0, s.stream>>>(planes, rec, plane_stride(s), pitch, prm.nx, r, ncells);
+    if (!save && vec)  lbm::lbm_unpack_rows<T, true><<<grid, lbm::kRecThreads, 0, s.stream>>>(rec, planes, plane_stride(s), pitch, prm.nx, r, ncells);
+    if (!save && !vec) lbm::lbm_unpack_rows<T, false><<<grid, lbm::kRecThreads, 0, s.stream>>>(rec, planes, plane_stride(s), pitch, prm.nx, r, ncells);
+    CK(cudaGetLastError());
+    launches++;
+  }
+
+  // Rows [row0, row0+nrows) between the lattice and the host's records, chunk by chunk through
+  // the two halves of the staging buffer: the kernel of chunk i+1 overlaps the copy of chunk i on
+  // copy_stream, one synchronisation per call.  A range that crosses slabs is cut at their
+  // boundaries.  After a load the side row and the ghost rows of the new contents are rebuilt
+  // (prepare), except on a slab handle that holds part of the grid: its pushes reach other
+  // processes' windows, so there lbm_gpu_ipc_prepare between two host barriers does it.
+  void move_rows(bool save, long long row0, long long nrows, void* host) {
+    const size_t row_bytes = (size_t)prm.nx * 9 * rec_bytes();
+    const size_t half = kStagingBytes / 2;
+    if (row_bytes > half) throw CudaError{"nx too large for the record staging buffer"};
+    check_rows(row0, nrows);
+    if (nrows == 0) return;
+    const int chunk_rows = (int)(half / row_bytes);
+    std::vector<Slab<real>*> used;
+    long long g = row0;
+    int i = 0;
+    while (g < row0 + nrows) {
+      Slab<real>& s = slab_of_row(g);
+      CK(cudaSetDevice(s.device));
+      if (used.empty() || used.back() != &s) {
+        used.push_back(&s);
+        i = 0;
+        CK(cudaEventRecord(s.stage_drained[0], s.stream));     // the halves are free once earlier work is done
+        CK(cudaEventRecord(s.stage_drained[1], s.stream));
+      }
+      const int n = (int)std::min<long long>({(long long)chunk_rows, s.row0 + s.rows - g, row0 + nrows - g});
+      const int b = i & 1;
+      char* st = (char*)s.staging + (size_t)b * half;
+      char* h = (char*)host + (size_t)(g - row0) * row_bytes;
+      const size_t bytes = (size_t)n * row_bytes;
+      const int r = (int)(g - s.row0);
+      if (save) {
+        CK(cudaStreamWaitEvent(s.stream, s.stage_drained[b], 0));
+        if (f16) launch_rec<uint16_t>(true, s, st, r, n);
+        else if (sizeof(real) == 8) launch_rec<uint64_t>(true, s, st, r, n);
+        else launch_rec<uint32_t>(true, s, st, r, n);
+        CK(cudaEventRecord(s.stage_filled[b], s.stream));
+        CK(cudaStreamWaitEvent(s.copy_stream, s.stage_filled[b], 0));
+        CK(cudaMemcpyAsync(h, st, bytes, cudaMemcpyDeviceToHost, s.copy_stream));
+        CK(cudaEventRecord(s.stage_drained[b], s.copy_stream));
+      } else {
+        CK(cudaStreamWaitEvent(s.copy_stream, s.stage_drained[b], 0));
+        CK(cudaMemcpyAsync(st, h, bytes, cudaMemcpyHostToDevice, s.copy_stream));
+        CK(cudaEventRecord(s.stage_filled[b], s.copy_stream));
+        CK(cudaStreamWaitEvent(s.stream, s.stage_filled[b], 0));
+        if (f16) launch_rec<uint16_t>(false, s, st, r, n);
+        else if (sizeof(real) == 8) launch_rec<uint64_t>(false, s, st, r, n);
+        else launch_rec<uint32_t>(false, s, st, r, n);
+        CK(cudaEventRecord(s.stage_drained[b], s.stream));
+      }
+      g += n;
+      i++;
+    }
+    for (Slab<real>* s : used) {
+      CK(cudaSetDevice(s->device));
+      CK(cudaStreamSynchronize(s->copy_stream));
+      CK(cudaStreamSynchronize(s->stream));
+    }
+    if (save) return;
+    if (!slab_mode || slabs[0].rows == prm.ny) prepare();
+    else loaded_unprepared = true;
   }
 
   // Fields of rows [row0, row0+nrows): computed chunk by chunk into one half of the staging
@@ -2289,6 +2376,30 @@ int lbm_gpu_digest(lbm_gpu* h, double* total_density, unsigned long long* checks
   if (reinterpret_cast<GridBase*>(h)->is_f64())
     return guarded<double>(h, "lbm_gpu_digest", [&](Grid<double>& g) { g.digest(total_density, checksum); });
   return guarded<float>(h, "lbm_gpu_digest", [&](Grid<float>& g) { g.digest(total_density, checksum); });
+}
+
+namespace {
+// lbm_gpu_save_rows / lbm_gpu_load_rows for either precision; refused before anything is enqueued
+int move_rows_impl(lbm_gpu* h, bool save, long long row0, long long nrows, void* p) {
+  const char* fn = save ? "lbm_gpu_save_rows" : "lbm_gpu_load_rows";
+  if (!h) return fail("%s: NULL handle", fn);
+  if (nrows < 0) return fail("%s: negative nrows (%lld)", fn, nrows);
+  if (!p && nrows > 0) return fail("%s: NULL %s for %lld rows", fn, save ? "output" : "input", nrows);
+  auto body = [&](auto& g) {
+    if (g.failed) throw CudaError{"an earlier run of this lattice was abandoned (a neighbouring slab never arrived); "
+                                  "its contents are void"};
+    g.move_rows(save, row0, nrows, p);
+  };
+  if (reinterpret_cast<GridBase*>(h)->is_f64()) return guarded<double>(h, fn, body);
+  return guarded<float>(h, fn, body);
+}
+}  // namespace
+
+int lbm_gpu_save_rows(lbm_gpu* h, long long row0, long long nrows, void* out) {
+  return move_rows_impl(h, true, row0, nrows, out);
+}
+int lbm_gpu_load_rows(lbm_gpu* h, long long row0, long long nrows, const void* in) {
+  return move_rows_impl(h, false, row0, nrows, const_cast<void*>(in));
 }
 
 int lbm_gpu_upload(lbm_gpu* h, const float* cells_aos) {

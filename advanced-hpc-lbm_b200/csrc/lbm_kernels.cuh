@@ -1275,6 +1275,91 @@ __global__ void lbm_soa_to_aos(const store* __restrict__ buf, real* __restrict__
   aos[i] = stored_value(buf + k * plane_stride + (r0 + row) * pitch + x, k, rest);
 }
 
+// lbm_gpu_save_rows / lbm_gpu_load_rows: the stored lattice <-> cell-major records (9 elements per
+// cell, speed order), bits moved unchanged.  T is the unsigned type of the stored element (uint32
+// fp32, uint64 fp64, uint16 binary16).  A block takes kRecCells consecutive cells of the chunk
+// (local rows [r0, r0 + ncells / nx)) and transposes them in shared memory, which holds them in
+// record order: the record side is then one contiguous run of 16-byte accesses (the chunk starts
+// 16-byte aligned and kRecCells * 9 elements is a multiple of 16 bytes), and the plane side reads
+// or writes x-consecutive elements, 16 bytes at a time when VEC (nx a multiple of 16 / sizeof(T),
+// so that a vector never crosses a row; pitch is a multiple of 32).  Columns nx..pitch-1 (padding)
+// are never touched.
+constexpr int kRecCells = 256;
+constexpr int kRecThreads = 256;
+
+template <typename T, bool VEC>
+__global__ void __launch_bounds__(kRecThreads) lbm_pack_rows(const T* __restrict__ buf, T* __restrict__ rec,
+                                                             long long plane_stride, int pitch, int nx, int r0,
+                                                             long long ncells) {
+  constexpr int V = 16 / sizeof(T);
+  __shared__ __align__(16) T sm[kRecCells * 9];
+  const long long c0 = (long long)blockIdx.x * kRecCells;
+  const int nc = (int)min((long long)kRecCells, ncells - c0);
+  const long long row_c0 = c0 / nx;
+  const int x_c0 = (int)(c0 - row_c0 * nx);
+  if (VEC) {
+    for (int j = threadIdx.x; j < 9 * (kRecCells / V); j += kRecThreads) {
+      const int k = j / (kRecCells / V), c = (j - k * (kRecCells / V)) * V;
+      if (c >= nc) continue;
+      const int xc = x_c0 + c, dr = xc / nx;
+      const uint4 v = *reinterpret_cast<const uint4*>(buf + k * plane_stride + (r0 + row_c0 + dr) * pitch + (xc - dr * nx));
+      const T* e = reinterpret_cast<const T*>(&v);
+#pragma unroll
+      for (int q = 0; q < V; q++) sm[(c + q) * 9 + k] = e[q];
+    }
+  } else {
+    for (int j = threadIdx.x; j < 9 * kRecCells; j += kRecThreads) {
+      const int k = j / kRecCells, c = j - k * kRecCells;
+      if (c >= nc) continue;
+      const int xc = x_c0 + c, dr = xc / nx;
+      sm[c * 9 + k] = buf[k * plane_stride + (r0 + row_c0 + dr) * pitch + (xc - dr * nx)];
+    }
+  }
+  __syncthreads();
+  T* out = rec + c0 * 9;
+  const int n = nc * 9, nv = n / V;
+  for (int j = threadIdx.x; j < nv; j += kRecThreads)
+    reinterpret_cast<uint4*>(out)[j] = reinterpret_cast<const uint4*>(sm)[j];
+  for (int j = nv * V + threadIdx.x; j < n; j += kRecThreads) out[j] = sm[j];
+}
+
+template <typename T, bool VEC>
+__global__ void __launch_bounds__(kRecThreads) lbm_unpack_rows(const T* __restrict__ rec, T* __restrict__ buf,
+                                                               long long plane_stride, int pitch, int nx, int r0,
+                                                               long long ncells) {
+  constexpr int V = 16 / sizeof(T);
+  __shared__ __align__(16) T sm[kRecCells * 9];
+  const long long c0 = (long long)blockIdx.x * kRecCells;
+  const int nc = (int)min((long long)kRecCells, ncells - c0);
+  const long long row_c0 = c0 / nx;
+  const int x_c0 = (int)(c0 - row_c0 * nx);
+  const T* in = rec + c0 * 9;
+  const int n = nc * 9, nv = n / V;
+  for (int j = threadIdx.x; j < nv; j += kRecThreads)
+    reinterpret_cast<uint4*>(sm)[j] = reinterpret_cast<const uint4*>(in)[j];
+  for (int j = nv * V + threadIdx.x; j < n; j += kRecThreads) sm[j] = in[j];
+  __syncthreads();
+  if (VEC) {
+    for (int j = threadIdx.x; j < 9 * (kRecCells / V); j += kRecThreads) {
+      const int k = j / (kRecCells / V), c = (j - k * (kRecCells / V)) * V;
+      if (c >= nc) continue;
+      const int xc = x_c0 + c, dr = xc / nx;
+      uint4 v;
+      T* e = reinterpret_cast<T*>(&v);
+#pragma unroll
+      for (int q = 0; q < V; q++) e[q] = sm[(c + q) * 9 + k];
+      *reinterpret_cast<uint4*>(buf + k * plane_stride + (r0 + row_c0 + dr) * pitch + (xc - dr * nx)) = v;
+    }
+  } else {
+    for (int j = threadIdx.x; j < 9 * kRecCells; j += kRecThreads) {
+      const int k = j / kRecCells, c = j - k * kRecCells;
+      if (c >= nc) continue;
+      const int xc = x_c0 + c, dr = xc / nx;
+      buf[k * plane_stride + (r0 + row_c0 + dr) * pitch + (xc - dr * nx)] = sm[c * 9 + k];
+    }
+  }
+}
+
 // int-per-cell obstacle rows -> bit mask rows; one warp packs 32 cells with a ballot.
 // Also counts the blocked cells.
 __global__ void lbm_pack_mask(const int* __restrict__ obst, uint32_t* __restrict__ mask, int mask_pitch,

@@ -23,9 +23,20 @@
  *                          timestep print its number, average velocity and total density
  *                          (one lbm_gpu_run + lbm_gpu_digest per step: slow, for eyeballing
  *                          mass conservation)
+ *   LBM_CHECKPOINT=path    after the last step, before final_state.dat, write a checkpoint
+ *                          (stored lattice bit for bit, av_vels so far; format in lbm_io.h) to
+ *                          path.tmp, then fsync and rename it to path
+ *   LBM_CHECKPOINT_EVERY=k also write one after every k steps (step counts that are multiples
+ *                          of k): the run is cut into lbm_gpu_run calls of k steps, which changes
+ *                          no output bit
+ *   LBM_RESTART=path       continue from a checkpoint of the same parameter file (maxIters may be
+ *                          larger), obstacle file, LBM_PRECISION and LBM_STRICT; LBM_GPUS may
+ *                          differ.  The header is checked before the GPU is touched; av_vels.dat
+ *                          then holds all maxIters lines and both files equal an uninterrupted run's
  */
 #define _POSIX_C_SOURCE 200809L
 #include <math.h>
+#include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -54,6 +65,42 @@ static double wtime(void)
   do {                                                                  \
     if ((call) != 0) die(lbm_gpu_last_error(), __LINE__, __FILE__);     \
   } while (0)
+
+/* the lattice side of a checkpoint (lbm_io.c streams the file a block of rows at a time) */
+static void save_rows_cb(void* gpu, long long row0, long long nrows, void* buf)
+{
+  GPU(lbm_gpu_save_rows((lbm_gpu*)gpu, row0, nrows, buf));
+}
+
+static void load_rows_cb(void* gpu, long long row0, long long nrows, void* buf)
+{
+  GPU(lbm_gpu_load_rows((lbm_gpu*)gpu, row0, nrows, buf));
+}
+
+/* one block of checkpoint rows, page-locked where the library can give it */
+static void* ckpt_buffer(const lbm_ckpt_header* h, int* pinned)
+{
+  const size_t rec = h->kind == LBM_CKPT_F64 ? 72 : h->kind == LBM_CKPT_F16 ? 18 : 36;
+  const size_t bytes = (size_t)lbm_ckpt_block_rows(h) * (size_t)h->nx * rec;
+  void* p = NULL;
+  *pinned = lbm_gpu_host_alloc(bytes, &p) == 0;
+  if (!*pinned) p = malloc(bytes);
+  if (p == NULL) die("cannot allocate memory for checkpoint rows", __LINE__, __FILE__);
+  return p;
+}
+
+static void write_checkpoint(const char* path, lbm_gpu* gpu, lbm_ckpt_header* h, int steps_done, const void* av_vels)
+{
+  unsigned long long checksum = 0;
+  GPU(lbm_gpu_digest(gpu, NULL, &checksum));
+  h->steps_done = steps_done;
+  h->checksum = checksum;
+  int pinned;
+  void* buf = ckpt_buffer(h, &pinned);
+  lbm_write_checkpoint(path, h, av_vels, save_rows_cb, gpu, buf);
+  if (pinned) lbm_gpu_host_free(buf);
+  else free(buf);
+}
 
 static int env_flag(const char* name)
 {
@@ -85,6 +132,19 @@ int main(int argc, char* argv[])
     else die("LBM_KERNEL must be scalar, vec4, persistent, tma, cluster, tb2, tb3 or pairs", __LINE__, __FILE__);
   }
 
+  const char* ckpt_path = getenv("LBM_CHECKPOINT");
+  const char* restart_path = getenv("LBM_RESTART");
+  if (ckpt_path != NULL && ckpt_path[0] == '\0') ckpt_path = NULL;
+  if (restart_path != NULL && restart_path[0] == '\0') restart_path = NULL;
+  long long every = 0;
+  if (getenv("LBM_CHECKPOINT_EVERY") != NULL) {
+    char* end = NULL;
+    every = strtoll(getenv("LBM_CHECKPOINT_EVERY"), &end, 10);
+    if (end == getenv("LBM_CHECKPOINT_EVERY") || *end != '\0' || every < 1)
+      die("LBM_CHECKPOINT_EVERY must be a positive number of steps", __LINE__, __FILE__);
+    if (ckpt_path == NULL) die("LBM_CHECKPOINT_EVERY needs LBM_CHECKPOINT=<path>", __LINE__, __FILE__);
+  }
+
   /* Total/init time starts here: load values from file, build the device lattice */
   const double tot_tic = wtime();
   const double init_tic = tot_tic;
@@ -100,17 +160,46 @@ int main(int argc, char* argv[])
   float* av_vels_f = (float*)malloc(sizeof(float) * (size_t)(iters > 0 ? iters : 1));
   if (av_vels == NULL || av_vels_f == NULL) die("cannot allocate memory for av_vels", __LINE__, __FILE__);
 
+  /* a checkpoint is checked against this run's inputs before the GPU is touched */
+  lbm_ckpt_header ckpt;
+  FILE* restart_fp = NULL;
+  lbm_ckpt_header restart_hdr;
+  int t0 = 0;
+  if (ckpt_path != NULL || restart_path != NULL) {
+    const uint32_t kind = f64 ? LBM_CKPT_F64 : (flags & LBM_GPU_STORE_F16) ? LBM_CKPT_F16 : LBM_CKPT_F32;
+    lbm_ckpt_header_init(&ckpt, kind, (flags & LBM_GPU_STRICT) != 0, &params, &params_d,
+                         lbm_obstacle_hash(obstacle_bits, nx, ny));
+  }
+  if (restart_path != NULL) {
+    restart_fp = lbm_open_checkpoint(restart_path, &ckpt, iters, &restart_hdr);
+    t0 = (int)restart_hdr.steps_done;
+  }
+
   /* the rest-state lattice (d2q9-bgk.c:2802-2823) is generated on the device */
   lbm_gpu* gpu = NULL;
   if (f64) GPU(lbm_gpu_create_f64(&params_d, NULL, obstacle_bits, n_gpus, NULL, flags, &gpu));
   else GPU(lbm_gpu_create(&params, NULL, obstacle_bits, n_gpus, NULL, flags, &gpu));
+  if (restart_fp != NULL) {      /* ... or the checkpoint's lattice and av_vels replace it */
+    int pinned;
+    void* buf = ckpt_buffer(&restart_hdr, &pinned);
+    lbm_read_checkpoint(restart_fp, &restart_hdr, f64 ? (void*)av_vels : (void*)av_vels_f, load_rows_cb, gpu, buf);
+    if (pinned) lbm_gpu_host_free(buf);
+    else free(buf);
+    if (!f64)
+      for (int t = 0; t < t0; t++) av_vels[t] = av_vels_f[t];
+    unsigned long long checksum = 0;
+    GPU(lbm_gpu_digest(gpu, NULL, &checksum));
+    if (checksum != restart_hdr.checksum)
+      die("checkpoint lattice checksum differs from the one in its header: the file is corrupt", __LINE__, __FILE__);
+  }
 
   /* Init time stops here, compute time starts */
   const double init_toc = wtime();
   const double comp_tic = init_toc;
 
+  double ckpt_secs = 0.0;        /* checkpoint writes, not counted as compute time */
   if (env_flag("LBM_DEBUG")) {
-    for (int tt = 0; tt < iters; tt++) {
+    for (int tt = t0; tt < iters; tt++) {
       double density;
       if (f64) {
         GPU(lbm_gpu_run_f64(gpu, 1, &av_vels[tt]));
@@ -123,17 +212,29 @@ int main(int argc, char* argv[])
       printf("av velocity: %.12E\n", av_vels[tt]);
       printf("tot density: %.12E\n", density);
     }
-  } else if (f64) {
-    GPU(lbm_gpu_run_f64(gpu, iters, av_vels));
   } else {
-    GPU(lbm_gpu_run(gpu, iters, av_vels_f));
-    for (int t = 0; t < iters; t++) av_vels[t] = av_vels_f[t];
+    /* steps [t0, iters), cut at the multiples of LBM_CHECKPOINT_EVERY */
+    for (int t = t0; t < iters;) {
+      const int next = every > 0 ? (int)(((long long)t / every + 1) * every < iters ? ((long long)t / every + 1) * every : iters)
+                                 : iters;
+      if (f64) GPU(lbm_gpu_run_f64(gpu, next - t, av_vels + t));
+      else GPU(lbm_gpu_run(gpu, next - t, av_vels_f + t));
+      t = next;
+      if (every > 0 && t < iters) {
+        const double tic = wtime();
+        write_checkpoint(ckpt_path, gpu, &ckpt, t, f64 ? (const void*)av_vels : (const void*)av_vels_f);
+        ckpt_secs += wtime() - tic;
+      }
+    }
+    if (!f64)
+      for (int t = 0; t < iters; t++) av_vels[t] = av_vels_f[t];
   }
 
   /* Compute time stops here (lbm_gpu_run returns with the device idle), collate time
    * starts: bring the results of all GPUs back to the host */
-  const double comp_toc = wtime();
-  const double col_tic = comp_toc;
+  const double comp_end = wtime();
+  const double comp_toc = comp_end - ckpt_secs;
+  const double col_tic = comp_end;
 
   double reynolds;
   if (f64) {
@@ -149,7 +250,7 @@ int main(int argc, char* argv[])
   }
 
   const double col_toc = wtime();
-  const double tot_toc = col_toc;
+  const double tot_toc = col_toc - ckpt_secs;
 
   /* write final values and free memory */
   printf("==done==\n");
@@ -182,6 +283,13 @@ int main(int argc, char* argv[])
       printf("Algorithmic GB/s (72 B/update):\t\t%.1f\n", updates * 72.0 / dev_s / 1e9);
     }
     printf("MLUPS (wall compute time):\t\t%.1f\n", updates / (comp_toc - comp_tic) / 1e6);
+  }
+
+  if (ckpt_path != NULL) {
+    const double tic = wtime();
+    write_checkpoint(ckpt_path, gpu, &ckpt, iters, f64 ? (const void*)av_vels : (const void*)av_vels_f);
+    ckpt_secs += wtime() - tic;
+    printf("Elapsed Checkpoint time:\t\t%.6lf (s)\n", ckpt_secs);
   }
 
   /* write_values (d2q9-bgk.c:2918-2999): the per-cell fields are computed on the GPU

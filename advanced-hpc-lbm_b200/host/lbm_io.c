@@ -8,6 +8,8 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <sys/types.h>
+#include <unistd.h>
 
 void die(const char* message, const int line, const char* file)
 {
@@ -285,6 +287,201 @@ void lbm_write_av_vels(const char* path, int n, const double* av_vels)
     o += lbm_format_e12(o, av_vels[ii]);
     *o++ = '\n';
     fwrite(line, 1, (size_t)(o - line), fp);
+  }
+  fclose(fp);
+}
+
+/* ---------------------------------------------------------------------------------
+ * Checkpoint file (layout in lbm_io.h).  Written and read through lbm_gpu_save_rows /
+ * lbm_gpu_load_rows a block of rows at a time: the whole lattice is never on the host.
+ * --------------------------------------------------------------------------------- */
+static const char ckpt_magic[8] = {'L', 'B', 'M', 'C', 'K', 'P', 'T', '\0'};
+
+static size_t ckpt_record_bytes(uint32_t kind) { return kind == LBM_CKPT_F64 ? 72 : kind == LBM_CKPT_F16 ? 18 : 36; }
+static size_t ckpt_av_bytes(uint32_t kind) { return kind == LBM_CKPT_F64 ? 8 : 4; }
+static const char* ckpt_kind_name(uint32_t kind)
+{
+  return kind == LBM_CKPT_F32 ? "fp32" : kind == LBM_CKPT_F64 ? "fp64 (LBM_PRECISION=f64)"
+       : kind == LBM_CKPT_F16 ? "binary16 (LBM_PRECISION=f16)" : "unknown";
+}
+
+static void put_le(unsigned char* p, uint64_t v, int n)
+{
+  for (int i = 0; i < n; i++) p[i] = (unsigned char)(v >> (8 * i));
+}
+static uint64_t get_le(const unsigned char* p, int n)
+{
+  uint64_t v = 0;
+  for (int i = 0; i < n; i++) v |= (uint64_t)p[i] << (8 * i);
+  return v;
+}
+
+/* the av_vels and lattice sections are copied as they are in memory */
+static void ckpt_require_little_endian(void)
+{
+  const uint16_t one = 1;
+  if (*(const unsigned char*)&one != 1) die("checkpoint files are little-endian and this host is not", __LINE__, __FILE__);
+}
+
+uint64_t lbm_obstacle_hash(const uint32_t* bits, int nx, int ny)
+{
+  const size_t n = (size_t)((nx + 31) / 32) * (size_t)ny;
+  uint64_t h = 0xcbf29ce484222325ULL;
+  for (size_t i = 0; i < n; i++) {
+    h ^= bits[i];
+    h *= 0x100000001b3ULL;
+  }
+  return h;
+}
+
+void lbm_ckpt_header_init(lbm_ckpt_header* h, uint32_t kind, int strict, const lbm_param* pf,
+                          const lbm_param_f64* pd, uint64_t obstacle_hash)
+{
+  memset(h, 0, sizeof *h);
+  h->version = 1;
+  h->kind = kind;
+  h->strict = strict ? 1u : 0u;
+  h->nx = pf->nx; h->ny = pf->ny; h->reynolds_dim = pf->reynolds_dim;
+  memcpy(&h->density_f32, &pf->density, 4); memcpy(&h->accel_f32, &pf->accel, 4); memcpy(&h->omega_f32, &pf->omega, 4);
+  memcpy(&h->density_f64, &pd->density, 8); memcpy(&h->accel_f64, &pd->accel, 8); memcpy(&h->omega_f64, &pd->omega, 8);
+  h->obstacle_hash = obstacle_hash;
+}
+
+static void ckpt_encode(const lbm_ckpt_header* h, unsigned char* b)
+{
+  memset(b, 0, LBM_CKPT_HEADER_BYTES);
+  memcpy(b, ckpt_magic, 8);
+  put_le(b + 8, h->version, 4); put_le(b + 12, h->kind, 4); put_le(b + 16, h->strict, 4);
+  put_le(b + 20, (uint32_t)h->nx, 4); put_le(b + 24, (uint32_t)h->ny, 4); put_le(b + 28, (uint32_t)h->reynolds_dim, 4);
+  put_le(b + 32, h->density_f32, 4); put_le(b + 36, h->accel_f32, 4); put_le(b + 40, h->omega_f32, 4);
+  put_le(b + 48, h->density_f64, 8); put_le(b + 56, h->accel_f64, 8); put_le(b + 64, h->omega_f64, 8);
+  put_le(b + 72, (uint64_t)h->steps_done, 8); put_le(b + 80, h->obstacle_hash, 8); put_le(b + 88, h->checksum, 8);
+}
+
+static void ckpt_decode(const unsigned char* b, lbm_ckpt_header* h)
+{
+  h->version = (uint32_t)get_le(b + 8, 4); h->kind = (uint32_t)get_le(b + 12, 4); h->strict = (uint32_t)get_le(b + 16, 4);
+  h->nx = (int32_t)get_le(b + 20, 4); h->ny = (int32_t)get_le(b + 24, 4); h->reynolds_dim = (int32_t)get_le(b + 28, 4);
+  h->density_f32 = (uint32_t)get_le(b + 32, 4); h->accel_f32 = (uint32_t)get_le(b + 36, 4); h->omega_f32 = (uint32_t)get_le(b + 40, 4);
+  h->density_f64 = get_le(b + 48, 8); h->accel_f64 = get_le(b + 56, 8); h->omega_f64 = get_le(b + 64, 8);
+  h->steps_done = (int64_t)get_le(b + 72, 8); h->obstacle_hash = get_le(b + 80, 8); h->checksum = get_le(b + 88, 8);
+}
+
+long long lbm_ckpt_block_rows(const lbm_ckpt_header* h)
+{
+  long long n = (long long)((64u << 20) / ((size_t)h->nx * ckpt_record_bytes(h->kind)));
+  if (n < 1) n = 1;
+  if (n > h->ny) n = h->ny;
+  return n;
+}
+
+void lbm_write_checkpoint(const char* path, const lbm_ckpt_header* h, const void* av_vels,
+                          lbm_ckpt_rows_fn save_rows, void* ctx, void* buf)
+{
+  char message[1024];
+  ckpt_require_little_endian();
+  char* tmp = (char*)malloc(strlen(path) + 5);
+  if (tmp == NULL) die("cannot allocate memory for the checkpoint path", __LINE__, __FILE__);
+  sprintf(tmp, "%s.tmp", path);
+  FILE* fp = fopen(tmp, "wb");
+  if (fp == NULL) {
+    snprintf(message, sizeof message, "could not open checkpoint file for writing: %s", tmp);
+    die(message, __LINE__, __FILE__);
+  }
+  unsigned char hb[LBM_CKPT_HEADER_BYTES];
+  ckpt_encode(h, hb);
+  int ok = fwrite(hb, 1, sizeof hb, fp) == sizeof hb;
+  const size_t avb = ckpt_av_bytes(h->kind);
+  if (ok && h->steps_done > 0) ok = fwrite(av_vels, avb, (size_t)h->steps_done, fp) == (size_t)h->steps_done;
+  const size_t row_bytes = (size_t)h->nx * ckpt_record_bytes(h->kind);
+  const long long block = lbm_ckpt_block_rows(h);
+  for (long long r0 = 0; ok && r0 < h->ny; r0 += block) {
+    const long long nr = (r0 + block <= h->ny) ? block : h->ny - r0;
+    save_rows(ctx, r0, nr, buf);
+    ok = fwrite(buf, row_bytes, (size_t)nr, fp) == (size_t)nr;
+  }
+  ok = ok && fflush(fp) == 0 && fsync(fileno(fp)) == 0;
+  ok = (fclose(fp) == 0) && ok;
+  if (!ok) {
+    snprintf(message, sizeof message, "could not write checkpoint file: %s", tmp);
+    die(message, __LINE__, __FILE__);
+  }
+  if (rename(tmp, path) != 0) {
+    snprintf(message, sizeof message, "could not rename %s to %s", tmp, path);
+    die(message, __LINE__, __FILE__);
+  }
+  free(tmp);
+}
+
+FILE* lbm_open_checkpoint(const char* path, const lbm_ckpt_header* want, int max_iters, lbm_ckpt_header* got)
+{
+  char message[1024];
+  ckpt_require_little_endian();
+  FILE* fp = fopen(path, "rb");
+  if (fp == NULL) {
+    snprintf(message, sizeof message, "could not open checkpoint file: %s", path);
+    die(message, __LINE__, __FILE__);
+  }
+  unsigned char hb[LBM_CKPT_HEADER_BYTES];
+  const size_t n = fread(hb, 1, sizeof hb, fp);
+  if (n < 8 || memcmp(hb, ckpt_magic, 8) != 0) {
+    snprintf(message, sizeof message, "checkpoint %s: not a checkpoint of this program (wrong magic)", path);
+    die(message, __LINE__, __FILE__);
+  }
+  if (n < sizeof hb) {
+    snprintf(message, sizeof message, "checkpoint %s: truncated header (%zu of %d bytes)", path, n, LBM_CKPT_HEADER_BYTES);
+    die(message, __LINE__, __FILE__);
+  }
+  ckpt_decode(hb, got);
+#define CKPT_MISMATCH(...)                                   \
+  do {                                                       \
+    int k_ = snprintf(message, sizeof message, "checkpoint %s: ", path);   \
+    snprintf(message + k_, sizeof message - (size_t)k_, __VA_ARGS__);      \
+    die(message, __LINE__, __FILE__);                        \
+  } while (0)
+  if (got->version != want->version)
+    CKPT_MISMATCH("format version %u, this program reads version %u", got->version, want->version);
+  if (got->kind != want->kind)
+    CKPT_MISMATCH("holds a %s lattice, this run asks for %s", ckpt_kind_name(got->kind), ckpt_kind_name(want->kind));
+  if (got->strict != want->strict)
+    CKPT_MISMATCH("written with LBM_STRICT=%u, this run has LBM_STRICT=%u", got->strict, want->strict);
+  if (got->nx != want->nx) CKPT_MISMATCH("nx is %d, the parameter file's is %d", got->nx, want->nx);
+  if (got->ny != want->ny) CKPT_MISMATCH("ny is %d, the parameter file's is %d", got->ny, want->ny);
+  if (got->reynolds_dim != want->reynolds_dim)
+    CKPT_MISMATCH("reynolds_dim is %d, the parameter file's is %d", got->reynolds_dim, want->reynolds_dim);
+  if (got->density_f32 != want->density_f32 || got->density_f64 != want->density_f64)
+    CKPT_MISMATCH("density differs from the parameter file's");
+  if (got->accel_f32 != want->accel_f32 || got->accel_f64 != want->accel_f64)
+    CKPT_MISMATCH("accel differs from the parameter file's");
+  if (got->omega_f32 != want->omega_f32 || got->omega_f64 != want->omega_f64)
+    CKPT_MISMATCH("omega differs from the parameter file's");
+  if (got->obstacle_hash != want->obstacle_hash)
+    CKPT_MISMATCH("written with another obstacle file (the obstacle mask hash differs)");
+  if (got->steps_done < 0 || got->steps_done > max_iters)
+    CKPT_MISMATCH("is at step %lld, beyond maxIters = %d of the parameter file", (long long)got->steps_done, max_iters);
+  const long long expect = LBM_CKPT_HEADER_BYTES + got->steps_done * (long long)ckpt_av_bytes(got->kind) +
+                           (long long)got->ny * got->nx * (long long)ckpt_record_bytes(got->kind);
+  if (fseeko(fp, 0, SEEK_END) != 0) CKPT_MISMATCH("cannot seek");
+  const long long size = (long long)ftello(fp);
+  if (size != expect)
+    CKPT_MISMATCH("file has %lld bytes, its header implies %lld (truncated or corrupt)", size, expect);
+#undef CKPT_MISMATCH
+  if (fseeko(fp, LBM_CKPT_HEADER_BYTES, SEEK_SET) != 0) die("cannot seek in the checkpoint file", __LINE__, __FILE__);
+  return fp;
+}
+
+void lbm_read_checkpoint(FILE* fp, const lbm_ckpt_header* h, void* av_vels, lbm_ckpt_rows_fn load_rows,
+                         void* ctx, void* buf)
+{
+  const size_t avb = ckpt_av_bytes(h->kind);
+  if (h->steps_done > 0 && fread(av_vels, avb, (size_t)h->steps_done, fp) != (size_t)h->steps_done)
+    die("could not read the av_vels of the checkpoint file", __LINE__, __FILE__);
+  const size_t row_bytes = (size_t)h->nx * ckpt_record_bytes(h->kind);
+  const long long block = lbm_ckpt_block_rows(h);
+  for (long long r0 = 0; r0 < h->ny; r0 += block) {
+    const long long nr = (r0 + block <= h->ny) ? block : h->ny - r0;
+    if (fread(buf, row_bytes, (size_t)nr, fp) != (size_t)nr) die("could not read the lattice of the checkpoint file", __LINE__, __FILE__);
+    load_rows(ctx, r0, nr, buf);
   }
   fclose(fp);
 }

@@ -12,6 +12,7 @@
 
 #include <stddef.h>
 #include <stdint.h>
+#include <stdio.h>
 #include "lbm_gpu.h"
 
 void die(const char* message, const int line, const char* file);
@@ -37,5 +38,64 @@ void lbm_write_av_vels(const char* path, int n, const double* av_vels);
 
 /* exact equivalent of sprintf(out, "%.12E", v); returns the number of characters */
 int lbm_format_e12(char* out, double v);
+
+/* ---------------------------------------------------------------------------------
+ * Checkpoint file (LBM_CHECKPOINT / LBM_RESTART): one binary file, little-endian.
+ *   header, LBM_CKPT_HEADER_BYTES bytes at fixed offsets:
+ *      0  char[8]  magic "LBMCKPT\0"        8  u32 format version (1)
+ *     12  u32 storage kind (LBM_CKPT_*)     16  u32 LBM_STRICT (0 or 1)
+ *     20  i32 nx    24  i32 ny    28  i32 reynolds_dim
+ *     32  u32 bits of the fp32 parse of density, 36 accel, 40 omega    44  u32 zero
+ *     48  u64 bits of the fp64 parse of density, 56 accel, 64 omega
+ *     72  i64 t, the timesteps done     80  u64 lbm_obstacle_hash of the obstacle bits
+ *     88  u64 lbm_gpu_digest checksum of the lattice
+ *   then t av_vels values as the run produced them (float; double for f64),
+ *   then the ny x nx records of lbm_gpu_save_rows (row 0 first): 36, 72 or 18 bytes per cell.
+ * --------------------------------------------------------------------------------- */
+#define LBM_CKPT_HEADER_BYTES 96
+enum { LBM_CKPT_F32 = 0, LBM_CKPT_F64 = 1, LBM_CKPT_F16 = 2 };
+
+typedef struct {
+  uint32_t version, kind, strict;
+  int32_t nx, ny, reynolds_dim;
+  uint32_t density_f32, accel_f32, omega_f32;
+  uint64_t density_f64, accel_f64, omega_f64;
+  int64_t steps_done;
+  uint64_t obstacle_hash;
+  uint64_t checksum;
+} lbm_ckpt_header;
+
+/* FNV-1a over the 32-bit words of the LBM_GPU_OBST_BITS mask (row-major) */
+uint64_t lbm_obstacle_hash(const uint32_t* bits, int nx, int ny);
+
+/* the header fields this run determines (steps_done and checksum are set when writing) */
+void lbm_ckpt_header_init(lbm_ckpt_header* h, uint32_t kind, int strict, const lbm_param* pf,
+                          const lbm_param_f64* pd, uint64_t obstacle_hash);
+
+/* Moves rows [row0, row0 + nrows) of the lattice between the device and buf (the host program
+ * passes lbm_gpu_save_rows / lbm_gpu_load_rows wrapped in its die() convention; this file makes
+ * no library calls, so that the readers and writers build without the library). */
+typedef void (*lbm_ckpt_rows_fn)(void* ctx, long long row0, long long nrows, void* buf);
+
+/* rows per block of the lattice section: about 64 MiB of records, at least 1, at most ny */
+long long lbm_ckpt_block_rows(const lbm_ckpt_header* h);
+
+/* Writes h (steps_done and checksum set by the caller), the first h->steps_done av_vels values
+ * and the lattice, a block of rows at a time through buf (lbm_ckpt_block_rows rows), to
+ * <path>.tmp; then fflush, fsync and rename to <path>, so that an interrupted write leaves an
+ * earlier checkpoint intact. */
+void lbm_write_checkpoint(const char* path, const lbm_ckpt_header* h, const void* av_vels,
+                          lbm_ckpt_rows_fn save_rows, void* ctx, void* buf);
+
+/* Opens a checkpoint and checks it against `want` (every field but steps_done and checksum),
+ * t <= max_iters and the exact size the header implies; die() names any mismatch.  Needs no
+ * GPU.  Returns the file positioned at the av_vels section and the header in `got`. */
+FILE* lbm_open_checkpoint(const char* path, const lbm_ckpt_header* want, int max_iters, lbm_ckpt_header* got);
+
+/* Reads the t av_vels values (float, or double for LBM_CKPT_F64) into av_vels, then the lattice
+ * a block of rows at a time through buf into load_rows; closes fp.  The caller compares the
+ * loaded lattice's checksum with h->checksum. */
+void lbm_read_checkpoint(FILE* fp, const lbm_ckpt_header* h, void* av_vels, lbm_ckpt_rows_fn load_rows,
+                         void* ctx, void* buf);
 
 #endif

@@ -312,6 +312,35 @@ int lbm_gpu_digest(lbm_gpu* h, double* total_density, unsigned long long* checks
 int lbm_gpu_upload(lbm_gpu* h, const float* cells_aos);
 int lbm_gpu_upload_f64(lbm_gpu* h, const double* cells_aos);
 
+/*
+ * Checkpoint and restart: global rows [row0, row0 + nrows) of the STORED lattice, in the handle's
+ * own storage type, nothing decoded or rounded.  Cell (ii, jj) is record ii + (jj - row0) * nx; a
+ * record is the cell's 9 stored elements in speed order 0..8:
+ *   fp32 handle                 float                                       36 bytes per cell
+ *   fp64 handle (create_f64)    double                                      72 bytes per cell
+ *   LBM_GPU_STORE_F16           uint16_t bit pattern of s_k = __float2half_rn(f_k - c_k)
+ *                               (the stored shifted value, see LBM_GPU_STORE_F16)   18 bytes per cell
+ * For fp32 and fp64 that is the t_speed AoS of lbm_gpu_download_rows / lbm_gpu_download_f64, byte for
+ * byte.  For binary16 it is the stored bits themselves, at half the bytes of lbm_gpu_download:
+ * download then upload decodes and re-encodes in fp32, which does not return every stored bit
+ * pattern (at density 10, 8195 of the finite binary16 values change, though each decodes to the
+ * same fp32 value as before), so a binary16 lattice is checkpointed with these two calls.
+ *
+ * After lbm_gpu_load_rows the handle behaves as if those rows had been computed into it: the side
+ * row of row ny-2 and the ghost rows its kernel needs are rebuilt; run(a); save; [any process, any
+ * slab layout] load; run(b) gives the bits of run(a + b).  steps_done, the kernel choice and the
+ * obstacle mask are not touched (loading changes contents, not geometry).  Load between runs only.
+ * A slab handle (lbm_gpu_create_slab) saves and loads the rows it holds; one that holds part of the
+ * grid cannot rebuild its neighbours' ghost rows itself, so after loading, every rank passes a host
+ * barrier, calls lbm_gpu_ipc_prepare, and passes a second barrier, as after creation; until its
+ * lbm_gpu_ipc_prepare, lbm_gpu_run on that handle is refused.
+ * Refused before anything is enqueued or written, with the call named in the message: a NULL
+ * pointer with nrows > 0, nrows < 0, rows beyond the grid or not held by this process, a handle
+ * whose earlier run was abandoned.  nrows = 0 succeeds and does nothing.
+ */
+int lbm_gpu_save_rows(lbm_gpu* h, long long row0, long long nrows, void* out);
+int lbm_gpu_load_rows(lbm_gpu* h, long long row0, long long nrows, const void* in);
+
 int lbm_gpu_get_info(lbm_gpu* h, lbm_gpu_info* info);
 
 /* Page-locked host memory for the caller's input/output arrays (the reference uses
