@@ -89,6 +89,7 @@ SYMBOLS = {
     "lbm_gpu_final_fields_f64": (C.c_int, [_P, C.c_longlong, C.c_longlong, _P, _P, _P, _P]),
     "lbm_gpu_av_velocity_f64": (C.c_int, [_P, _P]),
     "lbm_gpu_digest": (C.c_int, [_P, C.POINTER(C.c_double), C.POINTER(C.c_ulonglong)]),
+    "lbm_gpu_obstacle_force": (C.c_int, [_P, C.c_int, _P, _P]),
     "lbm_gpu_upload": (C.c_int, [_P, _P]),
     "lbm_gpu_upload_f64": (C.c_int, [_P, _P]),
     "lbm_gpu_save_rows": (C.c_int, [_P, C.c_longlong, C.c_longlong, _P]),
@@ -354,6 +355,19 @@ class Lattice:
         d, c = C.c_double(), C.c_ulonglong()
         _check(self.lib.lbm_gpu_digest(self.h, C.byref(d), C.byref(c)))
         return d.value, c.value
+
+    def obstacle_force(self, boxes=None):
+        """Momentum-exchange force (fx, fy) on the solid cells of each box, computed on the GPU
+        (lbm_gpu_obstacle_force): float64 array of shape (n, 2).  boxes: (n, 4) ints {x0, y0, x1, y1},
+        half-open global cell ranges; None is the whole grid.  A slab handle returns its rows' share."""
+        if boxes is None:
+            out = np.empty((1, 2), dtype=np.float64)
+            _check(self.lib.lbm_gpu_obstacle_force(self.h, 1, None, _ptr(out)))
+            return out
+        b = np.ascontiguousarray(boxes, dtype=np.int32).reshape(-1, 4)
+        out = np.empty((b.shape[0], 2), dtype=np.float64)
+        _check(self.lib.lbm_gpu_obstacle_force(self.h, b.shape[0], _ptr(b), _ptr(out)))
+        return out
 
     def info(self):
         i = Info()

@@ -1727,6 +1727,100 @@ class Grid : public GridBase {
     if (total_density) *total_density = bad ? std::nan("") : (double)(long long)mass / 4294967296.0;
     if (checksum) *checksum = sum;
   }
+
+  // Momentum-exchange force on the solid cells of each box (lbm_gpu_obstacle_force; the arithmetic
+  // is in lbm_obstacle_force).  boxes: n x {x0, y0, x1, y1}, already checked.  Each slab sums the
+  // solid cells of its rows; the slabs' 128-bit integer sums are added here before the one
+  // conversion to double, so any split of the rows over this process's slabs gives the same bits.
+  void obstacle_force(int n, const int* boxes, double* out) {
+    if (failed) throw CudaError{"an earlier run of this lattice was abandoned (a neighbouring slab never arrived); "
+                                "its contents are void"};
+    if (loaded_unprepared)
+      throw CudaError{"rows were loaded into this slab handle with lbm_gpu_load_rows and its ghost rows are stale: "
+                      "pass a host barrier over all ranks, lbm_gpu_ipc_prepare, and a second barrier first"};
+    if (!connected) throw CudaError{"lattice is not connected to its neighbours yet (its ghost rows are not filled)"};
+    const size_t table_bytes = (size_t)lbm::kForceMaxBoxes * sizeof(lbm::ForceBox);
+    const size_t out_words = (size_t)n * lbm::kForceOutWords;
+    std::vector<unsigned __int128> sum((size_t)2 * n, 0);
+    std::vector<char> bad(n, 0);
+    std::vector<unsigned long long> w(out_words);
+    std::vector<lbm::ForceBox> table(n);
+    for (auto& s : slabs) {
+      CK(cudaSetDevice(s.device));
+      // each box gets the blocks its mask words in this slab need, at most one resident wave
+      const long long cap = force_resident_blocks(s);
+      int total = 0;
+      for (int j = 0; j < n; j++) {
+        const int* q = boxes + 4 * j;
+        lbm::ForceBox& t = table[j];
+        const long long r0 = std::max<long long>(q[1], s.row0), r1 = std::min<long long>(q[3], s.row0 + s.rows);
+        t.x0 = q[0];
+        t.x1 = q[2];
+        t.r0 = (int)(r0 - s.row0);
+        t.w0 = q[0] / 32;
+        t.nw = q[2] > q[0] ? (q[2] + 31) / 32 - t.w0 : 0;
+        t.words = r1 > r0 ? (r1 - r0) * t.nw : 0;
+        t.first = total;
+        t.blocks = (int)std::min<long long>(cap, (t.words + lbm::kForceThreads - 1) / lbm::kForceThreads);
+        total += t.blocks;
+      }
+      lbm::ForceBox* d_table = (lbm::ForceBox*)s.staging;
+      unsigned long long* d_out = (unsigned long long*)((char*)s.staging + table_bytes);
+      CK(cudaMemsetAsync(d_out, 0, out_words * sizeof(unsigned long long), s.stream));
+      if (total > 0) {
+        CK(cudaMemcpyAsync(d_table, table.data(), (size_t)n * sizeof(lbm::ForceBox), cudaMemcpyHostToDevice, s.stream));
+        const bool whole = s.rows == prm.ny;
+        if (f16) {
+          lbm::ForceArgs<__half, float> a;
+          a.buf = hlat(s, cur);
+          a.side = (const float*)s.side[cur];
+          a.ghost_s = a.ghost_n = nullptr;      // a binary16 lattice is one slab that holds the whole grid
+          fill_force_args(a, s, whole, d_table, d_out, n);
+          lbm::lbm_obstacle_force<__half, float><<<total, lbm::kForceThreads, 0, s.stream>>>(a);
+        } else {
+          lbm::ForceArgs<real, real> a;
+          a.buf = s.lattice[cur];
+          a.side = s.side[cur];
+          a.ghost_s = whole ? nullptr : win_section(s.win, cur, 0);
+          a.ghost_n = whole ? nullptr : win_section(s.win, cur, 1);
+          fill_force_args(a, s, whole, d_table, d_out, n);
+          lbm::lbm_obstacle_force<real, real><<<total, lbm::kForceThreads, 0, s.stream>>>(a);
+        }
+        CK(cudaGetLastError());
+        launches++;
+      }
+      CK(cudaMemcpyAsync(w.data(), d_out, out_words * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s.stream));
+      CK(cudaStreamSynchronize(s.stream));
+      for (int j = 0; j < n; j++) {
+        const unsigned long long* o = &w[(size_t)j * lbm::kForceOutWords];
+        for (int c = 0; c < 2; c++) sum[2 * j + c] += ((unsigned __int128)o[2 * c + 1] << 64) | o[2 * c];
+        bad[j] |= o[4] != 0;
+      }
+    }
+    for (int j = 0; j < n; j++)
+      for (int c = 0; c < 2; c++)
+        out[2 * j + c] = bad[j] ? std::nan("") : std::ldexp((double)(__int128)sum[2 * j + c], -32);
+  }
+  // blocks of K14 resident on the slab's GPU at once (its register count decides)
+  long long force_resident_blocks(const Slab<real>& s) const {
+    int per_sm = 0, sms = 0;
+    if (f16) CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lbm::lbm_obstacle_force<__half, float>, lbm::kForceThreads, 0));
+    else CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lbm::lbm_obstacle_force<real, real>, lbm::kForceThreads, 0));
+    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s.device));
+    return std::max<long long>(1, (long long)per_sm * sms);
+  }
+  template <typename A>
+  void fill_force_args(A& a, const Slab<real>& s, bool whole, const lbm::ForceBox* d_table, unsigned long long* d_out, int n) {
+    a.mask = s.mask;
+    a.ghost_mask = s.ghost_mask;
+    a.boxes = d_table;
+    a.out = d_out;
+    a.plane_stride = plane_stride(s);
+    a.nx = prm.nx; a.rows = s.rows; a.pitch = pitch; a.mask_pitch = mask_pitch; a.accel_row = s.accel_row;
+    a.n_boxes = n;
+    a.whole = whole;
+    a.rest = rest();
+  }
 };
 
 // split ny rows over n slabs: remainder spread over the first slabs
@@ -2376,6 +2470,32 @@ int lbm_gpu_digest(lbm_gpu* h, double* total_density, unsigned long long* checks
   if (reinterpret_cast<GridBase*>(h)->is_f64())
     return guarded<double>(h, "lbm_gpu_digest", [&](Grid<double>& g) { g.digest(total_density, checksum); });
   return guarded<float>(h, "lbm_gpu_digest", [&](Grid<float>& g) { g.digest(total_density, checksum); });
+}
+
+int lbm_gpu_obstacle_force(lbm_gpu* h, int n_boxes, const int* boxes, double* force_out) {
+  const char* fn = "lbm_gpu_obstacle_force";
+  if (!h) return fail("%s: NULL handle", fn);
+  if (n_boxes < 1 || n_boxes > lbm::kForceMaxBoxes)
+    return fail("%s: n_boxes %d is not in 1..%d", fn, n_boxes, lbm::kForceMaxBoxes);
+  if (!force_out) return fail("%s: NULL force_out", fn);
+  if (!boxes && n_boxes != 1) return fail("%s: boxes is NULL with n_boxes %d (NULL means one box, the whole grid)", fn, n_boxes);
+  auto body = [&](auto& g) {
+    const int nx = g.prm.nx, ny = g.prm.ny;
+    const int whole[4] = {0, 0, nx, ny};
+    const int* b = boxes ? boxes : whole;
+    for (int j = 0; j < n_boxes; j++) {
+      const int* q = b + 4 * j;
+      if (!(0 <= q[0] && q[0] <= q[2] && q[2] <= nx && 0 <= q[1] && q[1] <= q[3] && q[3] <= ny)) {
+        char m[256];
+        snprintf(m, sizeof m, "box %d {x0 %d, y0 %d, x1 %d, y1 %d} is not within 0 <= x0 <= x1 <= nx = %d and "
+                 "0 <= y0 <= y1 <= ny = %d", j, q[0], q[1], q[2], q[3], nx, ny);
+        throw CudaError{m};
+      }
+    }
+    g.obstacle_force(n_boxes, b, force_out);
+  };
+  if (reinterpret_cast<GridBase*>(h)->is_f64()) return guarded<double>(h, fn, body);
+  return guarded<float>(h, fn, body);
 }
 
 namespace {

@@ -1589,6 +1589,192 @@ lbm_coarse_fields(const store* __restrict__ buf, const uint32_t* __restrict__ ma
   }
 }
 
+// K14 lbm_obstacle_force: the momentum-exchange force on the solid cells of each box
+// (lbm_gpu_obstacle_force, include/lbm_gpu.h).  A link is a solid cell x_s and a speed d whose
+// neighbour x_s + c_d is fluid; it adds -c_d * (f~_d(x_s) + f~_opp(d)(x_s + c_d)) to every box
+// that holds x_s, which is the header's formula regrouped by link.  f~ is the stored lattice,
+// and the side row on row ny-2.
+//
+// Each block serves one box: the host gives every box as many blocks as its mask words in this
+// slab need (at most one resident wave), from first block `first` on.  A thread takes one 32-cell
+// mask word of the box at a time (grid-stride over the box's words only), keeps the word's solid
+// cells that lie in the box's columns, and finds their links with word-wide bit operations on the
+// mask words of rows r-1, r, r+1 and their neighbouring words (periodic at nx, not at the pitch).
+// A word without links in the box reads no lattice value, so a box costs its own mask words plus
+// its boundary cells.  Rows r-1 and r+1:
+//   whole   the slab holds the whole grid: they wrap inside the slab (K1a-f16 reads them so);
+//   else    rows -1 and `rows` are the depth-0 ghost rows (planes 2,5,6 and 4,7,8, already
+//           accelerated, exactly the ones a pull across the edge needs) and their mask words
+//           are the ghost mask.
+// Each value enters as round_half_even(v * 2^32), the digest's conversion.  A thread keeps signed
+// 128-bit sums of its box's components in registers; the warp adds them with shuffles, the block
+// in shared memory, and the block's sums go into `out` as two 64-bit words with the carry of the
+// low word added to the high one: exact modulo 2^128 in any order.  A value that is not finite or
+// of magnitude 2^31 or more marks the box instead.
+constexpr int kForceThreads = 256;
+constexpr int kForceMaxBoxes = 256;
+constexpr int kForceOutWords = 5;                    // per box: fx lo, fx hi, fy lo, fy hi, mark
+
+// one box's share of the launch, in this slab's local coordinates (lbm_gpu.cu fills it)
+struct ForceBox {
+  int first, blocks;                                 // its blocks: [first, first + blocks)
+  int r0, w0, nw;                                    // local rows from r0, mask words [w0, w0 + nw) of each
+  int x0, x1;                                        // its columns [x0, x1)
+  long long words;                                   // rows x nw
+};
+
+template <typename store, typename val>
+struct ForceArgs {
+  const store* buf;                                  // lattice buffer of the current state
+  const val* side;                                   // its side row
+  const val* ghost_s;                                // depth-0 ghost rows -1 and `rows` (not whole)
+  const val* ghost_n;
+  const uint32_t* mask;
+  const uint32_t* ghost_mask;                        // mask words of rows -1 and `rows` (not whole)
+  const ForceBox* boxes;                             // n_boxes
+  unsigned long long* out;                           // n_boxes x kForceOutWords
+  long long plane_stride;
+  int nx, rows, pitch, mask_pitch, accel_row, n_boxes;
+  bool whole;
+  RestShift rest;
+};
+
+__device__ __forceinline__ void add_i128(unsigned long long* p, const __int128 v) {
+  const unsigned long long lo = (unsigned long long)v, hi = (unsigned long long)(v >> 64);
+  const unsigned long long old = atomicAdd(p, lo);
+  const unsigned long long h = hi + (old + lo < old ? 1ULL : 0ULL);
+  if (h) atomicAdd(p + 1, h);
+}
+
+template <typename store, typename val>
+__device__ __forceinline__ const uint32_t* force_mask_row(const ForceArgs<store, val>& a, int r) {
+  if (a.whole) return a.mask + (long long)(r < 0 ? r + a.rows : r >= a.rows ? r - a.rows : r) * a.mask_pitch;
+  if (r < 0) return a.ghost_mask;
+  if (r >= a.rows) return a.ghost_mask + a.mask_pitch;
+  return a.mask + (long long)r * a.mask_pitch;
+}
+
+// f~_k at local row r (-1 .. rows), column x
+template <typename store, typename val>
+__device__ __forceinline__ val force_value(const ForceArgs<store, val>& a, const int k, int r, const int x) {
+  if (a.whole) {
+    r = r < 0 ? r + a.rows : r >= a.rows ? r - a.rows : r;
+  } else {
+    if (r < 0) return a.ghost_s[(long long)k * a.pitch + x];
+    if (r >= a.rows) return a.ghost_n[(long long)k * a.pitch + x];
+  }
+  if (r == a.accel_row && k != 0 && k != 2 && k != 4) {
+    const int idx = (k == 1) ? 0 : (k == 3) ? 1 : k - 3;       // side row order 1,3,5,6,7,8
+    return a.side[(long long)idx * a.pitch + x];
+  }
+  return stored_value(a.buf + k * a.plane_stride + (long long)r * a.pitch + x, k, a.rest);
+}
+
+// round_half_even(v * 2^32) into acc; false when v has no fixed-point value
+template <typename val>
+__device__ __forceinline__ bool force_fixed(const val v, long long& q) {
+  if (!(::fabs((double)v) < 2147483648.0)) return false;
+  q = __double2ll_rn((double)v * 4294967296.0);
+  return true;
+}
+
+__device__ __forceinline__ __int128 warp_sum_i128(__int128 v) {
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    const unsigned long long lo = __shfl_down_sync(0xffffffffu, (unsigned long long)v, off);
+    const unsigned long long hi = __shfl_down_sync(0xffffffffu, (unsigned long long)(v >> 64), off);
+    v += (__int128)(((unsigned __int128)hi << 64) | lo);
+  }
+  return v;
+}
+
+template <typename store, typename val>
+__global__ void __launch_bounds__(kForceThreads) lbm_obstacle_force(const ForceArgs<store, val> a) {
+  __shared__ unsigned long long acc[4];
+  __shared__ unsigned mark;
+  __shared__ int box_of_block;
+  if (threadIdx.x == 0) {                            // the box whose blocks hold this one
+    int lo = 0, hi = a.n_boxes - 1;
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (a.boxes[mid].first <= (int)blockIdx.x) lo = mid; else hi = mid - 1;
+    }
+    box_of_block = lo;
+    mark = 0u;
+  }
+  if (threadIdx.x < 4) acc[threadIdx.x] = 0ULL;
+  __syncthreads();
+  const int j = box_of_block;
+  const ForceBox bx = a.boxes[j];
+  __int128 sx = 0, sy = 0;
+  bool bad = false;
+  const int wpr = (a.nx + 31) >> 5;
+  const int last = (a.nx - 1) & 31;                  // bit of column nx-1 in the row's last word
+  const long long stride = (long long)bx.blocks * blockDim.x;
+  for (long long i = (long long)(blockIdx.x - bx.first) * blockDim.x + threadIdx.x; i < bx.words; i += stride) {
+    const int rr = (int)(i / bx.nw), w = bx.w0 + (int)(i - (long long)rr * bx.nw);
+    const int r = bx.r0 + rr;
+    const uint32_t* m0 = force_mask_row(a, r);
+    // solid cells of the word inside the box's columns
+    const int lo = ::max(bx.x0 - 32 * w, 0), hi = ::min(bx.x1 - 32 * w, 32);
+    const uint32_t cols = (hi >= 32 ? 0xffffffffu : (1u << hi) - 1u) & ~((1u << lo) - 1u);
+    const uint32_t s = m0[w] & cols;
+    if (!s) continue;
+    // for row dy = -1, 0, 1: the mask at x (c), x + 1 (e) and x - 1 (wv) for the 32 columns of word w
+    uint32_t c[3], e[3], wv[3];
+#pragma unroll
+    for (int dy = 0; dy < 3; dy++) {
+      const uint32_t* m = dy == 1 ? m0 : force_mask_row(a, r + dy - 1);
+      c[dy] = m[w];
+      e[dy] = (c[dy] >> 1) | (w + 1 < wpr ? m[w + 1] << 31 : 0u);
+      if (w == wpr - 1) e[dy] |= (m[0] & 1u) << last;
+      wv[dy] = (c[dy] << 1) | (w > 0 ? m[w - 1] >> 31 : (m[wpr - 1] >> last) & 1u);
+    }
+    // solid cells of the word whose neighbour along speed d is fluid (c_d = (dx, dy), d = 1..8)
+    uint32_t link[9];
+    link[0] = 0u;
+    link[1] = s & ~e[1];  link[2] = s & ~c[2];  link[3] = s & ~wv[1]; link[4] = s & ~c[0];
+    link[5] = s & ~e[2];  link[6] = s & ~wv[2]; link[7] = s & ~wv[0]; link[8] = s & ~e[0];
+    uint32_t any = 0u;
+#pragma unroll
+    for (int d = 1; d < 9; d++) any |= link[d];
+    while (any) {
+      const int b = __ffs(any) - 1;
+      any &= any - 1;
+      const int x = w * 32 + b;
+#pragma unroll
+      for (int d = 1; d < 9; d++) {
+        if (!((link[d] >> b) & 1u)) continue;
+        const int dx = (d == 1 || d == 5 || d == 8) ? 1 : (d == 3 || d == 6 || d == 7) ? -1 : 0;
+        const int dy = (d == 2 || d == 5 || d == 6) ? 1 : (d == 4 || d == 7 || d == 8) ? -1 : 0;
+        const int opp = (d < 5) ? ((d + 1) & 3) + 1 : ((d - 3) & 3) + 5;
+        const int xn = x + dx < 0 ? a.nx - 1 : x + dx >= a.nx ? 0 : x + dx;
+        long long q0 = 0, q1 = 0;
+        bad |= !force_fixed(force_value(a, d, r, x), q0);
+        bad |= !force_fixed(force_value(a, opp, r + dy, xn), q1);
+        const __int128 q = (__int128)q0 + q1;
+        if (dx > 0) sx -= q; else if (dx < 0) sx += q;
+        if (dy > 0) sy -= q; else if (dy < 0) sy += q;
+      }
+    }
+  }
+  // warp sums, one shared atomic per warp and component, one global per block
+  if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) mark = 1u;
+  sx = warp_sum_i128(sx);
+  sy = warp_sum_i128(sy);
+  if ((threadIdx.x & 31) == 0) {
+    if (sx) add_i128(&acc[0], sx);
+    if (sy) add_i128(&acc[2], sy);
+  }
+  __syncthreads();
+  unsigned long long* o = a.out + (long long)j * kForceOutWords;
+  if (threadIdx.x < 2) {
+    const __int128 v = (__int128)(((unsigned __int128)acc[2 * threadIdx.x + 1] << 64) | acc[2 * threadIdx.x]);
+    if (v) add_i128(o + 2 * threadIdx.x, v);
+  }
+  if (threadIdx.x == 0 && mark) atomicOr(o + 4, 1ULL);
+}
+
 // Digest of the lattice rows [r0, r0+nrows): two wrapping 64-bit integer sums, so they
 // are exact, order-independent and additive over slabs / ranks.
 //   mass      sum over cells and speeds of round(f * 2^32): total_density of the reference

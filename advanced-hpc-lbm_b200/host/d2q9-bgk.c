@@ -33,6 +33,13 @@
  *                          larger), obstacle file, LBM_PRECISION and LBM_STRICT; LBM_GPUS may
  *                          differ.  The header is checked before the GPU is touched; av_vels.dat
  *                          then holds all maxIters lines and both files equal an uninterrupted run's
+ *   LBM_FORCE_EVERY=k      write forces.dat: the momentum-exchange force on the obstacles
+ *                          (lbm_gpu_obstacle_force) at every state t = k, 2k, ... <= maxIters, one
+ *                          line "t fx fy [fx fy ...]" (tab-separated, %.12E).  The run is cut into
+ *                          lbm_gpu_run calls at multiples of k, which changes no output bit; after
+ *                          LBM_RESTART the file holds the samples after the restart step
+ *   LBM_FORCE_BOXES="x0,y0,x1,y1;..."   the boxes of the force (half-open global cell ranges; a
+ *                          solid cell counts in every box that holds it); default: the whole grid
  */
 #define _POSIX_C_SOURCE 200809L
 #include <math.h>
@@ -47,6 +54,7 @@
 
 #define FINALSTATEFILE "final_state.dat"
 #define AVVELSFILE "av_vels.dat"
+#define FORCESFILE "forces.dat"
 
 static void usage(const char* exe)
 {
@@ -102,6 +110,13 @@ static void write_checkpoint(const char* path, lbm_gpu* gpu, lbm_ckpt_header* h,
   else free(buf);
 }
 
+/* one line of forces.dat: the force on each box at state t */
+static void sample_force(lbm_gpu* gpu, FILE* fp, long long t, int n_boxes, const int* boxes, double* force)
+{
+  GPU(lbm_gpu_obstacle_force(gpu, n_boxes, boxes, force));
+  lbm_write_force_line(fp, t, n_boxes, force);
+}
+
 static int env_flag(const char* name)
 {
   const char* v = getenv(name);
@@ -144,6 +159,9 @@ int main(int argc, char* argv[])
       die("LBM_CHECKPOINT_EVERY must be a positive number of steps", __LINE__, __FILE__);
     if (ckpt_path == NULL) die("LBM_CHECKPOINT_EVERY needs LBM_CHECKPOINT=<path>", __LINE__, __FILE__);
   }
+  const long long force_every = getenv("LBM_FORCE_EVERY") != NULL ? lbm_parse_force_every(getenv("LBM_FORCE_EVERY")) : 0;
+  if (getenv("LBM_FORCE_BOXES") != NULL && force_every == 0)
+    die("LBM_FORCE_BOXES needs LBM_FORCE_EVERY=<k>", __LINE__, __FILE__);
 
   /* Total/init time starts here: load values from file, build the device lattice */
   const double tot_tic = wtime();
@@ -154,6 +172,14 @@ int main(int argc, char* argv[])
   lbm_read_params(paramfile, &params, &params_d);
   const int nx = params.nx, ny = params.ny, iters = params.maxIters;
   uint32_t* obstacle_bits = lbm_read_obstacle_bits(obstaclefile, nx, ny);
+
+  /* the boxes of the force time series: the whole grid unless LBM_FORCE_BOXES names them */
+  static int force_boxes[4 * LBM_FORCE_MAX_BOXES];
+  static double force[2 * LBM_FORCE_MAX_BOXES];
+  int n_boxes = 1;
+  force_boxes[2] = nx;
+  force_boxes[3] = ny;
+  if (getenv("LBM_FORCE_BOXES") != NULL) n_boxes = lbm_parse_force_boxes(getenv("LBM_FORCE_BOXES"), nx, ny, force_boxes);
 
   /* a record of the av. velocity computed for each timestep (d2q9-bgk.c:2866) */
   double* av_vels = (double*)malloc(sizeof(double) * (size_t)(iters > 0 ? iters : 1));
@@ -197,7 +223,12 @@ int main(int argc, char* argv[])
   const double init_toc = wtime();
   const double comp_tic = init_toc;
 
-  double ckpt_secs = 0.0;        /* checkpoint writes, not counted as compute time */
+  double ckpt_secs = 0.0;        /* checkpoint writes and force samples, not counted as compute time */
+  FILE* forces_fp = NULL;
+  if (force_every > 0) {
+    forces_fp = fopen(FORCESFILE, "w");
+    if (forces_fp == NULL) die("could not open file " FORCESFILE, __LINE__, __FILE__);
+  }
   if (env_flag("LBM_DEBUG")) {
     for (int tt = t0; tt < iters; tt++) {
       double density;
@@ -211,16 +242,24 @@ int main(int argc, char* argv[])
       printf("==timestep: %d==\n", tt);
       printf("av velocity: %.12E\n", av_vels[tt]);
       printf("tot density: %.12E\n", density);
+      if (force_every > 0 && (tt + 1) % force_every == 0) sample_force(gpu, forces_fp, tt + 1, n_boxes, force_boxes, force);
     }
   } else {
-    /* steps [t0, iters), cut at the multiples of LBM_CHECKPOINT_EVERY */
+    /* steps [t0, iters), cut at the multiples of LBM_CHECKPOINT_EVERY and of LBM_FORCE_EVERY */
     for (int t = t0; t < iters;) {
-      const int next = every > 0 ? (int)(((long long)t / every + 1) * every < iters ? ((long long)t / every + 1) * every : iters)
-                                 : iters;
-      if (f64) GPU(lbm_gpu_run_f64(gpu, next - t, av_vels + t));
-      else GPU(lbm_gpu_run(gpu, next - t, av_vels_f + t));
-      t = next;
-      if (every > 0 && t < iters) {
+      long long next = iters;
+      if (every > 0 && ((long long)t / every + 1) * every < next) next = ((long long)t / every + 1) * every;
+      if (force_every > 0 && ((long long)t / force_every + 1) * force_every < next)
+        next = ((long long)t / force_every + 1) * force_every;
+      if (f64) GPU(lbm_gpu_run_f64(gpu, (int)next - t, av_vels + t));
+      else GPU(lbm_gpu_run(gpu, (int)next - t, av_vels_f + t));
+      t = (int)next;
+      if (force_every > 0 && t % force_every == 0) {
+        const double tic = wtime();
+        sample_force(gpu, forces_fp, t, n_boxes, force_boxes, force);
+        ckpt_secs += wtime() - tic;
+      }
+      if (every > 0 && t < iters && t % every == 0) {
         const double tic = wtime();
         write_checkpoint(ckpt_path, gpu, &ckpt, t, f64 ? (const void*)av_vels : (const void*)av_vels_f);
         ckpt_secs += wtime() - tic;
@@ -325,6 +364,7 @@ int main(int argc, char* argv[])
     fclose(fp);
   }
   lbm_write_av_vels(AVVELSFILE, iters, av_vels);
+  if (forces_fp != NULL && fclose(forces_fp) != 0) die("could not write " FORCESFILE, __LINE__, __FILE__);
 
   lbm_gpu_destroy(gpu);
   free(av_vels);

@@ -485,3 +485,75 @@ void lbm_read_checkpoint(FILE* fp, const lbm_ckpt_header* h, void* av_vels, lbm_
   }
   fclose(fp);
 }
+
+/* ------------------------------------------------------------------ obstacle force time series */
+long long lbm_parse_force_every(const char* text)
+{
+  char* end = NULL;
+  errno = 0;
+  const long long k = strtoll(text, &end, 10);
+  if (end == text || *end != '\0' || errno != 0 || k < 1 || k > 2147483647LL)
+    die("LBM_FORCE_EVERY must be a positive number of steps", __LINE__, __FILE__);
+  return k;
+}
+
+int lbm_parse_force_boxes(const char* spec, int nx, int ny, int* boxes)
+{
+  char msg[512];
+  int n = 0;
+  const char* p = spec;
+  for (;;) {
+    const char* end = strchr(p, ';');
+    const size_t len = end ? (size_t)(end - p) : strlen(p);
+    char item[128];
+    if (n == LBM_FORCE_MAX_BOXES) {
+      snprintf(msg, sizeof msg, "LBM_FORCE_BOXES: more than %d boxes", LBM_FORCE_MAX_BOXES);
+      die(msg, __LINE__, __FILE__);
+    }
+    long long v[4];
+    int ok = len > 0 && len < sizeof item;
+    if (ok) {
+      memcpy(item, p, len);
+      item[len] = '\0';
+      const char* q = item;
+      for (int i = 0; i < 4 && ok; i++) {
+        char* e = NULL;
+        errno = 0;
+        while (*q == ' ') q++;
+        v[i] = strtoll(q, &e, 10);
+        ok = e != q && errno == 0;
+        q = e;
+        while (*q == ' ') q++;
+        if (ok && i < 3) ok = *q++ == ',';
+      }
+      ok = ok && *q == '\0';
+    }
+    if (!ok) {
+      snprintf(msg, sizeof msg, "LBM_FORCE_BOXES: box %d (\"%.*s\") is not four integers x0,y0,x1,y1", n,
+               (int)(len < 100 ? len : 100), p);
+      die(msg, __LINE__, __FILE__);
+    }
+    if (!(0 <= v[0] && v[0] <= v[2] && v[2] <= nx && 0 <= v[1] && v[1] <= v[3] && v[3] <= ny)) {
+      snprintf(msg, sizeof msg, "LBM_FORCE_BOXES: box %d (%lld,%lld,%lld,%lld) is not within 0 <= x0 <= x1 <= nx = %d "
+               "and 0 <= y0 <= y1 <= ny = %d", n, v[0], v[1], v[2], v[3], nx, ny);
+      die(msg, __LINE__, __FILE__);
+    }
+    for (int i = 0; i < 4; i++) boxes[4 * n + i] = (int)v[i];
+    n++;
+    if (!end) break;
+    p = end + 1;
+  }
+  return n;
+}
+
+void lbm_write_force_line(FILE* fp, long long step, int n_boxes, const double* force)
+{
+  char line[32 + LBM_FORCE_MAX_BOXES * 2 * 24];
+  int o = snprintf(line, sizeof line, "%lld", step);
+  for (int i = 0; i < 2 * n_boxes; i++) {
+    line[o++] = '\t';
+    o += lbm_format_e12(line + o, force[i]);
+  }
+  line[o++] = '\n';
+  if (fwrite(line, 1, (size_t)o, fp) != (size_t)o) die("could not write forces.dat", __LINE__, __FILE__);
+}

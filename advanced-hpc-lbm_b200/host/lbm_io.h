@@ -98,4 +98,21 @@ FILE* lbm_open_checkpoint(const char* path, const lbm_ckpt_header* want, int max
 void lbm_read_checkpoint(FILE* fp, const lbm_ckpt_header* h, void* av_vels, lbm_ckpt_rows_fn load_rows,
                          void* ctx, void* buf);
 
+/* ---------------------------------------------------------------------------------
+ * Obstacle force time series (LBM_FORCE_EVERY / LBM_FORCE_BOXES): forces.dat has one line per
+ * sample state t = k, 2k, ... <= maxIters: t, then fx and fy of each box ("%.12E"), tab-separated.
+ * --------------------------------------------------------------------------------- */
+#define LBM_FORCE_MAX_BOXES 256      /* what lbm_gpu_obstacle_force accepts */
+
+/* LBM_FORCE_EVERY: a positive step count, else die() */
+long long lbm_parse_force_every(const char* text);
+
+/* LBM_FORCE_BOXES "x0,y0,x1,y1;...": half-open global cell ranges with 0 <= x0 <= x1 <= nx and
+ * 0 <= y0 <= y1 <= ny, at most LBM_FORCE_MAX_BOXES of them, into boxes[4 * i ...]; returns their
+ * number.  A malformed box or one outside the grid ends in die() with a message that names it. */
+int lbm_parse_force_boxes(const char* spec, int nx, int ny, int* boxes /* 4 * LBM_FORCE_MAX_BOXES */);
+
+/* one line of forces.dat: step, then force[0 .. 2 * n_boxes) */
+void lbm_write_force_line(FILE* fp, long long step, int n_boxes, const double* force);
+
 #endif

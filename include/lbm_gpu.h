@@ -308,6 +308,55 @@ int lbm_gpu_av_velocity_f64(lbm_gpu* h, double* av_out);
  */
 int lbm_gpu_digest(lbm_gpu* h, double* total_density, unsigned long long* checksum);
 
+/*
+ * Force on obstacles by momentum exchange, computed on the device: the drag (x) and lift (y) on
+ * the solid cells inside each of n_boxes boxes, for a time series of a flow past obstacles without
+ * moving the lattice across PCIe.
+ *
+ * At state t (after t steps):
+ *   f~    the values step t+1 streams: the stored lattice values, except that on row ny-2 speeds
+ *         1, 3, 5, 6, 7 and 8 hold their values after accelerate_flow (the side row);
+ *   S     the obstacle cells;  c_k the speed vectors (order above, +y = towards row ny-1);
+ *   x +- c_k wraps periodically in x and y.
+ * The force exerted on the solid cells of box B during step t+1 is
+ *
+ *   F_B(t) = sum over x_s in S and B of [   sum_{k=1..8, x_s - c_k not in S} c_k f~_k(x_s - c_k)
+ *                                         - sum_{k=1..8, x_s + c_k not in S} c_k f~_k(x_s)       ]
+ *
+ * the momentum streaming into the solid minus the momentum it sends back (the values it holds
+ * after its previous rebound).  Collision conserves momentum, so summed over all solid cells
+ * P_fluid(t+1) = P~_fluid(t) - F_all(t) up to the collision's rounding (P~: fluid momentum of f~).
+ * +x is the direction accelerate_flow pushes: F_x is the drag.
+ *
+ * Arithmetic: exact, and the same for any split of the rows over slabs.  Each value v that enters
+ * becomes the signed integer round_half_even(v * 2^32) (the digest's conversion); the signed sums
+ * S_B are exact integers in 128 bits.  Each integer is below 2^63 in magnitude and a solid cell
+ * adds at most 12 of them per component, so |S_B| < 12 * 2^63 * cells < 2^127 for any grid of fewer
+ * than 2^60 cells (18 EiB even as binary16): no sum the library can form wraps.  The output is the
+ * correctly rounded double of S_B * 2^-32 (for the
+ * binary16 lattice the values are the decoded fp32 ones).  A box with a contributing value that is
+ * NaN, infinite or of magnitude 2^31 or more reports NaN for both components; other boxes are
+ * unaffected.
+ *
+ *   boxes      n_boxes x {x0, y0, x1, y1}: half-open global cell ranges [x0, x1) x [y0, y1),
+ *              0 <= x0 <= x1 <= nx, 0 <= y0 <= y1 <= ny.  They may overlap or be empty; a solid cell
+ *              counts in every box that holds it.  NULL with n_boxes == 1: the whole grid.
+ *   force_out  n_boxes x {fx, fy}.
+ * n_boxes 1..256.  Works for fp32, fp64 and binary16 handles after any kernel.  The lattice,
+ * steps_done and the kernel choice are not touched, so run(a); obstacle_force; run(b) equals
+ * run(a+b).  A handle with several slabs in this process adds their integer sums before the
+ * conversion.  A slab handle (lbm_gpu_create_slab) returns the share of the solid cells in its
+ * rows (their links may reach the neighbours' rows): add the shares across ranks in double, one
+ * rounding per rank, as with lbm_gpu_run_sums.
+ * Refused before anything is enqueued or written, with a message that starts with
+ * "lbm_gpu_obstacle_force:" and names the cause: n_boxes out of range, a NULL force_out, NULL boxes
+ * with n_boxes != 1, a malformed box (named by its index), a handle whose earlier run was
+ * abandoned, a slab handle that is not connected to its neighbours yet, and a slab handle that
+ * loaded rows and has not called lbm_gpu_ipc_prepare yet (its ghost rows are stale, as for
+ * lbm_gpu_run).  A box costs its own area: the mask words it covers and its boundary cells.
+ */
+int lbm_gpu_obstacle_force(lbm_gpu* h, int n_boxes, const int* boxes, double* force_out);
+
 /* Replace the device lattice by the caller's (whole local rows, AoS). */
 int lbm_gpu_upload(lbm_gpu* h, const float* cells_aos);
 int lbm_gpu_upload_f64(lbm_gpu* h, const double* cells_aos);
